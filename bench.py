@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json's metric on its named config, on N B200s of one node.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|...]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|...] [--dump-outputs DIR]
 
 metric    decoded points/s (whole job, all N GPUs); output GB/s is reported beside it
 workload  N=1: BASELINE.json configs[1] -- 10,000 synthetic point clouds x 100,000 points, 14-bit quantized
@@ -19,12 +19,17 @@ cpu_baseline  the CPU oracle (a linear-time port of the reference's algorithm; t
           in the image, and it cannot decode point clouds at all) on a bounded sample, all host cores
 
 --impl reference times that CPU oracle as the reference arm (the one other place oracle/ is executed).
+--dump-outputs DIR  after the timed steps, what the last step decoded (see sample_outputs), so that two builds can be
+          compared output for output: the inputs are generated from fixed seeds.
+
+bench.py runs against the libraries build() left in the tree and writes nothing there.
 """
 import argparse
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -207,12 +212,44 @@ def profile_traffic(workload):
     return None
 
 
+DUMP_BUDGET = 60 << 20  # payload bytes of --dump-outputs; with the .npy headers the files stay under 64 MB
+
+
+def widened(dtype):
+    """float32 holds float32 and 8/16-bit integers exactly, float64 holds 32-bit integers exactly."""
+    dtype = np.dtype(dtype)
+    return np.dtype(np.float32 if dtype == np.float32 or dtype.itemsize <= 2 else np.float64)
+
+
+def sample_outputs(batch, fetch):
+    """The decoded attributes of a fixed, seeded sample of the batch's buffers, as a caller receives them
+    (PointAttribute.values: entries x components).  Buffers are taken in a seeded order until DUMP_BUDGET is reached.
+    fetch(off, nbytes) returns those bytes of the output arena.  Returns {buffer index: [array per attribute]}."""
+    from draco_sharp_b200.decoder import NP_DTYPES
+    out, used = {}, 0
+    for k in np.random.default_rng(0xD0D0).permutation(batch.n_bufs).tolist():
+        infos = [batch.attr_info(k, a) for a in range(batch.buffer_info(k).n_attrs)]
+        size = sum(ai.n_entries * ai.num_components * widened(NP_DTYPES[ai.data_type]).itemsize for ai in infos)
+        if used + size > DUMP_BUDGET:
+            break
+        used += size
+        out[k] = [fetch(ai.out_off, ai.out_bytes).view(NP_DTYPES[ai.data_type]).reshape(ai.n_entries, ai.num_components)
+                  for ai in infos]
+    return out
+
+
+def write_outputs(dirname, outputs):
+    """DIR/buf<k>_attr<a>.npy per attribute of sample_outputs(), widened to float32 / float64 without rounding."""
+    os.makedirs(dirname, exist_ok=True)
+    for k, arrays in outputs.items():
+        for a, v in enumerate(arrays):
+            np.save(os.path.join(dirname, "buf%05d_attr%d.npy" % (k, a)), v.astype(widened(v.dtype)))
+
+
 def cpu_oracle_rate(workload, seconds_target=15.0, threads=None):
     """The CPU oracle on a bounded sample of the same workload, one buffer per thread.  Returns points/s etc."""
     from oracle import pyoracle as O  # cpu_baseline / reference arm only
     from draco_sharp_b200 import synth_gen as G
-    from draco_sharp_b200 import build as B
-    B.build_oracle()
     O.lib()
     n_bufs, n_points, kw, _ = WORKLOADS[workload]
     threads = threads or host_cores()
@@ -246,11 +283,9 @@ def run_reference(args, rank, world):
         return
     if args.workload == "c1":
         from oracle import pyoracle as O
-        from draco_sharp_b200 import build as B
-        B.build_oracle()
         buf = np.fromfile(os.path.join(ROOT, "tests", "golden", "house_04.obj.drc"), dtype=np.uint8)
         r = O.decode(buf)
-        steps = max(args.steps, 20)
+        steps = args.steps
         t0 = time.perf_counter()
         for _ in range(steps):
             O.decode(buf)
@@ -295,12 +330,12 @@ def run_reference(args, rank, world):
 
 
 def make_cmp_mesh(side, topo):
-    """One grid mesh with CMP positions and geometric normals (SURVEY 8f-3), written by tests/drc_writer.py; cached under
-    bench_cache/ (git-ignored, travels with the snapshot) because the pure-Python writer needs about a minute per million
+    """One grid mesh with CMP positions and geometric normals (SURVEY 8f-3), written by tests/drc_writer.py; cached in the
+    temporary directory (the tree may be read-only) because the pure-Python writer needs about a minute per million
     vertices.  Returns (buffer, attr_section_off, checksum of the expected position floats, 1, None)."""
     import struct
     from draco_sharp_b200 import synth_gen as G
-    cache = os.path.join(ROOT, "bench_cache", "c4cmp_%d.npz" % side)
+    cache = os.path.join(tempfile.gettempdir(), "draco_sharp_b200_bench_%d" % os.getuid(), "c4cmp_%d.npz" % side)
     if os.path.exists(cache):
         z = np.load(cache)
         return z["buf"], int(z["aoff"]), int(z["sum"]), 1, None
@@ -351,8 +386,6 @@ def make_meshes(name, rank, n_meshes=None):
 def cpu_mesh_rate(name, threads=None):
     """CPU oracle on the mesh workload: one mesh per thread, maps handed over exactly as to the GPU path."""
     from oracle import pyoracle as O  # cpu_baseline / reference arm only
-    from draco_sharp_b200 import build as B
-    B.build_oracle()
     O.lib()
     threads = threads or host_cores()
     topo, meshes, nv = make_meshes(name, 0, n_meshes=threads)
@@ -381,10 +414,7 @@ def run_mesh(args, rank, local_rank, world):
     symbol decode, parallelogram inverse prediction, wrap and dequantisation run on the GPU."""
     import torch
     import draco_sharp_b200 as D
-    from draco_sharp_b200 import build as B
     from draco_sharp_b200 import synth_gen as G
-    if rank == 0 or not os.path.exists(os.path.join(ROOT, "draco_sharp_b200", "libdracob200.so")):
-        B.build_all()
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a B200: the decode path is CUDA only (no CPU fallback)")
     torch.cuda.set_device(local_rank)
@@ -445,6 +475,8 @@ def run_mesh(args, rank, local_rank, world):
     if dist:
         dist.barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, sample_outputs(batch, lambda off, n: d_out[off: off + n].cpu().numpy()))
     ms, (total_points, total_out, total_launches) = reduce_over_ranks(dist, "cuda", ev0.elapsed_time(ev1), [points, out_bytes, launches])
     ms_per_step = ms / args.steps
     stats = dec.stats()
@@ -523,8 +555,6 @@ def run_real_asset(args, rank, local_rank):
     import torch
     import draco_sharp_b200 as D
     from oracle import pyoracle as O  # cpu_baseline only
-    from draco_sharp_b200 import build as B
-    B.build_all()
     buf = np.fromfile(os.path.join(ROOT, "tests", "golden", "house_04.obj.drc"), dtype=np.uint8)
     torch.cuda.set_device(local_rank)
     dec = D.DracoBatchDecoder([local_rank])
@@ -536,13 +566,15 @@ def run_real_asset(args, rank, local_rank):
     for k in range(3):
         assert np.array_equal(np.asarray(d.attributes[k].buffer).view(np.uint8).ravel(), ref.attrs[k].out.view(np.uint8).ravel()), \
             "GPU decode differs from the oracle (attribute %d)" % k
-    steps = max(args.steps, 20)
+    steps = args.steps
     torch.cuda.synchronize()
     t0 = time.perf_counter()
     for _ in range(steps):
-        dec.decode_batch([buf])
+        (d,) = dec.decode_batch([buf])
     ms = (time.perf_counter() - t0) * 1e3 / steps
     st = dec.stats()
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {0: [a.values for a in d.attributes]})
     t0 = time.perf_counter()
     for _ in range(steps):
         O.decode(buf)
@@ -621,10 +653,17 @@ def run_sweep(args, rank, local_rank):
     dec.close()
 
 
+def positive(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be at least 1")
+    return v
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=60)
+    ap.add_argument("--steps", type=positive, default=60, help="timed steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c2", choices=sorted(WORKLOADS) + sorted(MESH_WORKLOADS) + ["c1"])
@@ -635,7 +674,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-copy-ceiling", action="store_true", help="skip the bare pinned-copy leg (e2e.host_ceiling_*)")
     ap.add_argument("--sweep", action="store_true", help="BASELINE configs[4]: points-per-buffer and batch-size sweep (one JSON line per cell)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the decoded attributes of the last step "
+                    "(a fixed sample of the buffers, at most 64 MB; rank 0's batch) as DIR/buf<k>_attr<a>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.sweep):
+        ap.error("--dump-outputs needs the GPU arm of a workload (not --impl reference, not --sweep)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -651,9 +694,6 @@ def main():
 
     import torch
     import draco_sharp_b200 as D
-    from draco_sharp_b200 import build as B
-    if rank == 0 or not os.path.exists(os.path.join(ROOT, "draco_sharp_b200", "libdracob200.so")):
-        B.build_all()
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a B200: the decode path is CUDA only (no CPU fallback)")
     torch.cuda.set_device(local_rank)
@@ -728,6 +768,8 @@ def main():
     if dist:
         dist.barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, sample_outputs(batch, lambda off, n: d_out[off: off + n].cpu().numpy()))
     ms, (total_points, total_out, total_launches) = reduce_over_ranks(dist, "cuda", ev0.elapsed_time(ev1),
                                                                       [points, out_bytes, launches])
     total_launches = int(total_launches)

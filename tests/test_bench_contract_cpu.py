@@ -19,6 +19,7 @@ def test_reference_arm_prints_the_contract_line():
     assert r.returncode == 0, r.stderr[-2000:]
     line = json.loads(r.stdout.strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["higher_is_better"] is True and line["unit"] == "points/s"
+    assert line["steps"] == 2
     for key in ("metric", "value", "n_gpus", "steps", "warmup", "ms_per_step", "scaling", "vs_baseline", "dtype", "data", "config",
                 "cpu_baseline", "e2e", "gpu_launches"):
         assert key in line, key

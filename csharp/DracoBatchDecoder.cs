@@ -70,6 +70,8 @@ public sealed class DracoBatchDecoder : IDisposable
     [DllImport(Lib)] private static extern int dcb_mesh_faces(IntPtr batch, int buf, uint[]? faces, ulong capFaces, out ulong nFaces);
     [DllImport(Lib)] private static extern int dcb_mesh_map(IntPtr batch, int buf, int attrDecoder, int which, uint[]? dst, ulong cap, out ulong n);
     [DllImport(Lib)] private static extern int dcb_index_finish(IntPtr ctx, IntPtr batch);
+    [DllImport(Lib)] private static extern int dcb_set_output_order(IntPtr batch, int order);
+    [DllImport(Lib)] private static extern unsafe int dcb_set_mesh_faces(IntPtr batch, int buf, uint* faces, ulong nFaces);
     [DllImport(Lib)] private static extern unsafe int dcb_decode_scatter(IntPtr ctx, IntPtr batch, byte** outs, int nOuts, uint flags);
     [DllImport(Lib)] private static extern int dcb_status(IntPtr batch, int buf);
     [DllImport(Lib)] private static extern void dcb_batch_free(IntPtr batch);
@@ -96,8 +98,11 @@ public sealed class DracoBatchDecoder : IDisposable
     /// <summary>
     /// Decodes every buffer. A malformed buffer yields a null entry and its exception in <paramref name="errors"/>
     /// (the same exception type DracoDecoder.Decode would have thrown for it); it never poisons its neighbours.
+    /// <paramref name="pointOrder"/>: attributes of Edgebreaker meshes arrive with one value per point (DCB_ORDER_POINTS,
+    /// the point-to-value map applied on the GPU) and carry the identity mapping; otherwise they hold the unique entries
+    /// and <see cref="IHostConnectivity.ApplyPointMapping"/> supplies the map.
     /// </summary>
-    public unsafe Draco?[] DecodeBatch(IReadOnlyList<ReadOnlyMemory<byte>> buffers, out Exception?[] errors)
+    public unsafe Draco?[] DecodeBatch(IReadOnlyList<ReadOnlyMemory<byte>> buffers, out Exception?[] errors, bool pointOrder = false)
     {
         int n = buffers.Count;
         var result = new Draco?[n];
@@ -118,6 +123,7 @@ public sealed class DracoBatchDecoder : IDisposable
                 lens[k] = (ulong)buffers[k].Length;
             }
             Check(dcb_index(_ctx, ptrs, lens, n, out batch));
+            if (pointOrder) Check(dcb_set_output_order(batch, 1));  // DCB_ORDER_POINTS
 
             // meshes: connectivity on the host, maps to the GPU
             var hostMeshes = new Mesh.Mesh?[n];
@@ -159,6 +165,14 @@ public sealed class DracoBatchDecoder : IDisposable
                     }
                     Check(dcb_set_mesh_maps(batch, k, d, Pin(m.Opposite), Pin(m.CornerToVertex), (ulong)m.Opposite.Length,
                         Pin(m.DataToCorner), (ulong)m.DataToCorner.Length, (int*)Pin(m.VertexToData), (ulong)m.VertexToData.Length));
+                }
+                // Edgebreaker meshes only: the library refuses faces for sequential meshes (their attributes are already in point
+                // order).  A hook that exports no faces leaves the buffer to fail alone with DCB_ERR_MAPS.
+                if (pointOrder && bi.EncoderMethod == 1 && hc.Faces != null)  // Mesh.Faces as point ids, borrowed (pinned) like the maps
+                {
+                    var h = GCHandle.Alloc(hc.Faces, GCHandleType.Pinned);
+                    mapPins.Add(h);
+                    Check(dcb_set_mesh_faces(batch, k, (uint*)h.AddrOfPinnedObject(), (ulong)hc.Faces.Length / 3));
                 }
             }
             if (anyMesh) Check(dcb_index_finish(_ctx, batch));
@@ -202,6 +216,16 @@ public sealed class DracoBatchDecoder : IDisposable
                 }
                 PointCloud.PointCloud pc = hostMeshes[k] ?? (bi.GeometryType == 1 ? new Mesh.Mesh() : new PointCloud.PointCloud());
                 pc.PointsCount = (int)bi.NPoints;
+                if (hostMeshes[k] == null && pc is Mesh.Mesh mesh)
+                {
+                    // the library decoded the connectivity: its faces (Mesh.SetFace, MeshEdgeBreakerDecoder.cs:622-636)
+                    Check(dcb_mesh_faces(batch, k, null, 0, out ulong nFaces));
+                    var faces = new uint[nFaces * 3];
+                    Check(dcb_mesh_faces(batch, k, faces, nFaces, out nFaces));
+                    for (int f = 0; f < (int)nFaces; ++f)
+                        mesh.SetFace(f, new[] { (int)faces[3 * f], (int)faces[3 * f + 1], (int)faces[3 * f + 2] });
+                }
+                bool pointRows = pointOrder && bi.GeometryType == 1 && bi.EncoderMethod == 1;
                 var list = new List<PointAttribute>();
                 for (int a = 0; a < bi.NAttrs; ++a)
                 {
@@ -214,8 +238,8 @@ public sealed class DracoBatchDecoder : IDisposable
                     var pa = new PointAttribute(ga);
                     pa.Reset(0);                        // keeps DataType / NumComponents, then:
                     pa.ResetBuffer(buffer, stride, 0);  // ... attach the decoded bytes (GeometryAttribute.cs:55-60)
-                    typeof(PointAttribute).GetProperty(nameof(PointAttribute.UniqueEntriesCount))!.SetValue(pa, ai.NEntries);
-                    if (bi.GeometryType == 0) pa.SetIdentityMapping(); // sequential point clouds: LinearSequencer
+                    typeof(PointAttribute).GetProperty(nameof(PointAttribute.UniqueEntriesCount))!.SetValue(pa, pointRows ? (uint)(ai.OutBytes / (ulong)stride) : ai.NEntries);
+                    if (bi.GeometryType == 0 || pointRows) pa.SetIdentityMapping(); // LinearSequencer / point order: row p is point p
                     else Connectivity?.ApplyPointMapping(k, ai.DecoderId, pa); // MeshTraversalSequencer.UpdatePointToAttributeIndexMapping
                     pc.AddAttribute(pa);
                     list.Add(pa);
@@ -278,6 +302,7 @@ public sealed class HostConnectivity
     public required Mesh.Mesh Mesh { get; init; }
     public required long AttributesSectionOffset { get; init; }             // DecoderBuffer position after DecodeConnectivity
     public required IReadOnlyList<HostDecoderMaps> Decoders { get; init; }  // one per attributes decoder
+    public uint[]? Faces { get; init; }                                      // Mesh.Faces, 3 point ids per face: needed for point order only
 }
 
 public sealed class HostDecoderMaps

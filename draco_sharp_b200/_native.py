@@ -12,6 +12,8 @@ SYNTH_PATH = os.path.join(HERE, "synth", "libdrcsynth.so")
 
 DCB_DUMP_SYMBOLS = 1
 DCB_DUMP_QINTS = 2
+DCB_ORDER_ENTRIES = 0
+DCB_ORDER_POINTS = 1
 
 ERR = {
     0: "DCB_OK", -1: "DCB_ERR_EOF", -2: "DCB_ERR_MAGIC", -3: "DCB_ERR_UNSUPPORTED", -4: "DCB_ERR_SCHEME",
@@ -93,6 +95,8 @@ EXPORTS = [
     ("dcb_mesh_faces", C.c_int, [_P, C.c_int, _P, C.c_uint64, C.POINTER(C.c_uint64)]),
     ("dcb_mesh_map", C.c_int, [_P, C.c_int, C.c_int, C.c_int, _P, C.c_uint64, C.POINTER(C.c_uint64)]),
     ("dcb_index_finish", C.c_int, [_P, _P]),
+    ("dcb_set_output_order", C.c_int, [_P, C.c_int]),
+    ("dcb_set_mesh_faces", C.c_int, [_P, C.c_int, _P, C.c_uint64]),
     ("dcb_decode", C.c_int, [_P, _P, _P, _P, C.c_uint32]),
     ("dcb_decode_scatter", C.c_int, [_P, _P, C.POINTER(_P), C.c_int, C.c_uint32]),
     ("dcb_upload", C.c_int, [_P, _P]),

@@ -115,6 +115,13 @@ struct BufRec {
   std::vector<uint32_t> faces;     // dcb_host_connectivity: 3 point ids per face
   uint64_t conn_off = 0;           // meshes: first byte after header + metadata
   std::vector<uint32_t> dec_entries;
+  // point order (Edgebreaker): faces set by dcb_set_mesh_faces / dcb_host_connectivity -- BORROWED like the maps, or
+  // the NULL form (point ids = corner_to_vertex of decoder 0)
+  const uint32_t *pt_faces = nullptr;
+  uint64_t pt_n_faces = 0;
+  bool pt_faces_set = false;
+  bool pt_failed = false;          // the status is the point-order face check's verdict (undone when indexing reruns)
+  uint64_t faces_dev_off = 0;      // explicit faces inside the shard's maps arena
 };
 
 struct Group {            // one kernel launch (or a few, for global tables)
@@ -163,6 +170,7 @@ struct Shard {
   std::vector<StreamDesc> streams, streams0;
   std::vector<BufWalk> walks, walks0;
   std::vector<uint8_t> tags_launched;
+  PointStage pstage{};         // point order: device job tables (plan_points)
   uint64_t in_bytes = 0, out_bytes = 0, dbg_bytes = 0, aux_bytes = 0, maps_bytes = 0;
   uint64_t out_base = 0, dbg_base = 0;  // offset of this shard inside the batch-wide host arenas
   // device
@@ -182,6 +190,16 @@ struct Shard {
   uint32_t epoch = 0;          // tags the look-back words of par_post2_kernel (30 bits, never 0): no clearing between decodes
   bool uploaded = false, dirty = true, own_out = false;
   uint8_t *ext_out = nullptr, *ext_dbg = nullptr;
+  // output arena layout per stream: where the attribute lands for the caller.  Entry order: the stream's own out_off /
+  // out_bytes.  A point-order shard (pts: it holds an Edgebreaker buffer in DCB_ORDER_POINTS) runs its kernels into an
+  // entry-order staging arena laid out by out_off (stage_bytes, at the front of d_pts) and the point stage fills the
+  // output arena from it.
+  std::vector<uint64_t> fin_off, fin_bytes;
+  bool pts = false;
+  uint64_t stage_bytes = 0;
+  uint8_t *d_pts = nullptr;    // staging | point maps | job tables
+  uint64_t cap_pts = 0;
+  std::vector<uint8_t> pts_tables;  // host copy of the job tables (source of the asynchronous upload)
 };
 
 }  // namespace
@@ -224,6 +242,8 @@ struct dcb_batch {
   uint64_t total_out = 0, total_dbg = 0, total_in = 0, total_points = 0, algo_bytes = 0;
   int n_devices = 1;
   uint64_t max_points = 0, points_per_byte = 0;  // plausibility limits (dcb_set_limits), copied from the context
+  int order = DCB_ORDER_ENTRIES;
+  bool conn_done = false;  // dcb_index_finish has run: a new order or new faces rerun it
 };
 
 namespace {
@@ -352,6 +372,22 @@ void check_plausible(const dcb_batch &b, BufRec &r) {
   if (r.info.status == DCB_OK && implausible(b, r.info.n_points, r.len)) r.info.status = DCB_ERR_ATTR;
 }
 
+// bytes of one value (StoreTypedValues; normals: three float32)
+uint64_t row_bytes(const StreamDesc &s) {
+  return (s.seq_type == SEQ_NORMALS) ? 12ull : (uint64_t)dcb_dtype_len(s.data_type) * s.nc;
+}
+
+// Point order walks the faces over the corners of every attributes decoder of an Edgebreaker buffer: they must be set
+// and have the corner count of each decoder (whose maps the indexer has checked are there).
+bool point_faces_ok(const BufRec &b, int n_dec) {
+  if (!b.pt_faces_set) return false;
+  if (n_dec <= 0) return true;
+  const uint64_t n_face_corners = b.pt_faces ? 3 * b.pt_n_faces : b.maps[0].n_corners;
+  for (int d = 0; d < n_dec; ++d)
+    if (b.maps[d].n_corners != n_face_corners) return false;
+  return true;
+}
+
 // DEC_ID + DEC_DATA: creates the StreamDescs of one buffer (appended to sh.streams) and its BufWalk.
 void parse_attr_section(BufRec &b, Shard &sh, int buf_index, const dcb_batch *batch = nullptr) {
   dcb_buffer_info &inf = b.info;
@@ -438,8 +474,13 @@ void parse_attr_section(BufRec &b, Shard &sh, int buf_index, const dcb_batch *ba
         s.n_corners = (uint32_t)b.maps[d].n_corners;
         s.n_vertices = (uint32_t)b.maps[d].n_vertices;
       }
-      const uint64_t esz = (s.seq_type == SEQ_NORMALS) ? 12ull : (uint64_t)dcb_dtype_len(s.data_type) * s.nc;
-      s.out_bytes = esz * n_entries;
+      s.out_bytes = row_bytes(s) * n_entries;
+    }
+  }
+  if (b.is_eb && batch && batch->order == DCB_ORDER_POINTS && n_dec > 0) {
+    if (!point_faces_ok(b, n_dec)) {
+      b.pt_failed = true;
+      return finish(DCB_ERR_MAPS);
     }
   }
   w.pos = b.arena_off + r.pos;
@@ -561,6 +602,8 @@ void free_shard_device(Shard &sh) {
   pool_free(sh.pool, sh.device, sh.d_streams, sh.cap_streams);
   pool_free(sh.pool, sh.device, sh.d_walks, sh.cap_walks);
   pool_free(sh.pool, sh.device, sh.d_order, sh.cap_order);
+  pool_free(sh.pool, sh.device, sh.d_pts, sh.cap_pts);
+  sh.d_pts = nullptr;
   if (sh.h_stage) pinned_free(sh.pool, sh.h_stage, sh.cap_stage);
   if (sh.h_maps) pinned_free(sh.pool, sh.h_maps, sh.cap_hmaps);
   sh.h_maps = nullptr;
@@ -743,6 +786,43 @@ int make_batch(dcb_ctx *ctx, const uint8_t *arena, const uint8_t *const *ptrs, c
   return DCB_OK;
 }
 
+// The caller's view of the output arena.  Entry order: the kernels' layout.  Point order: a shard holding an indexed
+// Edgebreaker buffer stages the kernels' entry-order layout (stage_bytes) and lays the output arena out again with
+// n_points rows for the attributes of its Edgebreaker buffers; every attribute keeps its place in (buffer, attribute)
+// order on a 128-byte boundary.
+void layout_points(const dcb_batch *b, Shard &sh) {
+  const size_t n = sh.streams.size();
+  sh.fin_off.resize(n);
+  sh.fin_bytes.resize(n);
+  sh.pts = false;
+  sh.stage_bytes = 0;
+  if (b->order == DCB_ORDER_POINTS)
+    for (size_t bi = 0; bi < sh.walks.size(); ++bi)
+      sh.pts = sh.pts || (b->bufs[sh.bufs[bi]].is_eb && sh.walks[bi].status == DCB_OK && sh.walks[bi].stream_count > 0);
+  if (!sh.pts) {
+    for (size_t i = 0; i < n; ++i) {
+      sh.fin_off[i] = sh.streams[i].out_off;
+      sh.fin_bytes[i] = sh.streams[i].out_bytes;
+    }
+    return;
+  }
+  sh.stage_bytes = sh.out_bytes;
+  uint64_t out = 0;
+  for (size_t bi = 0; bi < sh.walks.size(); ++bi) {
+    const BufWalk &w = sh.walks[bi];
+    const BufRec &r = b->bufs[sh.bufs[bi]];
+    for (int i = 0; i < w.stream_count; ++i) {
+      const size_t si = (size_t)w.stream_first + i;
+      const StreamDesc &s = sh.streams[si];
+      const uint64_t rows = r.is_eb ? r.info.n_points : s.n_entries;
+      sh.fin_off[si] = out;
+      sh.fin_bytes[si] = w.status ? 0 : rows * row_bytes(s);
+      out = align_up(out + sh.fin_bytes[si], 128);
+    }
+  }
+  sh.out_bytes = out;
+}
+
 void finalize_layout(dcb_batch *b) {
   uint64_t out_base = 0, dbg_base = 0;
   b->total_in = 0;
@@ -750,6 +830,7 @@ void finalize_layout(dcb_batch *b) {
   b->algo_bytes = 0;
   for (Shard &sh : b->shards) {
     layout_shard(sh);
+    layout_points(b, sh);
     sh.out_base = out_base;
     sh.dbg_base = dbg_base;
     out_base += align_up(sh.out_bytes, 128);
@@ -1059,6 +1140,11 @@ int issue_arena_copy(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index) {
   return DCB_OK;
 }
 
+// point order: the explicit faces of an indexed Edgebreaker buffer travel with its maps (the NULL form reads the maps)
+bool uploads_faces(const Shard &sh, const BufRec &r) {
+  return sh.pts && r.is_eb && r.pt_faces && sh.walks0[r.local].status == DCB_OK;
+}
+
 // Mesh connectivity maps (56 bytes per vertex, read by para_deps_kernel only): on the device's upload stream, issued
 // BEHIND the first rANS launch of the decode so that the copy hides behind the symbol chains; `st` then waits for it.
 // From pageable memory cudaMemcpyAsync stages through the driver and holds the calling thread, not the GPU.
@@ -1091,6 +1177,10 @@ int issue_maps_copy(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index) {
                 for (uint64_t o = 0; o < sz[j]; o += kPiece)
                   pieces.push_back({(const uint8_t *)src[j] + o, m.dev_off[j] + o, std::min(kPiece, sz[j] - o)});
             }
+        for (int k : sh.bufs)
+          if (const BufRec &r = b->bufs[k]; uploads_faces(sh, r))
+            for (uint64_t o = 0; o < r.pt_n_faces * 12; o += kPiece)
+              pieces.push_back({(const uint8_t *)r.pt_faces + o, r.faces_dev_off + o, std::min(kPiece, r.pt_n_faces * 12 - o)});
         std::unique_ptr<std::atomic<uint8_t>[]> done(new std::atomic<uint8_t>[pieces.size()]);
         for (size_t i = 0; i < pieces.size(); ++i) done[i].store(0, std::memory_order_relaxed);
         std::atomic<size_t> next{0};
@@ -1135,9 +1225,96 @@ int issue_maps_copy(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index) {
         if (m.n_entries) CUDA_TRY(cudaMemcpyAsync(sh.d_maps + m.dev_off[2], m.data_to_corner, m.n_entries * 4, cudaMemcpyHostToDevice, cs));
         if (m.n_vertices) CUDA_TRY(cudaMemcpyAsync(sh.d_maps + m.dev_off[3], m.vertex_to_data, m.n_vertices * 4, cudaMemcpyHostToDevice, cs));
       }
+  if (!staged)
+    for (int k : sh.bufs)
+      if (const BufRec &r = b->bufs[k]; uploads_faces(sh, r) && r.pt_n_faces)
+        CUDA_TRY(cudaMemcpyAsync(sh.d_maps + r.faces_dev_off, r.pt_faces, r.pt_n_faces * 12, cudaMemcpyHostToDevice, cs));
   tl_mark(ctx, "", cs, false);
   CUDA_TRY(cudaEventRecord(ctx->maps_ev[dev_index], cs));
   CUDA_TRY(cudaStreamWaitEvent(st, ctx->maps_ev[dev_index], 0));
+  return DCB_OK;
+}
+
+// Point order: the job tables of the point stage (dcb_points.cu) -- one map per (Edgebreaker buffer, attributes decoder)
+// with attributes, one gather per attribute (identity rows for point clouds and sequential meshes sharing the shard) --
+// and the shard's arena for them: entry-order staging | point maps (u32 per point and decoder) | tables.
+int plan_points(dcb_batch *b, Shard &sh, cudaStream_t st) {
+  std::vector<PointMapJob> mj;
+  std::vector<PointGatherJob> gj;
+  std::vector<uint64_t> cpre{0}, ppre{0}, upre{0};
+  for (size_t bi = 0; bi < sh.walks0.size(); ++bi) {
+    const BufWalk &w = sh.walks0[bi];
+    const BufRec &r = b->bufs[sh.bufs[bi]];
+    if (w.status != DCB_OK) continue;
+    std::vector<uint64_t> dec_map(r.is_eb ? r.maps.size() : 0, ~0ull);
+    for (int i = 0; i < w.stream_count; ++i) {
+      const uint32_t si = (uint32_t)(w.stream_first + i);
+      const StreamDesc &s = sh.streams0[si];
+      if (sh.fin_bytes[si] == 0) continue;
+      uint64_t map_off = ~0ull;
+      if (r.is_eb) {
+        const MeshMapsHost &m = r.maps[s.decoder_id];
+        if (dec_map[s.decoder_id] == ~0ull) {
+          PointMapJob j{};
+          j.faces_off = r.pt_faces ? r.faces_dev_off : r.maps[0].dev_off[1];
+          j.c2v_off = m.dev_off[1];
+          j.v2d_off = m.dev_off[3];
+          j.map_off = ppre.back();
+          j.n_corners = (uint32_t)m.n_corners;
+          j.n_points = r.info.n_points;
+          j.n_vertices = (uint32_t)m.n_vertices;
+          j.n_entries = (uint32_t)m.n_entries;
+          j.status_si = (uint32_t)w.stream_first;
+          dec_map[s.decoder_id] = j.map_off;
+          mj.push_back(j);
+          cpre.push_back(cpre.back() + m.n_corners);
+          ppre.push_back(ppre.back() + r.info.n_points);
+        }
+        map_off = dec_map[s.decoder_id];
+      }
+      PointGatherJob g{};
+      g.src_off = s.out_off;
+      g.dst_off = sh.fin_off[si];
+      g.map_off = map_off;
+      g.row_bytes = (uint32_t)row_bytes(s);
+      g.rows = (uint32_t)(sh.fin_bytes[si] / g.row_bytes);
+      g.st_first = (uint32_t)w.stream_first;
+      g.st_count = (uint32_t)w.stream_count;
+      while (g.vec_shift < 4 && g.row_bytes % (2u << g.vec_shift) == 0) ++g.vec_shift;
+      gj.push_back(g);
+      upre.push_back(upre.back() + (uint64_t)g.rows * (g.row_bytes >> g.vec_shift));
+    }
+  }
+  const uint64_t off_pmap = align_up(sh.stage_bytes, 256);
+  const uint64_t off_mj = align_up(off_pmap + 4 * ppre.back(), 256);
+  const uint64_t off_cpre = align_up(off_mj + mj.size() * sizeof(PointMapJob), 16);
+  const uint64_t off_ppre = align_up(off_cpre + cpre.size() * 8, 16);
+  const uint64_t off_gj = align_up(off_ppre + ppre.size() * 8, 16);
+  const uint64_t off_upre = align_up(off_gj + gj.size() * sizeof(PointGatherJob), 16);
+  const uint64_t total = off_upre + upre.size() * 8;
+  CUDA_TRY(pool_alloc(sh.pool, sh.device, total, &sh.d_pts, &sh.cap_pts));
+  std::vector<uint8_t> &t = sh.pts_tables;  // outlives the asynchronous upload
+  t.assign(total - off_mj, 0);
+  auto put = [&](uint64_t off, const void *src, uint64_t n) { if (n) memcpy(t.data() + (off - off_mj), src, n); };
+  put(off_mj, mj.data(), mj.size() * sizeof(PointMapJob));
+  put(off_cpre, cpre.data(), cpre.size() * 8);
+  put(off_ppre, ppre.data(), ppre.size() * 8);
+  put(off_gj, gj.data(), gj.size() * sizeof(PointGatherJob));
+  put(off_upre, upre.data(), upre.size() * 8);
+  CUDA_TRY(cudaMemcpyAsync(sh.d_pts + off_mj, t.data(), t.size(), cudaMemcpyHostToDevice, st));
+  PointStage &p = sh.pstage;
+  p.maps = reinterpret_cast<const PointMapJob *>(sh.d_pts + off_mj);
+  p.corner_prefix = reinterpret_cast<const uint64_t *>(sh.d_pts + off_cpre);
+  p.point_prefix = reinterpret_cast<const uint64_t *>(sh.d_pts + off_ppre);
+  p.n_maps = (uint32_t)mj.size();
+  p.gathers = reinterpret_cast<const PointGatherJob *>(sh.d_pts + off_gj);
+  p.unit_prefix = reinterpret_cast<const uint64_t *>(sh.d_pts + off_upre);
+  p.n_gathers = (uint32_t)gj.size();
+  p.pmap = reinterpret_cast<uint32_t *>(sh.d_pts + off_pmap);
+  p.pmap_words = ppre.back();
+  p.total_corners = cpre.back();
+  p.total_units = upre.back();
+  p.stage = sh.d_pts;
   return DCB_OK;
 }
 
@@ -1171,6 +1348,11 @@ int upload_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index) {
           mbytes = align_up(mbytes + sz[j] * 4, 16);
         }
       }
+  for (int k : sh.bufs)  // point order: explicit faces travel with the maps
+    if (BufRec &r = b->bufs[k]; uploads_faces(sh, r)) {
+      r.faces_dev_off = mbytes;
+      mbytes = align_up(mbytes + r.pt_n_faces * 12, 16);
+    }
   sh.maps_bytes = mbytes;
   if (mbytes) {
     CUDA_TRY(pool_alloc(sh.pool, sh.device, mbytes, &sh.d_maps, &sh.cap_maps));
@@ -1209,6 +1391,10 @@ int upload_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index) {
   if (sh.aux_bytes) {
     CUDA_TRY(pool_alloc(sh.pool, sh.device, sh.aux_bytes, &sh.d_aux, &sh.cap_aux));
     CUDA_TRY(cudaMemsetAsync(sh.d_aux, 0, sh.aux_bytes, st));  // look-back words start with epoch 0 (never a live epoch)
+  }
+  if (sh.pts) {
+    int rc = plan_points(b, sh, st);
+    if (rc) return rc;
   }
   sh.uploaded = true;
   sh.dirty = true;
@@ -1268,7 +1454,8 @@ int decode_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index, uint8_t *
     sh.dirty = false;
   }
   sh.tags_launched.assign(sh.streams.size(), 0);
-  DevArenas A{sh.d_in, d_out, d_dbg, sh.d_aux, sh.d_tab, sh.d_maps};
+  // point order: the kernels write the entry-order staging, the point stage fills d_out from it
+  DevArenas A{sh.d_in, sh.pts ? sh.d_pts : d_out, d_dbg, sh.d_aux, sh.d_tab, sh.d_maps};
   const uint32_t dump = flags & (DCB_DUMP_SYMBOLS | DCB_DUMP_QINTS);
   const bool dbg_tl = timed && sh.device == ctx->devices[0] && env_flags().debug_timing;
   auto tl_begin = [&](const char *name, cudaStream_t s) {
@@ -1281,6 +1468,19 @@ int decode_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index, uint8_t *
   };
   auto tl_end = [&](cudaStream_t s) {
     if (dbg_tl) cudaEventRecord(ctx->timeline.back().second.second, s);
+  };
+  // last writer of every attribute: behind the joins, on the main stream
+  auto point_stage = [&]() -> int {
+    if (!sh.pts) return DCB_OK;
+    int rc = issue_maps_copy(ctx, b, sh, dev_index);
+    if (rc) return rc;
+    DevArenas P = A;
+    P.out = d_out;
+    tl_begin("point stage", st);
+    CUDA_TRY(dcb_launch_point_stage(sh.pstage, sh.d_streams, P, num_sms, st));
+    tl_end(st);
+    stats.n_launches += 3;
+    return DCB_OK;
   };
   if (timed && dev_index == 0) CUDA_TRY(cudaEventRecord(ctx->ev[0], st));
 
@@ -1619,8 +1819,10 @@ int decode_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index, uint8_t *
   }
 
   if (n_order == 0) {
+    int rc = point_stage();
+    if (rc) return rc;
     if (timed && dev_index == 0) CUDA_TRY(cudaEventRecord(ctx->ev[1], st));
-    if (deferred_descs) return queue_desc_copyback(ctx, sh, st);
+    if (deferred_descs || sh.pts) return queue_desc_copyback(ctx, sh, st);
     return DCB_OK;
   }
   {
@@ -1877,10 +2079,15 @@ int decode_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index, uint8_t *
     CUDA_TRY(cudaEventRecord(ctx->ev[9], st));
     ctx->ev_para = true;
   }
+  {
+    int rc = point_stage();
+    if (rc) return rc;
+  }
   if (timed && dev_index == 0) CUDA_TRY(cudaEventRecord(ctx->ev[1], st));
-  if (has_para || deferred_descs) {
-    // parallelogram kernels validate the caller's maps on the device, resumed walks parse and validate on the device:
-    // their verdicts travel back behind the kernels and are folded in after the caller's synchronisation
+  if (has_para || deferred_descs || sh.pts) {
+    // parallelogram kernels and the point stage validate the caller's maps on the device, resumed walks parse and
+    // validate on the device: their verdicts travel back behind the kernels and are folded in after the caller's
+    // synchronisation
     int rc = queue_desc_copyback(ctx, sh, st);
     if (rc) return rc;
   }
@@ -1943,17 +2150,19 @@ int decode_all_impl(dcb_ctx *ctx, dcb_batch *b, void *dev_out, void *dev_dbg, ui
 
 // An error in the middle of a batch must not leave kernels or copies of the shards launched so far in flight: the
 // caller frees the batch next, and its arenas go back to the context's cache.
+void drain(dcb_ctx *ctx) {
+  (void)sync_all(ctx);
+  for (size_t d = 0; d < ctx->devices.size(); ++d) {  // side and copy streams too
+    cudaSetDevice(ctx->devices[d]);
+    cudaDeviceSynchronize();
+  }
+  cudaGetLastError();
+}
+
 int decode_all(dcb_ctx *ctx, dcb_batch *b, void *dev_out, void *dev_dbg, uint32_t flags, uint8_t *host_out = nullptr,
                uint8_t *host_dbg = nullptr) {
   const int rc = decode_all_impl(ctx, b, dev_out, dev_dbg, flags, host_out, host_dbg);
-  if (rc != DCB_OK && ctx) {
-    (void)sync_all(ctx);
-    for (size_t d = 0; d < ctx->devices.size(); ++d) {  // side and copy streams too
-      cudaSetDevice(ctx->devices[d]);
-      cudaDeviceSynchronize();
-    }
-    cudaGetLastError();
-  }
+  if (rc != DCB_OK && ctx) drain(ctx);
   return rc;
 }
 
@@ -2349,8 +2558,8 @@ int dcb_get_attr_info(const dcb_batch *b, int buf, int attr, dcb_attr_info *out)
     out->scheme = (s.scheme == SCHEME_TAGGED || s.scheme == SCHEME_RAW) ? (int32_t)s.scheme : -1;
     out->precision_bits = s.prec_bits;
     out->n_entries = s.n_entries;
-    out->out_bytes = s.out_bytes;
-    out->out_off = sh.out_base + s.out_off;
+    out->out_bytes = sh.fin_bytes[w.stream_first + attr];
+    out->out_off = sh.out_base + sh.fin_off[w.stream_first + attr];
     out->dbg_off = sh.dbg_base + s.dbg_off;
     out->xf_a = s.xf_a;
     out->xf_b = s.xf_b;
@@ -2466,6 +2675,16 @@ int dcb_host_connectivity(dcb_batch *b, int buf) {
       m.n_vertices = m.own->vertex_to_data.size();
       m.set = true;
     }
+    // point order: the faces just decoded; when they are the corner table of decoder 0 (no attribute seams:
+    // AssignPointsToCorners without attribute data) the NULL form gives the same map and uploads nothing
+    r.pt_faces_set = true;
+    r.pt_faces = nullptr;
+    r.pt_n_faces = 0;
+    if (r.maps.empty() || r.maps[0].n_corners != r.faces.size() ||
+        memcmp(r.maps[0].corner_to_vertex, r.faces.data(), r.faces.size() * 4) != 0) {
+      r.pt_faces = r.faces.data();
+      r.pt_n_faces = r.faces.size() / 3;
+    }
     return DCB_OK;
   });
 }
@@ -2513,6 +2732,10 @@ int dcb_index_finish(dcb_ctx *ctx, dcb_batch *b) {
     }
     for (size_t k = 0; k < b->bufs.size(); ++k) {
       BufRec &r = b->bufs[k];
+      if (r.pt_failed) {  // the face check runs again for the batch's current order and faces
+        r.info.status = DCB_OK;
+        r.pt_failed = false;
+      }
       if (r.info.needs_connectivity && r.info.status == DCB_OK) {
         if (r.info.attr_section_off == 0) r.info.status = DCB_ERR_CONNECTIVITY;
         r.info.needs_connectivity = 0;
@@ -2521,6 +2744,39 @@ int dcb_index_finish(dcb_ctx *ctx, dcb_batch *b) {
     parse_attr_section(r, b->shards[r.shard], (int)k, b);
     }
     finalize_layout(b);
+    b->conn_done = true;
+    return DCB_OK;
+  });
+}
+
+int dcb_set_output_order(dcb_batch *b, int order) {
+  return guarded([&]() -> int {
+    if (!b || (order != DCB_ORDER_ENTRIES && order != DCB_ORDER_POINTS)) return DCB_ERR_ARG;
+    for (const Shard &sh : b->shards)
+      if (sh.uploaded) return DCB_ERR_STATE;
+    if (order == b->order) return DCB_OK;
+    b->order = order;
+    if (b->conn_done) return dcb_index_finish(nullptr, b);
+    finalize_layout(b);
+    return DCB_OK;
+  });
+}
+
+int dcb_set_mesh_faces(dcb_batch *b, int buf, const uint32_t *faces, uint64_t n_faces) {
+  return guarded([&]() -> int {
+    if (!b || buf < 0 || buf >= (int)b->bufs.size()) return DCB_ERR_ARG;
+    if ((!faces && n_faces) || n_faces > 0xFFFFFFFFull / 3) return DCB_ERR_ARG;
+    BufRec &r = b->bufs[buf];
+    if (!r.is_eb) return DCB_ERR_STATE;
+    for (const Shard &sh : b->shards)
+      if (sh.uploaded) return DCB_ERR_STATE;
+    r.pt_faces = faces;
+    r.pt_n_faces = n_faces;
+    r.pt_faces_set = true;
+    // after dcb_index_finish: re-index only when the buffer's verdict flips (the layout follows the statuses alone)
+    if (b->conn_done && b->order == DCB_ORDER_POINTS && !r.info.needs_connectivity && (r.info.status == DCB_OK || r.pt_failed) &&
+        point_faces_ok(r, r.info.n_attr_decoders) == r.pt_failed)
+      return dcb_index_finish(nullptr, b);
     return DCB_OK;
   });
 }
@@ -2532,11 +2788,12 @@ int dcb_upload(dcb_ctx *ctx, dcb_batch *b) {
       if (r.info.needs_connectivity && r.info.status == DCB_OK) return DCB_ERR_STATE;
     for (int d = 0; d < b->n_devices; ++d) {
       int rc = upload_shard(ctx, b, b->shards[d], d);
-      if (rc) return rc;
-      rc = issue_arena_copy(ctx, b, b->shards[d], d);
-      if (rc) return rc;
-      rc = issue_maps_copy(ctx, b, b->shards[d], d);
-      if (rc) return rc;
+      if (!rc) rc = issue_arena_copy(ctx, b, b->shards[d], d);
+      if (!rc) rc = issue_maps_copy(ctx, b, b->shards[d], d);
+      if (rc) {  // copies and memsets of this and earlier shards may be in flight: nothing may outlive the call
+        drain(ctx);
+        return rc;
+      }
     }
     return sync_all(ctx);
   });
@@ -2599,9 +2856,10 @@ int dcb_decode_scatter(dcb_ctx *ctx, dcb_batch *b, uint8_t *const *outs, int n_o
       CUDA_TRY(cudaSetDevice(sh.device));
       for (int i = 0; i < w.stream_count; ++i, ++k) {
         if (k >= n_outs) break;
-        const StreamDesc &s = sh.streams[w.stream_first + i];
-        if (outs[k] && s.out_bytes && r.info.status == DCB_OK && w.status == DCB_OK)
-          CUDA_TRY(cudaMemcpyAsync(outs[k], sh.ext_out + s.out_off, s.out_bytes, cudaMemcpyDeviceToHost, ctx->streams[r.shard]));
+        const size_t si = (size_t)w.stream_first + i;
+        if (outs[k] && sh.fin_bytes[si] && r.info.status == DCB_OK && w.status == DCB_OK)
+          CUDA_TRY(cudaMemcpyAsync(outs[k], sh.ext_out + sh.fin_off[si], sh.fin_bytes[si], cudaMemcpyDeviceToHost,
+                                   ctx->streams[r.shard]));
       }
     }
     rc = sync_all(ctx);

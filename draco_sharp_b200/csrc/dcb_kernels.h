@@ -92,3 +92,41 @@ cudaError_t dcb_launch_oct_unit(StreamDesc *d_streams, const uint32_t *d_order, 
                                 const DevArenas &a, cudaStream_t st);
 cudaError_t dcb_launch_copy(StreamDesc *d_streams, const uint32_t *d_order, uint32_t n, uint64_t max_bytes,
                             const DevArenas &a, cudaStream_t st);
+
+// ---- point order (DCB_ORDER_POINTS, dcb_points.cu) ----
+// MeshTraversalSequencer.UpdatePointToAttributeIndexMapping: for each corner c of attributes decoder d,
+// map_d[faces[c]] = vertex_to_data_d[corner_to_vertex_d[c]]; the last corner of a point wins.
+#define DCB_POINT_NONE 0xFFFFFFFFu  // map value of a point no corner references: its rows are zero
+struct PointMapJob {               // one (Edgebreaker buffer, attributes decoder)
+  uint64_t faces_off;              // maps arena: point id per corner (explicit faces, or corner_to_vertex of decoder 0)
+  uint64_t c2v_off, v2d_off;       // maps arena: the decoder's corner_to_vertex and vertex_to_data
+  uint64_t map_off;                // point-map region, in u32: winning corner + 1, then the entry of each point
+  uint32_t n_corners, n_points, n_vertices, n_entries;
+  uint32_t status_si;              // stream that carries the buffer's DCB_ERR_MAPS
+  uint32_t pad_;
+};
+struct PointGatherJob {            // one attribute of a point-order shard
+  uint64_t src_off;                // entry-order staging
+  uint64_t dst_off;                // output arena
+  uint64_t map_off;                // point-map region (u32), ~0ull: identity rows (point clouds, sequential meshes)
+  uint32_t rows, row_bytes;
+  uint32_t st_first, st_count;     // the buffer's streams: a buffer with a failed stream is not gathered
+  uint32_t vec_shift;              // log2 of the copy unit (16, 8, 4, 2 or 1 bytes; divides row_bytes)
+  uint32_t pad_;
+};
+struct PointStage {
+  const PointMapJob *maps;         // n_maps jobs; corner_prefix / point_prefix: n_maps + 1 running sums
+  const uint64_t *corner_prefix, *point_prefix;
+  uint32_t n_maps;
+  const PointGatherJob *gathers;   // n_gathers jobs; unit_prefix: n_gathers + 1 running sums of rows * units per row
+  const uint64_t *unit_prefix;
+  uint32_t n_gathers;
+  uint32_t *pmap;                  // point-map region (zeroed by the launcher before the corner pass)
+  uint64_t pmap_words;             // = point_prefix[n_maps]
+  uint64_t total_corners, total_units;  // = corner_prefix[n_maps], unit_prefix[n_gathers] (grid sizes)
+  const uint8_t *stage;            // entry-order outputs of the shard's kernels
+};
+// point_win_kernel (one thread per corner) | point_resolve_kernel (one thread per point) | point_gather_kernel (one thread
+// per copy unit of every row of every attribute), on `st`
+cudaError_t dcb_launch_point_stage(const PointStage &p, StreamDesc *d_streams, const DevArenas &a, uint32_t num_sms,
+                                   cudaStream_t st);

@@ -43,11 +43,17 @@ class PointAttribute:  # src/Draco/IO/Attributes/PointAttribute.cs + GeometryAtt
     unique_entries_count: int
     buffer: np.ndarray            # uint8 view of the attribute bytes (DataBuffer)
     info: N.AttrInfo = None
+    point_ordered: bool = False   # rows are points (DCB_ORDER_POINTS on an Edgebreaker mesh), not unique entries
+
+    @property
+    def rows(self):
+        return self.buffer.size // self.byte_stride if self.byte_stride else 0
 
     @property
     def values(self):
+        """(rows, num_components): unique entries in entry order, or one row per point when point_ordered."""
         dt = NP_DTYPES[self.data_type]
-        return self.buffer.view(dt).reshape(self.unique_entries_count, self.num_components)
+        return self.buffer.view(dt).reshape(self.rows, self.num_components)
 
 
 @dataclass
@@ -77,6 +83,7 @@ class Batch:
         self.h = handle
         self.n_bufs = n_bufs
         self._keep = keep  # input buffers must outlive upload
+        self.point_order = False
 
     def free(self):
         if self.h:
@@ -136,6 +143,25 @@ class Batch:
         self._borrowed[(k, dec)] = (o, c, d, v)
         N.check(N.lib().dcb_set_mesh_maps(self.h, k, dec, o.ctypes.data, c.ctypes.data, o.size, d.ctypes.data, d.size,
                                           v.ctypes.data, v.size))
+
+    def set_output_order(self, points: bool):
+        """DCB_ORDER_POINTS (points=True): attributes of Edgebreaker meshes come out as one row per point."""
+        N.check(N.lib().dcb_set_output_order(self.h, N.DCB_ORDER_POINTS if points else N.DCB_ORDER_ENTRIES))
+        self.point_order = bool(points)
+
+    def set_mesh_faces(self, k, faces):
+        """Faces (point ids) of Edgebreaker buffer k for point order; None: the NULL form (faces = corner_to_vertex
+        of attributes decoder 0).  Borrowed by the library like the maps: kept alive with the batch."""
+        self._borrowed = getattr(self, "_borrowed", {})
+        if faces is None:
+            self._borrowed[(k, "faces")] = None
+            N.check(N.lib().dcb_set_mesh_faces(self.h, k, None, 0))
+            return
+        f = np.ascontiguousarray(faces, dtype=np.uint32).reshape(-1)
+        if f.size % 3:
+            raise ValueError("faces: 3 point ids per face")
+        self._borrowed[(k, "faces")] = f
+        N.check(N.lib().dcb_set_mesh_faces(self.h, k, f.ctypes.data if f.size else None, f.size // 3))
 
     def host_connectivity(self, k):
         """Decode the Edgebreaker connectivity of mesh buffer k on the host (dcb_host_connectivity)."""
@@ -249,11 +275,14 @@ class DracoBatchDecoder:
         return s
 
     # ---- the reference-shaped API ----
-    def decode_batch(self, buffers: Sequence) -> List[Draco]:
+    def decode_batch(self, buffers: Sequence, point_order: bool = False) -> List[Draco]:
         """DecodeBatch: one `Draco` per input buffer; a malformed buffer carries its status and no
-        attributes (the reference would have thrown for that buffer alone)."""
+        attributes (the reference would have thrown for that buffer alone).  point_order: attributes of
+        Edgebreaker meshes hold one row per point, so that `values[faces]` is the mesh's triangle soup."""
         batch = self.index(buffers)
         try:
+            if point_order:
+                batch.set_output_order(True)
             meshes = [k for k in range(batch.n_bufs) if batch.buffer_info(k).needs_connectivity]
             for k in meshes:
                 batch.host_connectivity(k)  # connectivity stays on the host (SURVEY 8f-1)
@@ -278,9 +307,10 @@ class DracoBatchDecoder:
             if bi.status == 0:
                 for a in range(bi.n_attrs):
                     ai = batch.attr_info(k, a)
-                    stride = ai.out_bytes // ai.n_entries if ai.n_entries else 0
+                    stride = ai.num_components * np.dtype(NP_DTYPES[ai.data_type]).itemsize
                     buf = out[ai.out_off: ai.out_off + ai.out_bytes]
+                    pts = batch.point_order and bi.geometry_type == 1 and bi.encoder_method == 1
                     d.attributes.append(PointAttribute(ai.att_type, ai.data_type, ai.num_components, bool(ai.normalized),
-                                                       ai.unique_id, stride, ai.n_entries, buf, ai))
+                                                       ai.unique_id, stride, ai.n_entries, buf, ai, pts))
             res.append(d)
         return res

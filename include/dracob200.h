@@ -103,7 +103,8 @@ typedef struct dcb_attr_info {
   int32_t scheme;         /* 0 tagged 1 raw -1 n/a */
   int32_t precision_bits;
   uint32_t n_entries;     /* UniqueEntriesCount */
-  uint64_t out_bytes;     /* n_entries * num_components * sizeof(data_type) */
+  uint64_t out_bytes;     /* rows * num_components * sizeof(data_type); rows = n_entries, or n_points for Edgebreaker
+                             meshes in DCB_ORDER_POINTS */
   uint64_t out_off;       /* offset of this attribute inside the batch output arena (128-byte aligned) */
   uint64_t dbg_off;       /* offset inside the debug arena (int32 per portable value), if requested */
   int32_t xf_a, xf_b;     /* wrap min/max or oct max_quantized_value/center_value */
@@ -178,6 +179,33 @@ int dcb_mesh_faces(const dcb_batch *b, int buf, uint32_t *faces, uint64_t cap_fa
 int dcb_mesh_map(const dcb_batch *b, int buf, int attr_decoder, int which, uint32_t *dst, uint64_t cap, uint64_t *n);
 /* Re-run the attribute indexing of mesh buffers once their maps are set. */
 int dcb_index_finish(dcb_ctx *ctx, dcb_batch *b);
+
+/* Output order of a batch.
+ *   DCB_ORDER_ENTRIES (default): every attribute holds its unique values in entry order -- the order the encoder's
+ *       traversal visited them (n_entries rows, PointAttribute with a point-to-value map in the reference).
+ *   DCB_ORDER_POINTS: every attribute of an Edgebreaker mesh holds n_points rows, row p being the value of the entry
+ *       the reference maps point p to (MeshTraversalSequencer.UpdatePointToAttributeIndexMapping,
+ *       MeshTraversalSequencer.cs:33-51): for each attributes decoder d, for each corner c in increasing order,
+ *           p = faces[c]; v = corner_to_vertex_d[c]; e = vertex_to_data_d[v]; map_d[p] = e
+ *       The last corner of a point wins.  p >= n_points, v >= the decoder's vertex count or e outside [0, n_entries)
+ *       fail that buffer alone with DCB_ERR_MAPS; a point no corner references gets zero bytes.  Each attribute uses
+ *       the maps of its own decoder.  The gather runs on the GPU.  Point clouds and sequential meshes map points to
+ *       entries one to one: their bytes are the same in both orders.  The debug arena (DCB_DUMP_*) stays in entry order.
+ * dcb_attr_info.out_off / out_bytes describe what lands in the output arena, so rows = out_bytes / (num_components *
+ * sizeof(type)); n_entries keeps its meaning.  dcb_batch_out_bytes is the size of the arena in the chosen order. */
+#define DCB_ORDER_ENTRIES 0
+#define DCB_ORDER_POINTS 1
+/* Before the first dcb_upload / dcb_decode* of the batch (DCB_ERR_STATE afterwards); re-lays out the output arena. */
+int dcb_set_output_order(dcb_batch *b, int order);
+/* Edgebreaker meshes whose connectivity the caller decoded: Mesh.Faces as 3 point ids per face, BORROWED like the
+ * maps (valid until the decode / upload that consumes them returns).  faces == NULL && n_faces == 0: the mesh has no
+ * attribute seams, point ids are vertex ids, faces = corner_to_vertex of attributes decoder 0 (AssignPointsToCorners
+ * without attribute data) -- nothing extra travels to the device.  dcb_host_connectivity installs its own faces.
+ * In point order an Edgebreaker buffer without faces, or whose 3 * n_faces is not the corner count of each of its
+ * decoders, fails with DCB_ERR_MAPS.  Point clouds and sequential meshes: DCB_ERR_STATE.  Install faces before
+ * dcb_index_finish, like the maps: afterwards, a call that turns a buffer's verdict (DCB_ERR_MAPS <-> ok) re-runs the
+ * attribute indexing of the whole batch. */
+int dcb_set_mesh_faces(dcb_batch *b, int buf, const uint32_t *faces, uint64_t n_faces);
 
 /* Phase 2 (device).  One-call form: host->device copy, kernels, device->host copy.
  * host_out: one arena of dcb_batch_out_bytes() bytes laid out by dcb_attr_info.out_off; host_dbg may be

@@ -52,6 +52,13 @@ public sealed class DracoBatchDecoder : IDisposable
         public int QBits, Resolved;
     }
 
+    [StructLayout(LayoutKind.Sequential)]
+    private struct FaceInfo
+    {
+        public ulong OutOff, OutBytes, NFaces;
+        public int Source, Reserved;
+    }
+
     [DllImport(Lib)] private static extern int dcb_version();
     [DllImport(Lib)] private static extern int dcb_device_count();
     [DllImport(Lib)] private static extern IntPtr dcb_error_string(int code);
@@ -72,6 +79,9 @@ public sealed class DracoBatchDecoder : IDisposable
     [DllImport(Lib)] private static extern int dcb_index_finish(IntPtr ctx, IntPtr batch);
     [DllImport(Lib)] private static extern int dcb_set_output_order(IntPtr batch, int order);
     [DllImport(Lib)] private static extern unsafe int dcb_set_mesh_faces(IntPtr batch, int buf, uint* faces, ulong nFaces);
+    [DllImport(Lib)] private static extern int dcb_set_face_output(IntPtr batch, int mode);
+    [DllImport(Lib)] private static extern int dcb_get_face_info(IntPtr batch, int buf, out FaceInfo info);
+    [DllImport(Lib)] private static extern unsafe int dcb_decode(IntPtr ctx, IntPtr batch, byte* hostOut, byte* hostDbg, uint flags);
     [DllImport(Lib)] private static extern unsafe int dcb_decode_scatter(IntPtr ctx, IntPtr batch, byte** outs, int nOuts, uint flags);
     [DllImport(Lib)] private static extern int dcb_status(IntPtr batch, int buf);
     [DllImport(Lib)] private static extern void dcb_batch_free(IntPtr batch);
@@ -101,8 +111,11 @@ public sealed class DracoBatchDecoder : IDisposable
     /// <paramref name="pointOrder"/>: attributes of Edgebreaker meshes arrive with one value per point (DCB_ORDER_POINTS,
     /// the point-to-value map applied on the GPU) and carry the identity mapping; otherwise they hold the unique entries
     /// and <see cref="IHostConnectivity.ApplyPointMapping"/> supplies the map.
+    /// <paramref name="facesInArena"/>: the faces of every mesh come out of the output arena (DCB_FACES_ARENA; plain
+    /// sequential indices decoded on the GPU) and the decode runs into one arena instead of the per-attribute scatter.
     /// </summary>
-    public unsafe Draco?[] DecodeBatch(IReadOnlyList<ReadOnlyMemory<byte>> buffers, out Exception?[] errors, bool pointOrder = false)
+    public unsafe Draco?[] DecodeBatch(IReadOnlyList<ReadOnlyMemory<byte>> buffers, out Exception?[] errors, bool pointOrder = false,
+                                       bool facesInArena = false)
     {
         int n = buffers.Count;
         var result = new Draco?[n];
@@ -124,6 +137,7 @@ public sealed class DracoBatchDecoder : IDisposable
             }
             Check(dcb_index(_ctx, ptrs, lens, n, out batch));
             if (pointOrder) Check(dcb_set_output_order(batch, 1));  // DCB_ORDER_POINTS
+            if (facesInArena) Check(dcb_set_face_output(batch, 1));  // DCB_FACES_ARENA, before the connectivity step
 
             // meshes: connectivity on the host, maps to the GPU
             var hostMeshes = new Mesh.Mesh?[n];
@@ -168,7 +182,7 @@ public sealed class DracoBatchDecoder : IDisposable
                 }
                 // Edgebreaker meshes only: the library refuses faces for sequential meshes (their attributes are already in point
                 // order).  A hook that exports no faces leaves the buffer to fail alone with DCB_ERR_MAPS.
-                if (pointOrder && bi.EncoderMethod == 1 && hc.Faces != null)  // Mesh.Faces as point ids, borrowed (pinned) like the maps
+                if ((pointOrder || facesInArena) && bi.EncoderMethod == 1 && hc.Faces != null)  // Mesh.Faces as point ids, borrowed (pinned) like the maps
                 {
                     var h = GCHandle.Alloc(hc.Faces, GCHandleType.Pinned);
                     mapPins.Add(h);
@@ -178,6 +192,7 @@ public sealed class DracoBatchDecoder : IDisposable
             if (anyMesh) Check(dcb_index_finish(_ctx, batch));
 
             // one DataBuffer per attribute: the GPU writes straight into their pinned byte arrays
+            byte[]? arena = null;
             var attrs = new List<(int buf, AttrInfo info, byte[] data, GCHandle pin)>();
             for (int k = 0; k < n; ++k)
             {
@@ -192,9 +207,25 @@ public sealed class DracoBatchDecoder : IDisposable
             try
             {
                 outs = (byte**)NativeMemory.Alloc((nuint)Math.Max(attrs.Count, 1), (nuint)sizeof(byte*));
-                for (int i = 0; i < attrs.Count; ++i)
-                    outs[i] = attrs[i].data.Length > 0 ? (byte*)attrs[i].pin.AddrOfPinnedObject() : null;
-                Check(dcb_decode_scatter(_ctx, batch, outs, attrs.Count, 0));
+                if (facesInArena)
+                {
+                    // dcb_decode_scatter has no slot for faces: one arena, sliced into the DataBuffers afterwards.  A .NET
+                    // array holds at most Array.MaxLength bytes (about 2 GB): larger batches must be split by the caller
+                    // (checked below rather than truncated)
+                    ulong arenaBytes = dcb_batch_out_bytes(batch);
+                    if (arenaBytes > (ulong)Array.MaxLength)
+                        throw new InvalidOperationException($"DecodeBatch(facesInArena): output arena of {arenaBytes} bytes exceeds one .NET array; split the batch");
+                    arena = new byte[arenaBytes];
+                    fixed (byte* p = arena) Check(dcb_decode(_ctx, batch, p, null, 0));
+                    foreach (var a in attrs)
+                        if (a.data.Length > 0) Array.Copy(arena, (long)a.info.OutOff, a.data, 0, a.data.Length);
+                }
+                else
+                {
+                    for (int i = 0; i < attrs.Count; ++i)
+                        outs[i] = attrs[i].data.Length > 0 ? (byte*)attrs[i].pin.AddrOfPinnedObject() : null;
+                    Check(dcb_decode_scatter(_ctx, batch, outs, attrs.Count, 0));
+                }
             }
             finally
             {
@@ -216,7 +247,16 @@ public sealed class DracoBatchDecoder : IDisposable
                 }
                 PointCloud.PointCloud pc = hostMeshes[k] ?? (bi.GeometryType == 1 ? new Mesh.Mesh() : new PointCloud.PointCloud());
                 pc.PointsCount = (int)bi.NPoints;
-                if (hostMeshes[k] == null && pc is Mesh.Mesh mesh)
+                if (hostMeshes[k] == null && pc is Mesh.Mesh arenaMesh && arena != null)
+                {
+                    // faces from the output arena: u32 point ids, 3 per face (dcb_get_face_info); offsets stay 64-bit until
+                    // the slice, which the array bounds check
+                    Check(dcb_get_face_info(batch, k, out var fi));
+                    var ids = MemoryMarshal.Cast<byte, uint>(arena.AsSpan(checked((int)fi.OutOff), checked((int)fi.OutBytes)));
+                    for (long f = 0; f < (long)fi.NFaces; ++f)
+                        arenaMesh.SetFace((int)f, new[] { (int)ids[(int)(3 * f)], (int)ids[(int)(3 * f + 1)], (int)ids[(int)(3 * f + 2)] });
+                }
+                else if (hostMeshes[k] == null && pc is Mesh.Mesh mesh)
                 {
                     // the library decoded the connectivity: its faces (Mesh.SetFace, MeshEdgeBreakerDecoder.cs:622-636)
                     Check(dcb_mesh_faces(batch, k, null, 0, out ulong nFaces));

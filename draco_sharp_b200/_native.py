@@ -14,6 +14,8 @@ DCB_DUMP_SYMBOLS = 1
 DCB_DUMP_QINTS = 2
 DCB_ORDER_ENTRIES = 0
 DCB_ORDER_POINTS = 1
+DCB_FACES_NONE = 0
+DCB_FACES_ARENA = 1
 
 ERR = {
     0: "DCB_OK", -1: "DCB_ERR_EOF", -2: "DCB_ERR_MAGIC", -3: "DCB_ERR_UNSUPPORTED", -4: "DCB_ERR_SCHEME",
@@ -43,6 +45,13 @@ class AttrInfo(C.Structure):
         ("n_entries", C.c_uint32), ("out_bytes", C.c_uint64), ("out_off", C.c_uint64), ("dbg_off", C.c_uint64),
         ("xf_a", C.c_int32), ("xf_b", C.c_int32), ("q_min", C.c_float * 4), ("q_range", C.c_float),
         ("q_bits", C.c_int32), ("resolved", C.c_int32),
+    ]
+
+
+class FaceInfo(C.Structure):
+    _fields_ = [
+        ("out_off", C.c_uint64), ("out_bytes", C.c_uint64), ("n_faces", C.c_uint64), ("source", C.c_int32),
+        ("reserved", C.c_int32),
     ]
 
 
@@ -97,6 +106,8 @@ EXPORTS = [
     ("dcb_index_finish", C.c_int, [_P, _P]),
     ("dcb_set_output_order", C.c_int, [_P, C.c_int]),
     ("dcb_set_mesh_faces", C.c_int, [_P, C.c_int, _P, C.c_uint64]),
+    ("dcb_set_face_output", C.c_int, [_P, C.c_int]),
+    ("dcb_get_face_info", C.c_int, [_P, C.c_int, C.POINTER(FaceInfo)]),
     ("dcb_decode", C.c_int, [_P, _P, _P, _P, C.c_uint32]),
     ("dcb_decode_scatter", C.c_int, [_P, _P, C.POINTER(_P), C.c_int, C.c_uint32]),
     ("dcb_upload", C.c_int, [_P, _P]),

@@ -122,6 +122,12 @@ struct BufRec {
   bool pt_faces_set = false;
   bool pt_failed = false;          // the status is the point-order face check's verdict (undone when indexing reruns)
   uint64_t faces_dev_off = 0;      // explicit faces inside the shard's maps arena
+  // faces in the output arena (DCB_FACES_ARENA).  pt_faces / pt_n_faces also carry the host-decoded faces of a sequential
+  // mesh there: they travel with the maps like an Edgebreaker buffer's explicit faces.
+  DcbSeqIndexLoc seq_loc;          // sequential, plain indices: located by dcb_host_connectivity, decoded on the GPU
+  int32_t face_src = 0;            // dcb_face_info.source of the current layout
+  int32_t idx_job = -1;            // Raw index differences decoded on the GPU: the buffer's slot in Shard::h_fstatus
+  uint64_t n_faces = 0, face_off = 0;  // face_off: shard-local offset of the faces region
 };
 
 struct Group {            // one kernel launch (or a few, for global tables)
@@ -200,6 +206,16 @@ struct Shard {
   uint8_t *d_pts = nullptr;    // staging | point maps | job tables
   uint64_t cap_pts = 0;
   std::vector<uint8_t> pts_tables;  // host copy of the job tables (source of the asynchronous upload)
+  // DCB_FACES_ARENA: job tables of the faces stage (dcb_faces.cu) and their host copy
+  FaceStage fstage{};
+  uint8_t *d_faces = nullptr;
+  uint64_t cap_faces = 0;
+  std::vector<uint8_t> faces_tables;
+  // Raw index differences of sequential meshes: one rANS stream each, appended to `streams` behind the attributes of
+  // all buffers (from idx_first on; no buffer's walk covers them); their per-buffer verdicts come back in h_fstatus
+  uint32_t idx_first = ~0u;
+  int32_t *h_fstatus = nullptr;
+  uint64_t cap_hfstatus = 0;
 };
 
 }  // namespace
@@ -243,6 +259,7 @@ struct dcb_batch {
   int n_devices = 1;
   uint64_t max_points = 0, points_per_byte = 0;  // plausibility limits (dcb_set_limits), copied from the context
   int order = DCB_ORDER_ENTRIES;
+  int faces = DCB_FACES_NONE;
   bool conn_done = false;  // dcb_index_finish has run: a new order or new faces rerun it
 };
 
@@ -388,6 +405,13 @@ bool point_faces_ok(const BufRec &b, int n_dec) {
   return true;
 }
 
+// DCB_FACES_ARENA: a mesh needs faces to put in the arena -- installed by dcb_host_connectivity or (Edgebreaker)
+// dcb_set_mesh_faces; the NULL form needs the corner table of attributes decoder 0
+bool faces_known(const BufRec &b) {
+  if (!b.pt_faces_set) return false;
+  return !b.is_eb || b.pt_faces || (!b.maps.empty() && b.maps[0].set);
+}
+
 // DEC_ID + DEC_DATA: creates the StreamDescs of one buffer (appended to sh.streams) and its BufWalk.
 void parse_attr_section(BufRec &b, Shard &sh, int buf_index, const dcb_batch *batch = nullptr) {
   dcb_buffer_info &inf = b.info;
@@ -409,6 +433,10 @@ void parse_attr_section(BufRec &b, Shard &sh, int buf_index, const dcb_batch *ba
   };
   if (inf.status) return finish(inf.status);
   if (inf.needs_connectivity) return finish(0);  // attributes are indexed by dcb_index_finish
+  if (batch && batch->faces == DCB_FACES_ARENA && inf.geometry_type == 1 && !faces_known(b)) {
+    b.pt_failed = true;
+    return finish(DCB_ERR_MAPS);
+  }
   HRd r{b.src, b.len, inf.attr_section_off, 0};
   const int n_dec = (int)r.u8();  // ConnectivityDecoder.cs:18
   if (r.err) return finish(r.err);
@@ -604,6 +632,10 @@ void free_shard_device(Shard &sh) {
   pool_free(sh.pool, sh.device, sh.d_order, sh.cap_order);
   pool_free(sh.pool, sh.device, sh.d_pts, sh.cap_pts);
   sh.d_pts = nullptr;
+  pool_free(sh.pool, sh.device, sh.d_faces, sh.cap_faces);
+  sh.d_faces = nullptr;
+  if (sh.h_fstatus) pinned_free(sh.pool, sh.h_fstatus, sh.cap_hfstatus);
+  sh.h_fstatus = nullptr;
   if (sh.h_stage) pinned_free(sh.pool, sh.h_stage, sh.cap_stage);
   if (sh.h_maps) pinned_free(sh.pool, sh.h_maps, sh.cap_hmaps);
   sh.h_maps = nullptr;
@@ -823,6 +855,74 @@ void layout_points(const dcb_batch *b, Shard &sh) {
   sh.out_bytes = out;
 }
 
+// DCB_FACES_ARENA: behind the attributes of a shard, a faces region per mesh buffer that is ok, in buffer order, each on a
+// 128-byte boundary
+// A sequential mesh whose Raw index differences the GPU decodes gets one more Raw rANS stream (one component, no zig-zag:
+// the value map holds the raw symbol; RECON_PARA_WRAP routes the symbols to the int32 scratch as for mesh corrections),
+// located by the walker code the attribute streams use, with scratch and debug space of its own.
+void add_index_stream(BufRec &r, int k, Shard &sh) {
+  StreamDesc s;
+  memset(&s, 0, sizeof s);
+  s.buf_begin = r.arena_off;
+  s.buf_end = r.arena_off + r.len;
+  s.buf_index = k;
+  s.attr_index = -1;
+  s.parent = -1;
+  s.n_entries = (uint32_t)r.seq_loc.n_idx;
+  s.nc = s.ncp = 1;
+  s.data_type = DT_INT32;
+  s.seq_type = SEQ_INTEGER;
+  s.pred_method = PRED_NONE;
+  s.transform = XF_NONE;
+  s.scheme = SCHEME_RAW;
+  s.compressed = 1;
+  s.zigzag = 0;
+  s.recon = RECON_PARA_WRAP;
+  s.store = STORE_NARROW;
+  s.max_bit_length = (uint8_t)r.seq_loc.mbl;
+  s.prec_bits = (uint8_t)dcb_rans_precision(r.seq_loc.mbl);
+  WalkRd wr{r.src - r.arena_off, r.arena_off + r.len, r.arena_off + r.seq_loc.off, 0};
+  s.table_off = wr.pos;
+  int e = walk_rans_table(wr, s.prec_bits, s.num_symbols, s.n_active, s.dense_prefix, s.narrow_blk, s.rec_need);
+  if (!e) e = walk_rans_payload(wr, s.prec_bits, s.payload_off, s.payload_len);
+  s.status = e;  // the host checked this stream already (dcb_host_sequential): cannot fail
+  s.state = ST_READY;
+  s.aux_off = align_up(sh.aux_bytes, 16);
+  sh.aux_bytes = align_up(s.aux_off + 4ull * s.n_entries, 16);
+  s.dbg_off = sh.dbg_bytes;
+  sh.dbg_bytes = align_up(s.dbg_off + 4ull * s.n_entries, 16);
+  sh.streams.push_back(s);
+}
+
+void layout_faces(dcb_batch *b, Shard &sh) {
+  uint64_t out = sh.out_bytes;
+  if (sh.idx_first != ~0u && sh.idx_first <= sh.streams.size()) sh.streams.resize(sh.idx_first);
+  sh.idx_first = (uint32_t)sh.streams.size();
+  for (int k : sh.bufs) {
+    BufRec &r = b->bufs[k];
+    r.face_src = 0;
+    r.idx_job = -1;
+    r.n_faces = r.face_off = 0;
+    if (b->faces != DCB_FACES_ARENA || r.info.geometry_type != 1 || r.info.needs_connectivity || r.info.status != DCB_OK)
+      continue;
+    if (r.is_eb) {
+      if (!r.pt_faces && (r.maps.empty() || !r.maps[0].set)) continue;  // no faces (failed at indexing; see faces_known)
+      r.n_faces = r.pt_faces ? r.pt_n_faces : r.maps[0].n_corners / 3;
+      r.face_src = 1;
+    } else if (r.seq_loc.located) {
+      if (r.seq_loc.width < 0 && r.seq_loc.n_idx) add_index_stream(r, k, sh);
+      r.n_faces = r.seq_loc.n_idx / 3;
+      r.face_src = 2;
+    } else {
+      r.n_faces = r.pt_n_faces;
+      r.face_src = 1;
+    }
+    r.face_off = align_up(out, 128);
+    out = r.face_off + 12 * r.n_faces;
+  }
+  sh.out_bytes = out;
+}
+
 void finalize_layout(dcb_batch *b) {
   uint64_t out_base = 0, dbg_base = 0;
   b->total_in = 0;
@@ -831,6 +931,7 @@ void finalize_layout(dcb_batch *b) {
   for (Shard &sh : b->shards) {
     layout_shard(sh);
     layout_points(b, sh);
+    layout_faces(b, sh);  // may append index streams: before streams0
     sh.out_base = out_base;
     sh.dbg_base = dbg_base;
     out_base += align_up(sh.out_bytes, 128);
@@ -851,6 +952,7 @@ void finalize_layout(dcb_batch *b) {
       for (int i = 0; i < w.stream_count; ++i) b->algo_bytes += sh.streams[w.stream_first + i].out_bytes;
       for (const MeshMapsHost &m : r.maps)
         if (m.set) b->algo_bytes += m.bytes();
+      b->algo_bytes += 12 * r.n_faces;
     }
   }
 }
@@ -1140,9 +1242,11 @@ int issue_arena_copy(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index) {
   return DCB_OK;
 }
 
-// point order: the explicit faces of an indexed Edgebreaker buffer travel with its maps (the NULL form reads the maps)
+// point order: the explicit faces of an indexed Edgebreaker buffer travel with its maps (the NULL form reads the maps);
+// faces in the arena: so do the host-decoded faces of sequential meshes
 bool uploads_faces(const Shard &sh, const BufRec &r) {
-  return sh.pts && r.is_eb && r.pt_faces && sh.walks0[r.local].status == DCB_OK;
+  if (!r.pt_faces || sh.walks0[r.local].status != DCB_OK) return false;
+  return (sh.pts && r.is_eb) || r.face_src == 1;
 }
 
 // Mesh connectivity maps (56 bytes per vertex, read by para_deps_kernel only): on the device's upload stream, issued
@@ -1318,6 +1422,118 @@ int plan_points(dcb_batch *b, Shard &sh, cudaStream_t st) {
   return DCB_OK;
 }
 
+// DCB_FACES_ARENA: the job tables of the faces stage (dcb_faces.cu) -- one job per mesh buffer with faces: fixed-width
+// plain indices from the input arena, u32 faces from the maps arena, varint runs with their checkpoints
+int plan_faces(dcb_batch *b, Shard &sh, cudaStream_t st) {
+  std::vector<FaceJob> pj, vj, ij;
+  std::vector<uint64_t> upre{0}, cpre{0}, ckpt, ipre{0};
+  for (uint32_t si = sh.idx_first; si < sh.streams.size(); ++si) {
+    BufRec &r = b->bufs[sh.streams[si].buf_index];
+    FaceJob f{};
+    f.dst_off = r.face_off;
+    f.n_idx = 3 * r.n_faces;
+    f.stream = si;
+    r.idx_job = (int32_t)ij.size();
+    ij.push_back(f);
+    ipre.push_back(ipre.back() + (f.n_idx + DCB_INDEX_CHUNK - 1) / DCB_INDEX_CHUNK);
+  }
+  for (int k : sh.bufs) {
+    const BufRec &r = b->bufs[k];
+    if (!r.face_src || !r.n_faces || r.idx_job >= 0) continue;
+    FaceJob f{};
+    f.dst_off = r.face_off;
+    f.n_idx = 3 * r.n_faces;
+    if (r.face_src == 2) {
+      f.src_off = r.arena_off + r.seq_loc.off;
+      f.width = (uint32_t)r.seq_loc.width;
+      f.n_bytes = r.seq_loc.bytes;
+    } else {
+      f.from_maps = 1;
+      f.width = 4;
+      f.src_off = r.pt_faces ? r.faces_dev_off : r.maps[0].dev_off[1];
+    }
+    if (f.width) {
+      pj.push_back(f);
+      upre.push_back(upre.back() + (f.n_idx + 3) / 4);
+    } else {
+      f.ckpt_off = ckpt.size();
+      ckpt.insert(ckpt.end(), r.seq_loc.ckpt.begin(), r.seq_loc.ckpt.end());
+      vj.push_back(f);
+      cpre.push_back(cpre.back() + r.seq_loc.ckpt.size());
+    }
+  }
+  FaceStage &p = sh.fstage;
+  p = FaceStage{};
+  if (pj.empty() && vj.empty() && ij.empty()) return DCB_OK;
+  const uint64_t off_pj = 0;
+  const uint64_t off_upre = align_up(off_pj + pj.size() * sizeof(FaceJob), 16);
+  const uint64_t off_vj = align_up(off_upre + upre.size() * 8, 16);
+  const uint64_t off_cpre = align_up(off_vj + vj.size() * sizeof(FaceJob), 16);
+  const uint64_t off_ckpt = align_up(off_cpre + cpre.size() * 8, 16);
+  const uint64_t off_ij = align_up(off_ckpt + ckpt.size() * 8, 16);
+  const uint64_t off_ipre = align_up(off_ij + ij.size() * sizeof(FaceJob), 16);
+  const uint64_t n_ich = ipre.back();
+  // device-written: chunk sums, minima, maxima (int64 each) and one status per index job
+  const uint64_t off_csum = align_up(off_ipre + ipre.size() * 8, 16);
+  const uint64_t off_cmin = off_csum + 8 * n_ich, off_cmax = off_cmin + 8 * n_ich, off_stat = off_cmax + 8 * n_ich;
+  const uint64_t total = off_stat + 4 * ij.size();
+  CUDA_TRY(pool_alloc(sh.pool, sh.device, total, &sh.d_faces, &sh.cap_faces));
+  std::vector<uint8_t> &t = sh.faces_tables;  // outlives the asynchronous upload
+  t.assign(total, 0);
+  auto put = [&](uint64_t off, const void *src, uint64_t n) { if (n) memcpy(t.data() + off, src, n); };
+  put(off_pj, pj.data(), pj.size() * sizeof(FaceJob));
+  put(off_upre, upre.data(), upre.size() * 8);
+  put(off_vj, vj.data(), vj.size() * sizeof(FaceJob));
+  put(off_cpre, cpre.data(), cpre.size() * 8);
+  put(off_ckpt, ckpt.data(), ckpt.size() * 8);
+  put(off_ij, ij.data(), ij.size() * sizeof(FaceJob));
+  put(off_ipre, ipre.data(), ipre.size() * 8);
+  CUDA_TRY(cudaMemcpyAsync(sh.d_faces, t.data(), off_csum, cudaMemcpyHostToDevice, st));
+  if (!ij.empty() && (!sh.h_fstatus || sh.cap_hfstatus < 4 * ij.size())) {
+    if (sh.h_fstatus) pinned_free(sh.pool, sh.h_fstatus, sh.cap_hfstatus);
+    uint8_t *hp = nullptr;
+    CUDA_TRY(pinned_alloc(sh.pool, 4 * ij.size(), &hp, &sh.cap_hfstatus));
+    sh.h_fstatus = reinterpret_cast<int32_t *>(hp);
+  }
+  p.plain = reinterpret_cast<const FaceJob *>(sh.d_faces + off_pj);
+  p.unit_prefix = reinterpret_cast<const uint64_t *>(sh.d_faces + off_upre);
+  p.n_plain = (uint32_t)pj.size();
+  p.varint = reinterpret_cast<const FaceJob *>(sh.d_faces + off_vj);
+  p.chunk_prefix = reinterpret_cast<const uint64_t *>(sh.d_faces + off_cpre);
+  p.n_varint = (uint32_t)vj.size();
+  p.ckpt = reinterpret_cast<const uint64_t *>(sh.d_faces + off_ckpt);
+  p.total_units = upre.back();
+  p.total_chunks = cpre.back();
+  p.index = reinterpret_cast<const FaceJob *>(sh.d_faces + off_ij);
+  p.index_prefix = reinterpret_cast<const uint64_t *>(sh.d_faces + off_ipre);
+  p.n_index = (uint32_t)ij.size();
+  p.total_index_chunks = n_ich;
+  p.chunk_sum = reinterpret_cast<int64_t *>(sh.d_faces + off_csum);
+  p.chunk_min = reinterpret_cast<int64_t *>(sh.d_faces + off_cmin);
+  p.chunk_max = reinterpret_cast<int64_t *>(sh.d_faces + off_cmax);
+  p.status = reinterpret_cast<int32_t *>(sh.d_faces + off_stat);
+  return DCB_OK;
+}
+
+// DCB_FACES_ARENA: fills the faces regions of a shard, on its stream behind its decode (the maps copy first)
+int faces_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index, uint8_t *d_out) {
+  if (!sh.fstage.total_units && !sh.fstage.total_chunks && !sh.fstage.n_index) return DCB_OK;
+  int rc = issue_maps_copy(ctx, b, sh, dev_index);
+  if (rc) return rc;
+  cudaStream_t st = ctx->streams[dev_index];
+  CUDA_TRY(cudaSetDevice(sh.device));
+  tl_mark(ctx, "faces s" + std::to_string(dev_index), st, true);
+  // behind the joins of decode_shard: the Raw index streams have left their symbols in the scratch
+  DevArenas A{sh.d_in, d_out, nullptr, sh.d_aux, nullptr, sh.d_maps};
+  CUDA_TRY(dcb_launch_faces(sh.fstage, sh.d_streams, A, (uint32_t)ctx->num_sms[dev_index], st));
+  tl_mark(ctx, "", st, false);
+  if (sh.fstage.n_index)  // per-buffer verdicts of the index scan, folded in by collect_status after the caller's sync
+    CUDA_TRY(cudaMemcpyAsync(sh.h_fstatus, sh.fstage.status, 4ull * sh.fstage.n_index, cudaMemcpyDeviceToHost, st));
+  dcb_launch_stats &stats = dev_index == 0 ? ctx->stats : ctx->dev_stats[dev_index];
+  stats.n_launches += (sh.fstage.total_units ? 1 : 0) + (sh.fstage.total_chunks ? 1 : 0) + (sh.fstage.n_index ? 3 : 0);
+  return DCB_OK;
+}
+
 int upload_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index) {
   if (sh.uploaded) return DCB_OK;
   cudaStream_t st = ctx->streams[dev_index];
@@ -1394,6 +1610,10 @@ int upload_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index) {
   }
   if (sh.pts) {
     int rc = plan_points(b, sh, st);
+    if (rc) return rc;
+  }
+  if (b->faces == DCB_FACES_ARENA) {
+    int rc = plan_faces(b, sh, st);
     if (rc) return rc;
   }
   sh.uploaded = true;
@@ -1723,6 +1943,25 @@ int decode_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index, uint8_t *
         has_para = true;
       }
     }
+  }
+  // Raw index differences of sequential meshes (DCB_FACES_ARENA): one-component streams without zig-zag; they depend on
+  // nothing else in their buffer, so their group runs beside the attribute groups (side streams when there are several)
+  for (uint32_t si = sh.idx_first; si < sh.streams.size(); ++si) {
+    const StreamDesc &s = sh.streams[si];
+    if (s.status || sh.walks[b->bufs[s.buf_index].local].status != DCB_OK) continue;
+    const RawKey key = raw_key_of(s, false, -1);
+    const uint32_t entries = key.compact ? s.n_active : s.num_symbols;
+    Group &g = raw[key];
+    if (g.order.empty()) {
+      g.kind = 0; g.ncp = 1; g.wide = key.wide != 0; g.compact = (uint32_t)key.compact; g.prec_bits = (uint32_t)key.prec;
+      g.zig = 0; g.mode = (uint32_t)key.mode;
+    }
+    g.entries = std::max(g.entries, entries);
+    if (key.compact) g.exc = std::max(g.exc, s.n_active - std::min(s.n_active, s.dense_prefix));
+    g.total_symbols += s.n_entries;
+    g.max_entries = std::max(g.max_entries, s.n_entries);
+    g.note_table(s);
+    g.order.push_back(si);
   }
   std::vector<Group *> rgs;
   for (auto &kv : raw) rgs.push_back(&kv.second);
@@ -2106,6 +2345,7 @@ void collect_status(dcb_batch *b) {
       const StreamDesc &s = sh.streams[w.stream_first + i];
       if (s.status) { r.info.status = s.status; break; }
     }
+    if (!r.info.status && r.idx_job >= 0 && sh.h_fstatus) r.info.status = sh.h_fstatus[r.idx_job];
   }
 }
 
@@ -2219,6 +2459,8 @@ int decode_all_impl(dcb_ctx *ctx, dcb_batch *b, void *dev_out, void *dev_dbg, ui
     int rc = issue_arena_copy(ctx, b, sh, d);
     if (rc) return rc;
     rc = decode_shard(ctx, b, sh, d, sh.ext_out, sh.ext_dbg, flags, true);
+    if (rc) return rc;
+    rc = faces_shard(ctx, b, sh, d, sh.ext_out);
     if (rc) return rc;
     if (host_out || host_dbg) {  // host-buffer decode: this shard's results start travelling while the next one decodes
       rc = download_shard(ctx, b, d, host_out, host_dbg);
@@ -2627,7 +2869,11 @@ int dcb_host_connectivity(dcb_batch *b, int buf) {
       uint32_t n_points = 0;
       int st;
       try {
-        st = dcb_host_sequential(r.src, r.len, r.conn_off, &attr_off, &n_points, &r.faces);
+        // DCB_FACES_ARENA: plain indices are located, the GPU decodes them into the arena
+        r.seq_loc = DcbSeqIndexLoc{};
+        r.faces.clear();
+        st = dcb_host_sequential(r.src, r.len, r.conn_off, &attr_off, &n_points, &r.faces,
+                                 b->faces == DCB_FACES_ARENA ? &r.seq_loc : nullptr);
       } catch (const std::bad_alloc &) {
         st = DCB_ERR_OOM;
       } catch (...) {
@@ -2639,6 +2885,9 @@ int dcb_host_connectivity(dcb_batch *b, int buf) {
       }
       r.info.attr_section_off = attr_off;
       r.info.n_points = n_points;
+      r.pt_faces_set = true;  // faces for DCB_FACES_ARENA: decoded here, or located for the GPU
+      r.pt_faces = r.faces.empty() ? nullptr : r.faces.data();
+      r.pt_n_faces = r.faces.size() / 3;
       return DCB_OK;
     }
     std::vector<DcbHostMaps> maps;
@@ -2693,6 +2942,7 @@ int dcb_mesh_faces(const dcb_batch *b, int buf, uint32_t *faces, uint64_t cap_fa
   return guarded([&]() -> int {
     if (!b || buf < 0 || buf >= (int)b->bufs.size() || !n_faces) return DCB_ERR_ARG;
     const BufRec &r = b->bufs[buf];
+    if (r.seq_loc.located) return DCB_ERR_STATE;  // decoded on the GPU, into the output arena
     *n_faces = r.faces.size() / 3;
     if (faces) {
       if (cap_faces < *n_faces) return DCB_ERR_ARG;
@@ -2728,6 +2978,7 @@ int dcb_index_finish(dcb_ctx *ctx, dcb_batch *b) {
     // rebuild every shard's stream list with the connectivity-dependent buffers included
     for (Shard &sh : b->shards) {
       sh.streams.clear();
+      sh.idx_first = ~0u;
       std::fill(sh.walks.begin(), sh.walks.end(), BufWalk{});
     }
     for (size_t k = 0; k < b->bufs.size(); ++k) {
@@ -2762,6 +3013,36 @@ int dcb_set_output_order(dcb_batch *b, int order) {
   });
 }
 
+int dcb_set_face_output(dcb_batch *b, int mode) {
+  return guarded([&]() -> int {
+    if (!b || (mode != DCB_FACES_NONE && mode != DCB_FACES_ARENA)) return DCB_ERR_ARG;
+    for (const Shard &sh : b->shards)
+      if (sh.uploaded) return DCB_ERR_STATE;
+    if (mode == b->faces) return DCB_OK;
+    // indices dcb_host_connectivity only located for the GPU are not on the host: they need this mode
+    for (const BufRec &r : b->bufs)
+      if (r.seq_loc.located) return DCB_ERR_STATE;
+    b->faces = mode;
+    if (b->conn_done) return dcb_index_finish(nullptr, b);
+    finalize_layout(b);
+    return DCB_OK;
+  });
+}
+
+int dcb_get_face_info(const dcb_batch *b, int buf, dcb_face_info *out) {
+  return guarded([&]() -> int {
+    if (!b || !out || buf < 0 || buf >= (int)b->bufs.size()) return DCB_ERR_ARG;
+    const BufRec &r = b->bufs[buf];
+    memset(out, 0, sizeof *out);
+    if (!r.face_src) return DCB_OK;
+    out->out_off = b->shards[r.shard].out_base + r.face_off;
+    out->out_bytes = 12 * r.n_faces;
+    out->n_faces = r.n_faces;
+    out->source = r.info.status == DCB_OK ? r.face_src : 0;
+    return DCB_OK;
+  });
+}
+
 int dcb_set_mesh_faces(dcb_batch *b, int buf, const uint32_t *faces, uint64_t n_faces) {
   return guarded([&]() -> int {
     if (!b || buf < 0 || buf >= (int)b->bufs.size()) return DCB_ERR_ARG;
@@ -2770,6 +3051,7 @@ int dcb_set_mesh_faces(dcb_batch *b, int buf, const uint32_t *faces, uint64_t n_
     if (!r.is_eb) return DCB_ERR_STATE;
     for (const Shard &sh : b->shards)
       if (sh.uploaded) return DCB_ERR_STATE;
+    const bool known_before = faces_known(r);
     r.pt_faces = faces;
     r.pt_n_faces = n_faces;
     r.pt_faces_set = true;
@@ -2777,6 +3059,10 @@ int dcb_set_mesh_faces(dcb_batch *b, int buf, const uint32_t *faces, uint64_t n_
     if (b->conn_done && b->order == DCB_ORDER_POINTS && !r.info.needs_connectivity && (r.info.status == DCB_OK || r.pt_failed) &&
         point_faces_ok(r, r.info.n_attr_decoders) == r.pt_failed)
       return dcb_index_finish(nullptr, b);
+    if (b->conn_done && b->faces == DCB_FACES_ARENA) {  // faces in the arena: a new verdict or a new region size
+      if (r.pt_failed || faces_known(r) != known_before) return dcb_index_finish(nullptr, b);
+      finalize_layout(b);
+    }
     return DCB_OK;
   });
 }
@@ -2847,6 +3133,7 @@ int dcb_decode(dcb_ctx *ctx, dcb_batch *b, uint8_t *host_out, uint8_t *host_dbg,
 int dcb_decode_scatter(dcb_ctx *ctx, dcb_batch *b, uint8_t *const *outs, int n_outs, uint32_t flags) {
   return guarded([&]() -> int {
     if (!outs && n_outs) return DCB_ERR_ARG;
+    if (b && b->faces == DCB_FACES_ARENA) return DCB_ERR_STATE;  // no slot for the faces
     int rc = decode_all(ctx, b, nullptr, nullptr, flags & ~(DCB_DUMP_SYMBOLS | DCB_DUMP_QINTS));
     if (rc) return rc;
     int k = 0;

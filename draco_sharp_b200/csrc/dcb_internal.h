@@ -11,6 +11,9 @@
 #define DCB_HD inline
 #endif
 
+// DCB_FACES_ARENA: bytes of a varint index run per checkpoint = one CTA iteration of seq_varint_kernel (dcb_faces.cu)
+#define DCB_VARINT_CHUNK 4096u
+
 // wire enums (numeric values are part of the bitstream; src/Draco/IO/Enums/*.cs)
 enum : int32_t {
   DT_INT8 = 1, DT_UINT8 = 2, DT_INT16 = 3, DT_UINT16 = 4, DT_INT32 = 5, DT_UINT32 = 6,

@@ -130,3 +130,42 @@ struct PointStage {
 // per copy unit of every row of every attribute), on `st`
 cudaError_t dcb_launch_point_stage(const PointStage &p, StreamDesc *d_streams, const DevArenas &a, uint32_t num_sms,
                                    cudaStream_t st);
+
+// ---- faces in the output arena (DCB_FACES_ARENA, dcb_faces.cu) ----
+struct FaceJob {                   // the faces of one mesh buffer
+  uint64_t src_off;                // first index byte: input arena (sequential plain indices) or maps arena (u32 faces)
+  uint64_t dst_off;                // faces region in the output arena (128-byte aligned)
+  uint64_t n_idx;                  // 3 * n_faces
+  uint64_t n_bytes;                // varint: bytes of the index run
+  uint64_t ckpt_off;               // varint: first checkpoint of the job (FaceStage::ckpt)
+  uint32_t width;                  // bytes per index: 1, 2 or 4; 0 = varint
+  uint32_t from_maps;              // 1: src_off is in the maps arena
+  uint32_t stream;                 // Raw index differences: the shard-wide index of their rANS stream (symbols at its aux_off)
+  uint32_t pad_;
+};
+struct FaceStage {
+  const FaceJob *plain;            // fixed-width jobs; unit_prefix: n_plain + 1 running sums of ceil(n_idx / 4)
+  const uint64_t *unit_prefix;
+  uint32_t n_plain;
+  const FaceJob *varint;           // varint jobs; chunk_prefix: n_varint + 1 running sums of their DCB_VARINT_CHUNK-byte chunks
+  const uint64_t *chunk_prefix;
+  uint32_t n_varint;
+  const uint64_t *ckpt;            // per chunk: indices that end in front of it (located by the host)
+  uint64_t total_units, total_chunks;  // = unit_prefix[n_plain], chunk_prefix[n_varint] (grid sizes)
+  // Raw index differences (method 0): the rANS kernels leave the symbols in the int32 scratch; three passes over
+  // DCB_INDEX_CHUNK-index chunks turn them into indices
+  const FaceJob *index;            // index_prefix: n_index + 1 running sums of their chunks
+  const uint64_t *index_prefix;
+  uint32_t n_index;
+  uint64_t total_index_chunks;
+  int64_t *chunk_sum, *chunk_min, *chunk_max;  // per chunk: sum of its steps (then the index in front of it), extreme prefixes
+  int32_t *status;                 // per index job: DCB_ERR_CONNECTIVITY or the failure of its rANS stream
+};
+#define DCB_INDEX_CHUNK 4096u
+// seq_plain_kernel (one thread per 4 indices of every fixed-width job: widen to u32) | seq_varint_kernel (one CTA per
+// chunk of a varint run: terminator bytes, their ordinals by a block scan from the chunk's checkpoint, values assembled
+// backwards by the terminator's thread), on `st`
+// seq_index_sum_kernel | seq_index_base_kernel | seq_index_store_kernel: Raw index differences (sign-magnitude steps,
+// symbol >> 1, negative when bit 0 is set) -> inclusive int64 scan per buffer (chunk sums, then one thread per buffer over
+// its chunks, then the chunks again) with the range checks of dcb_host_sequential (0 <= index <= INT32_MAX)
+cudaError_t dcb_launch_faces(const FaceStage &p, const StreamDesc *d_streams, const DevArenas &a, uint32_t num_sms, cudaStream_t st);

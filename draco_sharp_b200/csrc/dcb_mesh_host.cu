@@ -18,6 +18,7 @@
 #include <stdint.h>
 #include <string.h>
 
+#include <algorithm>
 #include <vector>
 
 #include "dcb_internal.h"
@@ -84,10 +85,14 @@ struct RabsBits {
   }
 };
 
-// Raw / Tagged symbols of the valence contexts (SymbolDecoding.cs:7-67), host side, small counts
-int host_symbols(Reader &r, uint32_t n, std::vector<uint32_t> &out) {
-  out.assign(n, 0);
-  if (n == 0) return DCB_OK;
+// Raw / Tagged symbols of the valence contexts and of sequential-mesh indices (SymbolDecoding.cs:7-67), host side.
+// raw_loc != NULL: a Raw stream is only checked and located (RANS_TABLE at raw_loc->off, payload behind it), not decoded;
+// raw_loc->located stays false for a Tagged one, which is decoded as usual.
+int host_symbols(Reader &r, uint32_t n, std::vector<uint32_t> &out, DcbSeqIndexLoc *raw_loc = nullptr) {
+  if (n == 0) {
+    out.clear();
+    return DCB_OK;
+  }
   const uint32_t scheme = r.u8();
   if (r.err) return r.err;
   int mbl = 5;
@@ -100,6 +105,7 @@ int host_symbols(Reader &r, uint32_t n, std::vector<uint32_t> &out) {
   }
   const int pb = dcb_rans_precision(mbl);
   const uint32_t prec = 1u << pb, lbase = 4u << pb;
+  const uint64_t table_off = r.pos;
   const uint64_t ns = r.varint();
   if (r.err) return r.err;
   if (ns == 0) return DCB_ERR_NUM_SYMBOLS;
@@ -124,9 +130,6 @@ int host_symbols(Reader &r, uint32_t n, std::vector<uint32_t> &out) {
   for (uint64_t i = 0; i < ns; ++i) { cum[i] = (uint32_t)c; c += prob[i]; if (c > prec) return DCB_ERR_TABLE; }
   if (c != prec) return DCB_ERR_TABLE;
   cum[ns] = prec;
-  std::vector<uint32_t> lut(prec);
-  for (uint64_t i = 0; i < ns; ++i)
-    for (uint32_t j = cum[i]; j < cum[i + 1]; ++j) lut[j] = (uint32_t)i;
   const uint64_t nb = r.varint();
   if (r.err) return r.err;
   if (r.len - r.pos < nb) return DCB_ERR_EOF;
@@ -141,6 +144,17 @@ int host_symbols(Reader &r, uint32_t n, std::vector<uint32_t> &out) {
   uint32_t state = v + lbase;
   int64_t off = (int64_t)nb - (tg + 1);
   if (state >= lbase * 256u) return DCB_ERR_RANS_INIT;
+  if (raw_loc && scheme == 1) {  // every check the decode makes is behind us: the symbols themselves cannot fail
+    raw_loc->off = table_off;
+    raw_loc->bytes = r.pos - table_off;
+    raw_loc->mbl = mbl;
+    raw_loc->located = true;
+    return DCB_OK;
+  }
+  out.assign(n, 0);
+  std::vector<uint32_t> lut(prec);
+  for (uint64_t i = 0; i < ns; ++i)
+    for (uint32_t j = cum[i]; j < cum[i + 1]; ++j) lut[j] = (uint32_t)i;
   auto read = [&]() {
     while (state < lbase && off > 0) state = state * 256u + buf[--off];
     const uint32_t q = state >> pb, rem = state & (prec - 1u), s = lut[rem];
@@ -716,7 +730,7 @@ int dcb_host_edgebreaker(const uint8_t *buf, uint64_t len, uint64_t conn_off, ui
 // bit the other way round (:97) and cannot decode an ordinary mesh (SURVEY Appendix B).  Its range checks are kept:
 // an index may neither drop below zero (:99) nor pass int.MaxValue (:107).
 int dcb_host_sequential(const uint8_t *buf, uint64_t len, uint64_t conn_off, uint64_t *attr_section_off, uint32_t *n_points,
-                        std::vector<uint32_t> *faces) {
+                        std::vector<uint32_t> *faces, DcbSeqIndexLoc *loc) {
   Reader r{buf, len, conn_off};
   const uint64_t n_faces = r.varint();
   const uint64_t points = r.varint();
@@ -728,8 +742,18 @@ int dcb_host_sequential(const uint8_t *buf, uint64_t len, uint64_t conn_off, uin
   if (n_idx > 65536 + 4096 * (len - r.pos)) return DCB_ERR_CONNECTIVITY;
   std::vector<uint32_t> idx;
   if (method == 0) {
-    const int st = host_symbols(r, (uint32_t)n_idx, idx);
+    if (loc) {
+      loc->ckpt.clear();
+      loc->n_idx = n_idx;
+      loc->width = -1;
+    }
+    const int st = host_symbols(r, (uint32_t)n_idx, idx, loc && n_idx ? loc : nullptr);
     if (st) return st;
+    if (loc && loc->located) {
+      *attr_section_off = r.pos;
+      *n_points = (uint32_t)points;
+      return DCB_OK;
+    }
     int64_t cur = 0;
     for (uint64_t i = 0; i < n_idx; ++i) {
       const int64_t step = (int64_t)(idx[i] >> 1);
@@ -742,6 +766,55 @@ int dcb_host_sequential(const uint8_t *buf, uint64_t len, uint64_t conn_off, uin
     const int width = points < 256 ? 1 : points < 65536 ? 2 : points < (1u << 21) ? 0 : 4;
     if (width && (len - r.pos) / (uint64_t)width < n_idx) return DCB_ERR_EOF;
     if (!width && len - r.pos < n_idx) return DCB_ERR_EOF;  // a varint is at least one byte
+    if (loc) {
+      // locate only: fixed widths by arithmetic; varints by their terminator bytes (bit 7 clear), with Reader::varint's
+      // framing -- the run may not leave the buffer and a varint ends within 10 bytes
+      loc->ckpt.clear();
+      loc->n_idx = n_idx;
+      loc->off = r.pos;
+      loc->width = width;
+      if (width) {
+        r.pos += (uint64_t)width * n_idx;
+      } else {
+        // whole chunks branch-free (terminators counted, the longest continuation run tracked) while they cannot hold
+        // the last index; the chunk that does, byte by byte to the exact end
+        uint64_t ended = 0, run = 0;
+        while (ended < n_idx) {
+          if (r.pos >= len) return DCB_ERR_EOF;
+          loc->ckpt.push_back(ended);
+          const uint64_t n = std::min<uint64_t>(DCB_VARINT_CHUNK, len - r.pos);
+          const uint8_t *c = buf + r.pos;
+          uint64_t cnt = 0, worst = 0;
+          for (uint64_t i = 0; i < n; ++i) {
+            const uint64_t cont = c[i] >> 7;
+            run = cont ? run + 1 : 0;
+            worst = run > worst ? run : worst;
+            cnt += cont ^ 1u;
+          }
+          if (ended + cnt < n_idx && worst < 10 && n == DCB_VARINT_CHUNK) {
+            ended += cnt;
+            r.pos += n;
+            continue;
+          }
+          run = 0;  // redo this chunk exactly: the run in front of it ended at a terminator or is carried below
+          for (uint64_t q = r.pos; q > loc->off && (buf[q - 1] & 0x80u); --q) ++run;
+          for (uint64_t i = 0; i < n && ended < n_idx; ++i) {
+            if (c[i] & 0x80u) {
+              if (++run == 10) return DCB_ERR_EOF;
+            } else {
+              run = 0;
+              ++ended;
+            }
+            ++r.pos;
+          }
+        }
+      }
+      loc->bytes = r.pos - loc->off;
+      loc->located = true;
+      *attr_section_off = r.pos;
+      *n_points = (uint32_t)points;
+      return DCB_OK;
+    }
     idx.resize((size_t)n_idx);
     for (uint64_t i = 0; i < n_idx; ++i) {
       if (width == 0) {

@@ -18,6 +18,7 @@
 #include <algorithm>
 
 #include "dcb_internal.h"
+#include "dcb_jobs.cuh"
 #include "dcb_kernels.h"
 
 namespace {
@@ -26,45 +27,12 @@ constexpr uint32_t kThreads = 256;
 constexpr uint32_t kPerThread = 4;
 constexpr uint32_t kTile = kThreads * kPerThread;  // consecutive elements of one block iteration
 
-// last job j with prefix[j] <= i (prefix: n + 1 non-decreasing running sums, i < prefix[n])
-__device__ __forceinline__ uint32_t find_job(const uint64_t *prefix, uint32_t n, uint64_t i) {
-  uint32_t lo = 0, hi = n;
-  while (hi - lo > 1) {
-    const uint32_t mid = (lo + hi) >> 1;
-    if (prefix[mid] <= i) lo = mid;
-    else hi = mid;
-  }
-  return lo;
-}
-
-// f(job, index inside the job) over the elements [0, prefix[n]) of n jobs: one binary search per tile, then every
-// thread walks forward (jobs are contiguous, elements of a thread increase)
-template <typename F>
-__device__ __forceinline__ void for_each_element(const uint64_t *prefix, uint32_t n, F &&f) {
-  __shared__ uint32_t s_job;
-  const uint64_t total = prefix[n];
-  for (uint64_t t0 = (uint64_t)blockIdx.x * kTile; t0 < total; t0 += (uint64_t)gridDim.x * kTile) {
-    __syncthreads();
-    if (threadIdx.x == 0) s_job = find_job(prefix, n, t0);
-    __syncthreads();
-    uint32_t j = s_job;
-    uint64_t next = prefix[j + 1];
-#pragma unroll
-    for (uint32_t k = 0; k < kPerThread; ++k) {
-      const uint64_t i = t0 + k * kThreads + threadIdx.x;
-      if (i >= total) break;
-      while (i >= next) next = prefix[++j + 1];
-      f(j, i - prefix[j]);
-    }
-  }
-}
-
 __device__ __forceinline__ void fail_maps(StreamDesc *streams, uint32_t si) {
   atomicCAS(&streams[si].status, (int32_t)DCB_OK, (int32_t)DCB_ERR_MAPS);
 }
 
 __global__ void __launch_bounds__(kThreads) point_win_kernel(PointStage p, StreamDesc *streams, const uint8_t *__restrict__ maps) {
-  for_each_element(p.corner_prefix, p.n_maps, [&](uint32_t j, uint64_t ci) {
+  dcb_for_each_element<kThreads, kPerThread>(p.corner_prefix, p.n_maps, [&](uint32_t j, uint64_t ci) {
     const PointMapJob &m = p.maps[j];
     const uint32_t c = (uint32_t)ci;
     const uint32_t pt = reinterpret_cast<const uint32_t *>(maps + m.faces_off)[c];
@@ -78,7 +46,7 @@ __global__ void __launch_bounds__(kThreads) point_win_kernel(PointStage p, Strea
 }
 
 __global__ void __launch_bounds__(kThreads) point_resolve_kernel(PointStage p, StreamDesc *streams, const uint8_t *__restrict__ maps) {
-  for_each_element(p.point_prefix, p.n_maps, [&](uint32_t j, uint64_t pi) {
+  dcb_for_each_element<kThreads, kPerThread>(p.point_prefix, p.n_maps, [&](uint32_t j, uint64_t pi) {
     const PointMapJob &m = p.maps[j];
     uint32_t *slot = p.pmap + m.map_off + pi;
     const uint32_t win = *slot;
@@ -102,7 +70,7 @@ __device__ __forceinline__ void copy_unit(uint8_t *dst, const uint8_t *src) {
 __global__ void __launch_bounds__(kThreads) point_gather_kernel(PointStage p, const StreamDesc *streams, uint8_t *__restrict__ out) {
   uint32_t cur = 0xFFFFFFFFu;
   bool ok = false;
-  for_each_element(p.unit_prefix, p.n_gathers, [&](uint32_t j, uint64_t u) {
+  dcb_for_each_element<kThreads, kPerThread>(p.unit_prefix, p.n_gathers, [&](uint32_t j, uint64_t u) {
     const PointGatherJob &g = p.gathers[j];
     if (j != cur) {  // a thread meets few jobs: check the buffer's statuses once per job
       cur = j;

@@ -84,6 +84,7 @@ class Batch:
         self.n_bufs = n_bufs
         self._keep = keep  # input buffers must outlive upload
         self.point_order = False
+        self.faces_in_arena = False
 
     def free(self):
         if self.h:
@@ -148,6 +149,18 @@ class Batch:
         """DCB_ORDER_POINTS (points=True): attributes of Edgebreaker meshes come out as one row per point."""
         N.check(N.lib().dcb_set_output_order(self.h, N.DCB_ORDER_POINTS if points else N.DCB_ORDER_ENTRIES))
         self.point_order = bool(points)
+
+    def set_face_output(self, on: bool):
+        """DCB_FACES_ARENA (on=True): every mesh buffer's faces land in the output arena (face_info).  Set it before
+        host_connectivity, so that the plain indices of sequential meshes are decoded on the GPU."""
+        N.check(N.lib().dcb_set_face_output(self.h, N.DCB_FACES_ARENA if on else N.DCB_FACES_NONE))
+        self.faces_in_arena = bool(on)
+
+    def face_info(self, k):
+        """Where buffer k's faces lie in the output arena (dcb_face_info; all zero without a faces region)."""
+        fi = N.FaceInfo()
+        N.check(N.lib().dcb_get_face_info(self.h, k, C.byref(fi)))
+        return fi
 
     def set_mesh_faces(self, k, faces):
         """Faces (point ids) of Edgebreaker buffer k for point order; None: the NULL form (faces = corner_to_vertex
@@ -275,14 +288,18 @@ class DracoBatchDecoder:
         return s
 
     # ---- the reference-shaped API ----
-    def decode_batch(self, buffers: Sequence, point_order: bool = False) -> List[Draco]:
+    def decode_batch(self, buffers: Sequence, point_order: bool = False, faces_in_arena: bool = False) -> List[Draco]:
         """DecodeBatch: one `Draco` per input buffer; a malformed buffer carries its status and no
         attributes (the reference would have thrown for that buffer alone).  point_order: attributes of
-        Edgebreaker meshes hold one row per point, so that `values[faces]` is the mesh's triangle soup."""
+        Edgebreaker meshes hold one row per point, so that `values[faces]` is the mesh's triangle soup.
+        faces_in_arena: the faces come out of the output arena (sequential plain indices decoded on the GPU);
+        `Draco.faces` is then a view of it."""
         batch = self.index(buffers)
         try:
             if point_order:
                 batch.set_output_order(True)
+            if faces_in_arena:
+                batch.set_face_output(True)
             meshes = [k for k in range(batch.n_bufs) if batch.buffer_info(k).needs_connectivity]
             for k in meshes:
                 batch.host_connectivity(k)  # connectivity stays on the host (SURVEY 8f-1)
@@ -301,7 +318,11 @@ class DracoBatchDecoder:
             if bi.status not in (-1, -2) or bi.version_major:
                 hdr = DracoHeader(bi.version_major, bi.version_minor, bi.geometry_type, bi.encoder_method, bi.flags)
             d = Draco(header=hdr, status=bi.status, points_count=bi.n_points)
-            if bi.status == 0 and bi.geometry_type == 1:
+            if bi.status == 0 and bi.geometry_type == 1 and batch.faces_in_arena:
+                fi = batch.face_info(k)
+                f = out[fi.out_off: fi.out_off + fi.out_bytes].view(np.uint32).reshape(-1, 3)
+                d.faces = f if fi.n_faces else None
+            elif bi.status == 0 and bi.geometry_type == 1:
                 f = batch.faces(k)
                 d.faces = f if f.shape[0] else None  # None: the caller supplied the connectivity itself
             if bi.status == 0:

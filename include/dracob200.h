@@ -171,7 +171,8 @@ int dcb_set_mesh_maps(dcb_batch *b, int buf, int attr_decoder, const uint32_t *o
  * dcb_set_mesh_maps would.  A buffer whose connectivity is invalid or unsupported gets its own status. */
 int dcb_host_connectivity(dcb_batch *b, int buf);
 /* Faces (3 point ids each) of a mesh decoded by dcb_host_connectivity (Mesh.SetFace, MeshEdgeBreakerDecoder.cs:622-636).
- * faces == NULL: only *n_faces is written. */
+ * faces == NULL: only *n_faces is written.  DCB_ERR_STATE for a sequential mesh whose indices the GPU decodes into the
+ * output arena (DCB_FACES_ARENA): they are not on the host. */
 int dcb_mesh_faces(const dcb_batch *b, int buf, uint32_t *faces, uint64_t cap_faces, uint64_t *n_faces);
 /* Read back one installed map of an attributes decoder: which = 0 opposite, 1 corner_to_vertex, 2 data_to_corner,
  * 3 vertex_to_data (int32 bit patterns).  dst == NULL: only *n is written.  What a host needs to build the
@@ -206,6 +207,42 @@ int dcb_set_output_order(dcb_batch *b, int order);
  * dcb_index_finish, like the maps: afterwards, a call that turns a buffer's verdict (DCB_ERR_MAPS <-> ok) re-runs the
  * attribute indexing of the whole batch. */
 int dcb_set_mesh_faces(dcb_batch *b, int buf, const uint32_t *faces, uint64_t n_faces);
+
+/* Faces of meshes in the output arena.
+ *   DCB_FACES_NONE (default): faces stay on the host (dcb_mesh_faces); the arena holds attributes only.
+ *   DCB_FACES_ARENA: every mesh buffer that is ok after dcb_index_finish gets a faces region in the output arena:
+ *       3 u32 point ids per face (Mesh.Faces, the ids dcb_mesh_faces returns), behind the attributes of its shard, on a
+ *       128-byte boundary.  dcb_batch_out_bytes includes the regions; attribute out_off / out_bytes keep their meaning.
+ *       Independent of the output order: in DCB_ORDER_POINTS, values[faces] is the triangle soup, on the device.
+ *   Where the faces come from:
+ *     Edgebreaker    the faces installed by dcb_host_connectivity or dcb_set_mesh_faces (the NULL form: corner_to_vertex
+ *                    of attributes decoder 0); they travel with the maps and are copied into the region on the device.
+ *                    A buffer without faces fails with DCB_ERR_MAPS at dcb_index_finish.
+ *     sequential     dcb_host_connectivity called while the batch is in this mode.  Plain indices (connectivity
+ *                    method 1: 1, 2 or 4 bytes, or varints for 65536 <= points < 2^21) are only LOCATED on the host --
+ *                    framing errors give the statuses the host decode gives -- and decoded on the GPU; so are Raw index
+ *                    differences (method 0): one more Raw rANS stream, then a scan that fails the buffer alone with
+ *                    DCB_ERR_CONNECTIVITY when an index drops below 0 or passes INT32_MAX.  dcb_mesh_faces then returns
+ *                    DCB_ERR_STATE.  Tagged index differences cannot be located without decoding them (their bit area
+ *                    has no length prefix, SymbolDecoding.cs:37-49): they are decoded on the host as before and travel
+ *                    with the maps.  A sequential buffer whose connectivity the caller installed with
+ *                    dcb_set_attr_section has no faces: DCB_ERR_MAPS.
+ *   dcb_decode_scatter has no slot for faces: DCB_ERR_STATE for a batch in this mode. */
+#define DCB_FACES_NONE 0
+#define DCB_FACES_ARENA 1
+/* Before the first dcb_upload / dcb_decode* of the batch (DCB_ERR_STATE afterwards); re-lays out the output arena.
+ * Set it before dcb_host_connectivity for the sequential indices to be decoded on the GPU; once dcb_host_connectivity has
+ * located indices for the GPU, turning the mode off fails with DCB_ERR_STATE (those faces are not on the host). */
+int dcb_set_face_output(dcb_batch *b, int mode);
+typedef struct dcb_face_info {
+  uint64_t out_off;    /* offset of the faces region in the output arena, 128-byte aligned */
+  uint64_t out_bytes;  /* 12 * n_faces: u32 point ids, 3 per face */
+  uint64_t n_faces;
+  int32_t source;      /* 0 none (point cloud, failed buffer, mode off), 1 decoded on the host, 2 decoded on the GPU */
+  int32_t reserved;
+} dcb_face_info;
+/* All zero for a batch in DCB_FACES_NONE and for buffers without a faces region. */
+int dcb_get_face_info(const dcb_batch *b, int buf, dcb_face_info *out);
 
 /* Phase 2 (device).  One-call form: host->device copy, kernels, device->host copy.
  * host_out: one arena of dcb_batch_out_bytes() bytes laid out by dcb_attr_info.out_off; host_dbg may be

@@ -1730,6 +1730,12 @@ int decode_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index, uint8_t *
     std::vector<Group *> gs{&g};
     plan_rans_groups(gs, num_sms, (uint32_t)sh.share);
     if (g.table_global) return DCB_ERR_STATE;  // cannot happen: tag alphabets are tiny (<= 2^24 guarded by table size)
+    if (env_flags().debug_plan)
+      fprintf(stderr, "[dcb plan] tag group compact=%u prec=%u entries=%u: %u streams, %llu symbols, k=%u lut=%uB lutb=%uB ent=%uB "
+                      "lanes=%u pairs=%u split=%u direct=%u global=%d rec_ka=%u rec=%uB (need x8: %u %u %u %u, exc %u)\n",
+              g.compact, g.prec_bits, g.entries, (uint32_t)g.order.size(), (unsigned long long)g.total_symbols, g.lut_shift, g.lut_bytes,
+              g.lutb_bytes, g.ent_bytes, g.lanes, g.pairs, g.split, g.direct, (int)g.table_global, g.rec_ka, g.rec_bytes, g.rec_max[0],
+              g.rec_max[1], g.rec_max[2], g.rec_max[3], g.exc_all);
     int rc = ensure_order(sh, g.order.size() + blocked.size());
     if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(sh.d_order, g.order.data(), g.order.size() * 4, cudaMemcpyHostToDevice, st));

@@ -55,7 +55,9 @@ def normalize_probs(freq, prec_bits):
     return prob
 
 
-def table_bytes(prob):
+def table_bytes(prob, pad=0):
+    """RANS_TABLE.  pad: write that many extra bytes by giving the first non-zero probabilities a longer encoding than
+    they need (a zero extra byte); the decoder reads the same table, the payload behind it moves by `pad` bytes."""
     out = bytearray(varint(len(prob)))
     i = 0
     n = len(prob)
@@ -69,18 +71,25 @@ def table_bytes(prob):
             i += off + 1
         else:
             extra = 0 if p < (1 << 6) else (1 if p < (1 << 14) else 2)
+            more = min(pad, 2 - extra)
+            extra += more
+            pad -= more
             out.append(((p << 2) & 0xFC) | extra)
             for b in range(extra):
                 out.append((p >> (8 * (b + 1) - 2)) & 0xFF)
             i += 1
+    assert pad == 0, "not enough entries to pad the table"
     return bytes(out)
 
 
-def rans_payload(symbols, prob, prec_bits):
+def rans_payload(symbols, prob, prec_bits, final_state=None):
+    """rANS payload of `symbols` under `prob`.  final_state: the state the decoder ends in (the encoder's initial
+    state, in [L, 256 L)); L by default."""
     P = 1 << prec_bits
     l_base = 4 * P
     cum = np.concatenate([[0], np.cumsum(prob)])
-    state = l_base
+    state = l_base if final_state is None else int(final_state)
+    assert l_base <= state < 256 * l_base
     buf = bytearray()
     for s in reversed([int(x) for x in symbols]):
         p = int(prob[s])
@@ -119,6 +128,58 @@ def symbols_raw(symbols, mbl=None):
     return bytes([1, mbl]) + table_bytes(prob) + varint(len(pay)) + pay
 
 
+def _check_table(prob, prec_bits, symbols):
+    prob = [int(p) for p in prob]
+    assert sum(prob) == 1 << prec_bits, "probabilities must sum to 2^%d" % prec_bits
+    assert all(0 <= s < len(prob) and prob[s] > 0 for s in symbols), "a symbol without probability"
+    return prob
+
+
+def symbols_raw_table(symbols, prob, mbl, final_state=None, pad=0):
+    """SYMBOLS field, Raw scheme, with a probability table the caller chooses (not derived from the symbols): any
+    table summing to 2^precision(mbl), symbols with a probability that never occur included."""
+    symbols = [int(s) for s in symbols]
+    if not symbols:
+        return b""
+    pb = rans_precision(mbl)
+    prob = _check_table(prob, pb, symbols)
+    pay = rans_payload(symbols, prob, pb, final_state)
+    return bytes([1, mbl]) + table_bytes(prob, pad) + varint(len(pay)) + pay
+
+
+def tagged_bits(symbols, nc, tags):
+    """The LSB-first bit area of a Tagged stream: per point, nc fields of (tags[i] & 0xFF) bits.  Returns (bytes, bits)."""
+    acc, nacc, bits, total = 0, 0, bytearray(), 0
+    for i, t in enumerate(tags):
+        w = int(t) & 0xFF
+        for c in range(nc):
+            acc |= (int(symbols[i * nc + c]) & ((1 << w) - 1)) << nacc
+            nacc += w
+            total += w
+            while nacc >= 8:
+                bits.append(acc & 0xFF)
+                acc >>= 8
+                nacc -= 8
+    if nacc:
+        bits.append(acc & 0xFF)
+    return bytes(bits), total
+
+
+def symbols_tagged_table(symbols, nc, tag_prob, tags=None, final_state=None):
+    """SYMBOLS field, Tagged scheme, with a tag table the caller chooses (precision 12).  tags: the tag symbol of every
+    point (default: the bit length of its largest value); the decoder uses tag & 0xFF as the field width."""
+    symbols = [int(s) for s in symbols]
+    if not symbols:
+        return b""
+    n = len(symbols) // nc
+    if tags is None:
+        tags = [max(1, max(symbols[i * nc:(i + 1) * nc]).bit_length()) for i in range(n)]
+    tags = [int(t) for t in tags]
+    tag_prob = _check_table(tag_prob, 12, tags)
+    pay = rans_payload(tags, tag_prob, 12, final_state)
+    return bytes([0]) + table_bytes(tag_prob) + varint(len(pay)) + pay + tagged_bits(symbols, nc, tags)[0]
+
+
 def symbols_tagged(symbols, nc):
     """SYMBOLS field, Tagged scheme (scheme byte 0): one bit-length tag per point, LSB-first bit fields."""
     symbols = [int(s) for s in symbols]
@@ -148,8 +209,10 @@ def symbols_tagged(symbols, nc):
     return bytes([0]) + table_bytes(prob) + varint(len(pay)) + pay + bytes(bits)
 
 
-def portable_int(corr, nc, pred_method=0, transform=1, scheme="raw", pred_data=b"", zig=True, num_bytes=None, mbl=None):
-    """PORTABLE(int-like): corrections (flat, entry-major) -> bytes."""
+def portable_int(corr, nc, pred_method=0, transform=1, scheme="raw", pred_data=b"", zig=True, num_bytes=None, mbl=None,
+                 prob=None, tag_prob=None, tags=None):
+    """PORTABLE(int-like): corrections (flat, entry-major) -> bytes.  prob (Raw, with mbl) / tag_prob (Tagged, with
+    optional tags): a caller-chosen table instead of one derived from the symbols."""
     out = bytearray(struct.pack("<b", pred_method))
     if pred_method != -2:
         out += struct.pack("<b", transform)
@@ -161,7 +224,10 @@ def portable_int(corr, nc, pred_method=0, transform=1, scheme="raw", pred_data=b
             out += int(s & ((1 << (8 * num_bytes)) - 1)).to_bytes(num_bytes, "little") if num_bytes else b""
     else:
         out.append(1)
-        out += symbols_raw(syms, mbl) if scheme == "raw" else symbols_tagged(syms, nc)
+        if scheme == "raw":
+            out += symbols_raw(syms, mbl) if prob is None else symbols_raw_table(syms, prob, mbl)
+        else:
+            out += symbols_tagged(syms, nc) if tag_prob is None else symbols_tagged_table(syms, nc, tag_prob, tags)
     out += pred_data
     return bytes(out)
 

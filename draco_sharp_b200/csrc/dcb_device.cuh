@@ -337,27 +337,31 @@ struct RansLane {
   uint32_t d_freq, d_off, d_ent;
   const uint8_t *ent0;  // entry region (generic pointer: shared or global)
   const uint8_t *lut0;  // GLOBAL only
-  // byte supply
-  const uint8_t *arena;
-  int64_t end;          // arena offset one past the first unread byte at init
+  // byte supply: the payload is requested into the ring downwards from its end rounded up to 16 bytes
+  const uint8_t *lo_ptr;  // lowest byte requested so far
+  uint32_t lo;            // low 32 bits of its arena offset (a multiple of 16)
   uint32_t p1_init;
-  uint32_t off_init;    // unread payload bytes at init (BufferOffset)
-  int64_t loaded_lo;
+  uint32_t off_init;      // unread payload bytes at init (BufferOffset)
 
   __device__ __forceinline__ uint32_t consumed() const { return p1_init - p1; }
   __device__ __forceinline__ uint32_t bytes_left() const { return off_init - consumed(); }
 
+  // Requests the 16-byte chunks that keep the ring filled down to 128 bytes below the read position (at most
+  // MAX_CHUNKS of them) and commits them as one group.  The chunk count comes from one 32-bit distance, every chunk has
+  // a predicate of its own and its source is a fixed offset from lo_ptr: no branch and no 64-bit compare chain (the main
+  // loops call this once per 4 entries).
   template <int MAX_CHUNKS>
   __device__ __forceinline__ void top_up() {
-    const int64_t ptr = end - (int64_t)consumed();
-    const int64_t floor_lo = ((ptr + 15) & ~15ll) - (int64_t)DCB_RING_BYTES;
+    const uint32_t floor_lo = ((p1 + 16u) & ~15u) - DCB_RING_BYTES;  // never above lo
+    const uint32_t n = min((lo - floor_lo) >> 4, (uint32_t)MAX_CHUNKS);
 #pragma unroll
     for (int k = 0; k < MAX_CHUNKS; ++k) {
-      if (loaded_lo - 16 >= floor_lo) {
-        loaded_lo -= 16;
-        cp_async16(ring | ((uint32_t)loaded_lo & (DCB_RING_BYTES - 1u)), arena + loaded_lo);
-      }
+      asm volatile("{\n .reg .pred p;\n setp.gt.u32 p, %2, %3;\n @p cp.async.ca.shared.global [%0], [%1], 16;\n}\n"
+                   ::"r"(ring | ((lo - 16u * (k + 1)) & (DCB_RING_BYTES - 1u))), "l"(lo_ptr - 16 * (k + 1)), "r"(n),
+                   "r"((uint32_t)k) : "memory");
     }
+    lo -= n << 4;
+    lo_ptr -= n << 4;
     cp_async_commit();
   }
 
@@ -611,11 +615,11 @@ struct RansLane {
     x = v + L;
     if (x >= L * 256u) return DCB_ERR_RANS_INIT;
     off_init = (uint32_t)(n - (tag + 1));
-    arena = arena_;
-    end = (int64_t)(d.payload_off + off_init);
+    const uint64_t end = d.payload_off + off_init;  // arena offset one past the first unread byte
     p1_init = (uint32_t)end - 1u;
     p1 = p1_init;
-    loaded_lo = (end + 15) & ~15ll;
+    lo_ptr = arena_ + ((end + 15u) & ~15ull);
+    lo = ((uint32_t)end + 15u) & ~15u;
     return DCB_OK;
   }
   __device__ __forceinline__ void init_ring(uint32_t ring_addr) {
@@ -866,41 +870,57 @@ __device__ __forceinline__ void decode_entry(RansLane<T, TG> &rl, const TableGeo
 // left to itself clumps that independent work (profiles/r2_rans_raw_fused_c2_step_cycles.txt); the gate of
 // step_lean<.., true> pins the post-processing of symbol j-1 in front of the probe of symbol j+1.
 // PROBE: 1 two-region LUT (step_lean), 2 direct slot LUT (step_lean_direct).  COMPACT: the table has a value map.
-template <int NCP, int MODE, bool LAST, int PROBE, bool COMPACT>
+// One call decodes E entries from entry 4*g on (E a multiple of 4; the LAST group: 4).  Every 4 entries are stored
+// and the byte ring is topped up in the body; the wait for those chunks sits in front of the next quad's first byte
+// window, not between the last state update and the next renormalisation.  The caller has checked that the bytes of
+// the group, and for a middle group those of the next group's first symbol, are there.
+template <int NCP, int MODE, bool LAST, int PROBE, bool COMPACT, int E = 4>
 __device__ __forceinline__ void lean_sp_group(RansLane<uint16_t, false> &rl, const PostParams &pp, uint8_t *optr, uint32_t g,
                                               int32_t *prev, uint32_t &ca_prev, uint32_t &gate, uint32_t zero) {
-  constexpr int kSyms = 4 * NCP;
-  float f[kSyms];
-  int32_t v[4][NCP];
+  static_assert(E % 4 == 0 && (!LAST || E == 4), "groups of whole quads; the LAST group is one quad");
+  constexpr int kQuad = 4 * NCP;  // symbols of 4 entries
+  constexpr int kSyms = E * NCP;
 #pragma unroll
-  for (int s = 1; s <= kSyms; ++s) {
-    uint32_t ca = 0;
-    if (!(LAST && s == kSyms)) {
-      const int sp = s % kSyms;  // position inside its own group: the windows restart with every group (as run_stream_lean)
-      if (sp % 3 == 0) rl.window_open();
-      if (PROBE == 2) ca = (sp % 3 == 0) ? rl.template step_lean_direct<true>(gate, zero) : rl.template step_lean_direct<false>(gate, zero);
-      else ca = (sp % 3 == 0) ? rl.template step_lean<true, true>(gate, zero) : rl.template step_lean<false, true>(gate, zero);
-      if (sp % 3 == 2 || sp == kSyms - 1) rl.window_close();
+  for (int qd = 0; qd < E / 4; ++qd) {
+    float f[kQuad];
+    int32_t v[4][NCP];
+#pragma unroll
+    for (int t = 1; t <= kQuad; ++t) {
+      const int s = qd * kQuad + t;
+      uint32_t ca = 0;
+      if (!(LAST && s == kSyms)) {
+        const int sp = s % kSyms;  // position inside its own group: the windows restart with every group (as run_stream_lean)
+        if (sp % 3 == 0) {
+          // the quad's first window: every chunk committed before the previous top-up has landed
+          if (sp != 0 && sp <= qd * kQuad + 3) cp_async_wait<1>();
+          rl.window_open();
+        }
+        if (PROBE == 2) ca = (sp % 3 == 0) ? rl.template step_lean_direct<true>(gate, zero) : rl.template step_lean_direct<false>(gate, zero);
+        else ca = (sp % 3 == 0) ? rl.template step_lean<true, true>(gate, zero) : rl.template step_lean<false, true>(gate, zero);
+        if (sp % 3 == 2 || sp == kSyms - 1) rl.window_close();
+      }
+      const int c = (t - 1) % NCP;
+      const int32_t corr = COMPACT ? rl.value_at(ca_prev) : zigzag_dec((ca_prev - rl.cum_addr) >> 1);
+      if (MODE == 3 || MODE == 4) prev[c] = corr;  // corrections for oct_chain / the parallelogram kernels
+      else prev[c] = wrap_regular(prev[c], corr, pp.mn, pp.mx, pp.max_diff);
+      if (MODE == 1) {
+        f[t - 1] = pp.dequant(prev[c], c);
+        gate = __float_as_uint(f[t - 1]);
+      } else {
+        v[(t - 1) / NCP][c] = prev[c];
+        gate = (uint32_t)corr;  // the value map's load: the integer wrap behind it is three ALU levels
+      }
+      ca_prev = ca;
     }
-    const int c = (s - 1) % NCP;
-    const int32_t corr = COMPACT ? rl.value_at(ca_prev) : zigzag_dec((ca_prev - rl.cum_addr) >> 1);
-    if (MODE == 3 || MODE == 4) prev[c] = corr;  // corrections for oct_chain / the parallelogram kernels
-    else prev[c] = wrap_regular(prev[c], corr, pp.mn, pp.mx, pp.max_diff);
+    const uint32_t gq = g + (uint32_t)qd;
     if (MODE == 1) {
-      f[s - 1] = pp.dequant(prev[c], c);
-      gate = __float_as_uint(f[s - 1]);
-    } else {
-      v[(s - 1) / NCP][c] = prev[c];
-      gate = (uint32_t)corr;  // the value map's load: the integer wrap behind it is three ALU levels
-    }
-    ca_prev = ca;
-  }
-  if (MODE == 1) {
-    float4 *o = reinterpret_cast<float4 *>(reinterpret_cast<float *>(optr) + (uint64_t)g * kSyms);
+      float4 *o = reinterpret_cast<float4 *>(reinterpret_cast<float *>(optr) + (uint64_t)gq * kQuad);
 #pragma unroll
-    for (int k = 0; k < NCP; ++k) o[k] = make_float4(f[4 * k], f[4 * k + 1], f[4 * k + 2], f[4 * k + 3]);
-  } else {
-    store_group4<NCP>(pp, store_of<MODE>(pp), dsize_of<MODE>(pp), optr, (uint64_t)g * 4, v);
+      for (int k = 0; k < NCP; ++k) o[k] = make_float4(f[4 * k], f[4 * k + 1], f[4 * k + 2], f[4 * k + 3]);
+    } else {
+      store_group4<NCP>(pp, store_of<MODE>(pp), dsize_of<MODE>(pp), optr, (uint64_t)gq * 4, v);
+    }
+    rl.template top_up<(4 * NCP * 3 + 15) / 16 + 1>();
   }
 }
 

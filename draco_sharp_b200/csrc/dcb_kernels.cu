@@ -118,39 +118,51 @@ __device__ __forceinline__ void run_stream_lean(RansLane<uint16_t, false> &rl, c
   run_tail<NCP, uint16_t, false, false, MODE, 2, true>(rl, geom, pp, optr, nullptr, 0u, n_entries, g, prev);
 }
 
-// Software-pipelined lean main loop (lean_sp_group, dcb_device.cuh) around the two-region LUT.
-template <int NCP, int MODE>
+// Software-pipelined lean main loop (lean_sp_group, dcb_device.cuh) around the two-region LUT, E entries per group.
+// The bounds are tested once per RUN of groups: a run is as many groups as the lane of `live` with the fewest bytes
+// left cannot run out of (step_lean shifts in at most two bytes per symbol), so the groups need no test of their own
+// and the loop counter is warp-uniform.  A lane whose own budget is down to zero leaves the run and finishes alone: the
+// LAST group, then the careful tail.  `live`: the lanes of the warp that call this.
+template <int NCP, int MODE, int E>
 __device__ __forceinline__ void run_stream_lean_sp(RansLane<uint16_t, false> &rl, const TableGeom &geom, const PostParams &pp,
-                                                   uint8_t *optr, uint32_t n_entries, uint32_t g_min, uint32_t zero) {
+                                                   uint8_t *optr, uint32_t n_entries, uint32_t g_min, uint32_t zero,
+                                                   uint32_t live) {
   int32_t prev[NCP];
   const int32_t p0 = 0 > pp.mx ? pp.mx : (0 < pp.mn ? pp.mn : 0);  // the clamp the first prediction (zero) would get
 #pragma unroll
   for (int c = 0; c < NCP; ++c) prev[c] = p0;
-  constexpr uint32_t kGroupBytes = 4u * NCP * 3u;
-  uint32_t g = 0;
-  if (g_min > 0 && rl.bytes_left() >= kGroupBytes) {
+  constexpr uint32_t kQuads = E / 4;
+  constexpr uint32_t kMaxGroupBytes = 2u * E * NCP;
+  constexpr uint32_t kMargin = 2u * 4u * NCP;  // the symbol in the open window + symbols 1.. of the LAST group
+  uint32_t g = 0;  // in groups of 4 entries
+  const bool fast = g_min > 0 && rl.bytes_left() >= kMargin;
+  uint32_t run = __ballot_sync(live, fast);
+  if (fast) {
     // prologue: symbol 0 of group 0 (the window stays open: symbols 1 and 2 follow in the loop)
     rl.window_open();
     uint32_t ca_prev = rl.template step_lean<true>();
     uint32_t gate = 0;
-    // a group in the middle decodes symbols 1..12 past its base (one ahead) and needs the bytes of the next group's
-    // first symbol: 2 more than kGroupBytes, and p1 lags the open window by at most 2
-    while (g + 1 < g_min && rl.bytes_left() >= 2u * kGroupBytes + 4u) {
-      lean_sp_group<NCP, MODE, false, 1, true>(rl, pp, optr, g, prev, ca_prev, gate, zero);
-      ++g;
-      rl.template top_up<(kGroupBytes + 15) / 16 + 1>();
-      cp_async_wait<1>();
+    for (;;) {
+      // a middle group leaves at least one group of 4 entries (g_min is the warp's minimum) for the LAST group
+      const uint32_t by_bytes = rl.bytes_left() >= kMargin + kMaxGroupBytes ? (rl.bytes_left() - kMargin) / kMaxGroupBytes : 0u;
+      const uint32_t mine = min(by_bytes, (g_min - 1u - g) / kQuads);
+      run = __ballot_sync(run, mine > 0);
+      if (mine == 0) break;
+      const uint32_t n = __reduce_min_sync(run, mine);
+      for (uint32_t i = 0; i < n; ++i) {
+        lean_sp_group<NCP, MODE, false, 1, true, E>(rl, pp, optr, g, prev, ca_prev, gate, zero);
+        g += kQuads;
+      }
     }
     lean_sp_group<NCP, MODE, true, 1, true>(rl, pp, optr, g, prev, ca_prev, gate, zero);
     ++g;
-    rl.template top_up<(kGroupBytes + 15) / 16 + 1>();
     cp_async_wait<1>();
   }
   rl.prefetch();  // the careful tail reads through the two-word peek
   run_tail<NCP, uint16_t, false, false, MODE, 2, true>(rl, geom, pp, optr, nullptr, 0u, n_entries, g, prev);
 }
 
-template <int NCP, typename T, bool DUMP, bool TABLE_GLOBAL, int MODE, int TAB>
+template <int NCP, typename T, bool DUMP, bool TABLE_GLOBAL, int MODE, int TAB, int E>
 __global__ void __launch_bounds__(32) rans_raw_fused_kernel(const uint8_t *__restrict__ arena, StreamDesc *streams,
                                                             const uint32_t *__restrict__ order, uint32_t n_streams,
                                                             uint32_t lanes, TableGeom geom, uint8_t *__restrict__ out,
@@ -224,7 +236,8 @@ __global__ void __launch_bounds__(32) rans_raw_fused_kernel(const uint8_t *__res
   uint32_t g_min = n_entries ? (n_entries >> 2) : 0xFFFFFFFFu;
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) g_min = min(g_min, __shfl_xor_sync(0xffffffffu, g_min, o));
-  if (n_entries == 0) return;  // idle lane, empty or failed stream (no warp-level operation below)
+  const uint32_t live = __ballot_sync(0xffffffffu, n_entries != 0);
+  if (n_entries == 0) return;  // idle lane, empty or failed stream (below, warp-level operations use `live`)
   rl.fill_lut(geom, lut, lutb, blk, ent, use_split);
   rl.init_ring(smem_base + lay.ring0 + lane * DCB_RING_BYTES);
 
@@ -251,7 +264,7 @@ __global__ void __launch_bounds__(32) rans_raw_fused_kernel(const uint8_t *__res
     // lean main loop: every active lane of the warp decodes a regular delta + wrap stream through the two-region LUT
     if (use_lean) {
 #ifndef DCB_NO_LEAN_SP
-      run_stream_lean_sp<NCP, MODE>(rl, geom, pp, optr, n_entries, g_min, blockIdx.y);  // blockIdx.y: an opaque zero
+      run_stream_lean_sp<NCP, MODE, E>(rl, geom, pp, optr, n_entries, g_min, blockIdx.y, live);  // blockIdx.y: an opaque zero
       return;
 #endif
       if constexpr (MODE == 1 || MODE == 2) {
@@ -908,9 +921,23 @@ static uint32_t no_split_bit() {
   return bit;
 }
 
-template <int NCP, typename T, bool DUMP, bool TG, int MODE, int TAB = 0>
+// entries per group of the software-pipelined lean loop (run_stream_lean_sp); DCB_LEAN_GROUP=4|8|16 picks another
+// instance (A/B measurements, tests), any other value keeps the default.  8 measures best on configs[1] (DESIGN 3.1,
+// profiles/lean_group_b200.jsonl): 4 pays the group boundary twice as often, 16's unrolled body (~2,900 SASS
+// instructions, 46 KB) runs 30 % slower than 8's.
+constexpr int kLeanGroup = 8;
+static int lean_group() {
+  static const int e = [] {
+    const char *v = getenv("DCB_LEAN_GROUP");
+    const int x = v ? atoi(v) : 0;
+    return (x == 4 || x == 8 || x == 16) ? x : kLeanGroup;
+  }();
+  return e;
+}
+
+template <int NCP, typename T, bool DUMP, bool TG, int MODE, int TAB = 0, int E = 4>
 static cudaError_t launch_raw_t(const RansLaunch &p, const DevArenas &a, cudaStream_t st) {
-  auto k = rans_raw_fused_kernel<NCP, T, DUMP, TG, MODE, TAB>;
+  auto k = rans_raw_fused_kernel<NCP, T, DUMP, TG, MODE, TAB, E>;
   const uint32_t smem_bytes = dcb_rans_smem_bytes(p, TG);
   if (smem_bytes > 48 * 1024) {
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes);
@@ -936,14 +963,19 @@ static cudaError_t launch_raw_n(const RansLaunch &p, bool table_global, const De
 cudaError_t dcb_launch_rans_raw(const RansLaunch &p, int ncp, bool wide, bool table_global, const DevArenas &a,
                                 cudaStream_t st) {
 #ifdef DCB_DEV_ONLY_C2  // development builds (SASS inspection of the headline instantiation alone): never shipped
-  return launch_raw_t<3, uint16_t, false, false, 1, 2>(p, a, st);
+  return launch_raw_t<3, uint16_t, false, false, 1, 2, kLeanGroup>(p, a, st);
 #else
-  // specialised hot shapes (u16 tables in shared memory, no debug dump)
+  // specialised hot shapes (u16 tables in shared memory, no debug dump); compact tables may take the lean loop
   if (!wide && !table_global && !p.dump) {
 #define DCB_SPEC(M, N)                                                                           \
-  if (p.mode == M && ncp == N)                                                                   \
-    return p.compact ? launch_raw_t<N, uint16_t, false, false, M, 2>(p, a, st)                   \
-                     : launch_raw_t<N, uint16_t, false, false, M, 1>(p, a, st);
+  if (p.mode == M && ncp == N) {                                                                 \
+    if (!p.compact) return launch_raw_t<N, uint16_t, false, false, M, 1>(p, a, st);              \
+    switch (lean_group()) {                                                                      \
+      case 4: return launch_raw_t<N, uint16_t, false, false, M, 2, 4>(p, a, st);                 \
+      case 16: return launch_raw_t<N, uint16_t, false, false, M, 2, 16>(p, a, st);               \
+      default: return launch_raw_t<N, uint16_t, false, false, M, 2, 8>(p, a, st);                \
+    }                                                                                            \
+  }
     DCB_SPEC(1, 3)
     DCB_SPEC(1, 2)
     DCB_SPEC(2, 3)

@@ -280,14 +280,11 @@ __device__ __forceinline__ uint32_t fused_direct_loop(RansLane<uint16_t, false> 
     uint32_t ca_prev = rl.template step_lean_direct<true>(0u, zero);
     uint32_t gate = 0;
     while (g + 1 < g_min && rl.bytes_left() >= 2u * kGroupBytes + 4u) {
-      lean_sp_group<NCP, MODE, false, 2, COMPACT>(rl, pp, optr, g, prev, ca_prev, gate, zero);
+      lean_sp_group<NCP, MODE, false, 2, COMPACT>(rl, pp, optr, g, prev, ca_prev, gate, zero);  // tops the ring up
       ++g;
-      rl.template top_up<(kGroupBytes + 15) / 16 + 1>();
-      cp_async_wait<1>();
     }
     lean_sp_group<NCP, MODE, true, 2, COMPACT>(rl, pp, optr, g, prev, ca_prev, gate, zero);
     ++g;
-    rl.template top_up<(kGroupBytes + 15) / 16 + 1>();
     cp_async_wait<1>();
   }
   rl.prefetch();  // the careful tail reads through the two-word peek

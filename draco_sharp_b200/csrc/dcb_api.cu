@@ -46,12 +46,10 @@ inline uint64_t align_up(uint64_t v, uint64_t a) { return (v + a - 1) / a * a; }
 
 // experiment / test switches, read once per process (never per stream or per decode)
 struct EnvFlags {
-  bool no_par_post, no_fanout, debug_plan, debug_timing, lutb_full, rans_pc, no_direct, no_fast_tagged, no_threads;
-  int ctas_per_sm, pairs, par_run, rec_ka;
+  bool debug_plan, debug_timing, lutb_full, rans_pc, no_direct, no_fast_tagged, no_threads;
+  int rec_ka;
   bool no_rec, split;
   EnvFlags() {
-    no_par_post = getenv("DCB_NO_PAR_POST") != nullptr;
-    no_fanout = getenv("DCB_NO_FANOUT") != nullptr;
     debug_plan = getenv("DCB_DEBUG_PLAN") != nullptr;
     debug_timing = getenv("DCB_DEBUG_TIMING") != nullptr;
     lutb_full = getenv("DCB_LUTB_FULL") != nullptr;
@@ -59,9 +57,6 @@ struct EnvFlags {
     no_direct = getenv("DCB_NO_DIRECT") != nullptr;  // never plan the direct slot LUT
     no_threads = getenv("DCB_NO_THREADS") != nullptr;          // multi-device decodes on the calling thread only
     no_fast_tagged = getenv("DCB_NO_FAST_TAGGED") != nullptr;  // always fetch the resumed walks before classifying
-    ctas_per_sm = getenv("DCB_CTAS_PER_SM") ? atoi(getenv("DCB_CTAS_PER_SM")) : 0;
-    pairs = getenv("DCB_PAIRS") ? atoi(getenv("DCB_PAIRS")) : 0;
-    par_run = getenv("DCB_PAR_RUN") ? atoi(getenv("DCB_PAR_RUN")) : 0;  // run length of par_post2_kernel, in chunks
     no_rec = getenv("DCB_REC") == nullptr;                               // the bucket-record kernels are opt-in (DCB_REC=1): measured
                                                                          // slower than the fused kernel at full residency (DESIGN 3.1)
     split = getenv("DCB_SPLIT") != nullptr;                              // warp-pair kernels: consumers on their own sub-partition
@@ -130,18 +125,21 @@ struct BufRec {
   uint64_t n_faces = 0, face_off = 0;  // face_off: shard-local offset of the faces region
 };
 
-struct Group {            // one kernel launch (or a few, for global tables)
-  int kind;               // 0 raw, 1 tag, 2 serial post, 3 para, 4 copy
+struct Stage {                 // the streams of one stage's launch
+  std::vector<uint32_t> order;
+  uint64_t order_off = 0;      // offset (in uint32) inside the shard's device order array
+  uint32_t max_entries = 0;
+  uint64_t max_bytes = 0;
+};
+
+struct Group : Stage {    // one rANS launch (or a few, for global tables) and its geometry
+  bool tag;               // the tags of Tagged streams (16 symbols per step), not the values of Raw ones
   int ncp;
   bool wide, table_global;
   uint32_t compact, prec_bits, entries, exc, lut_shift, lut_bytes, lutb_bytes, ent_bytes, lanes, zig, mode;
   uint32_t pairs;         // chain/consumer warp pairs per CTA (0: the single-warp kernels of dcb_kernels.cu)
   uint32_t direct;        // direct slot LUT (warp-pair kernels)
-  uint32_t ctas_per_sm;   // planned residency (reporting)
-  uint64_t total_symbols, max_bytes;
-  uint32_t max_entries;
-  std::vector<uint32_t> order;
-  uint64_t order_off;     // offset (in uint32) inside the shard's device order array
+  uint64_t total_symbols;
   // earliest / latest 128-slot block (over the group's streams) holding the first entry narrower than 2^k slots
   uint32_t nb_min[8], nb_max[8];
   bool nb_any;
@@ -160,6 +158,28 @@ struct Group {            // one kernel launch (or a few, for global tables)
     for (int j = 0; j < 4; ++j) rec_max[j] = nb_any ? std::max<uint32_t>(rec_max[j], s.rec_need[j]) : s.rec_need[j];
     exc_all = std::max(exc_all, s.n_active - std::min(s.n_active, s.dense_prefix));
     nb_any = true;
+  }
+};
+
+// The launches of one decode of a shard after its tag rounds, planned on the host from the ready streams (plan_shard):
+// built without a CUDA call, then issued by decode_shard.  Stage arrays are indexed by component count 1..4.
+struct ShardPlan {
+  std::vector<Group> raw;  // Raw rANS groups, in RawKey order
+  int dom = -1;            // raw[dom]: the group with the most symbols (statistics and kernel name of the decode)
+  Stage post[5], para[5], cmp[5], par[5], copy, octs, octc, tex, geo, wide;
+  struct ParPost {         // par_post2_kernel of par[n]: per group the run prefix of its streams and one ticket word
+    bool delta = false;
+    uint32_t run_len = 1, claim = 1, rounds = 0;
+    std::vector<uint32_t> runs;
+    uint64_t runs_off = 0;  // offset (in uint32) of `runs` inside the device order array
+  } pp[5];
+  bool has_para = false;        // mesh kernels validate the caller's maps on the device
+  bool side_followers = false;  // oct_chain / oct_unit run next to the rANS kernels of other groups
+  std::vector<uint32_t> order;  // the device order array: every stage list, then the runs
+  bool flag_kernels() const {   // crease flags / flip bits of the 8f-3 predictors
+    bool any = !geo.order.empty();
+    for (int n = 1; n <= 4; ++n) any = any || !cmp[n].order.empty();
+    return any;
   }
 };
 
@@ -192,7 +212,7 @@ struct Shard {
   uint8_t *h_desc = nullptr;   // pinned staging: device-updated stream descriptors + walks travel back without blocking
   uint64_t cap_hdesc = 0;
   bool desc_pending = false;   // h_desc holds a copy-back that absorb_descs folds into streams / walks after the sync
-  std::vector<uint32_t> order_host;  // the order lists of the decode in flight (source of an asynchronous upload)
+  ShardPlan plan;              // of the decode in flight (its order array is the source of an asynchronous upload)
   uint32_t epoch = 0;          // tags the look-back words of par_post2_kernel (30 bits, never 0): no clearing between decodes
   bool uploaded = false, dirty = true, own_out = false;
   uint8_t *ext_out = nullptr, *ext_dbg = nullptr;
@@ -1050,7 +1070,6 @@ void plan_rans_groups(std::vector<Group *> &gs, uint32_t num_sms, uint32_t share
       want = std::max<uint32_t>(1u, (uint32_t)(my / lane_bytes));
     }
     g.pairs = 0;
-    g.ctas_per_sm = 0;
     // what the group's tables need of the two-region LUT's narrow region: it covers the slots from the first entry
     // narrower than 2^k on, for the k whose wide region still fits the LUT
     auto lutb_need = [&]() -> uint32_t {
@@ -1066,7 +1085,7 @@ void plan_rans_groups(std::vector<Group *> &gs, uint32_t num_sms, uint32_t share
       return need == 0xFFFFFFFFu ? need : std::max<uint32_t>(16u, (uint32_t)align_up(need, 16));
     };
     g.direct = 0;
-    const uint32_t ksym = g.kind == 1 ? 16u : 4u * (uint32_t)g.ncp;
+    const uint32_t ksym = g.tag ? 16u : 4u * (uint32_t)g.ncp;
     const uint64_t sm_cap = (uint64_t)sm_bytes + 1024 / share;
     auto pc_cta_bytes = [&](uint32_t pairs, uint32_t lanes, uint32_t lut, uint32_t lutb, uint32_t direct) -> uint64_t {
       RansLaunch L{};
@@ -1091,7 +1110,6 @@ void plan_rans_groups(std::vector<Group *> &gs, uint32_t num_sms, uint32_t share
         g.direct = 1;
         g.pairs = pairs;
         g.lanes = lanes;
-        g.ctas_per_sm = 1;
         g.lut_bytes = dlut;
         g.lutb_bytes = 0;
         continue;
@@ -1124,7 +1142,6 @@ void plan_rans_groups(std::vector<Group *> &gs, uint32_t num_sms, uint32_t share
           g.split = split ? 1u : 0u;
           g.pairs = pairs;
           g.lanes = lanes;
-          g.ctas_per_sm = 1;
           g.lutb_bytes = 0;
           continue;
         }
@@ -1133,8 +1150,7 @@ void plan_rans_groups(std::vector<Group *> &gs, uint32_t num_sms, uint32_t share
     if (!g.wide && env_flags().rans_pc && !g.force_single_warp) {
       // ---- chain / consumer warp pairs with the two-level tables (experiment: measured slower than one warp per
       // sub-partition when the SM is full of streams -- the two warps of a pair compete for the same issue port) ----
-      uint32_t target = std::max<uint32_t>(1u, 4u / share);
-      if (env_flags().pairs > 0) target = (uint32_t)env_flags().pairs;
+      const uint32_t target = std::max<uint32_t>(1u, 4u / share);
       const uint32_t lutb_min = g.compact ? 16u : 0u;
       uint32_t pairs = 1, lanes = 1, ctas = 1;
       if (env_flags().split && share == 1 && (want + 2) / 3 <= 32) {
@@ -1145,7 +1161,6 @@ void plan_rans_groups(std::vector<Group *> &gs, uint32_t num_sms, uint32_t share
           g.split = 1;
           g.lanes = l3;
           g.pairs = p3;
-          g.ctas_per_sm = 1;
           g.lutb_bytes = 0;
           if (g.compact) {
             const uint64_t base = pc_cta_bytes(p3, l3, g.lut_bytes, lutb_min0, 0);
@@ -1167,7 +1182,6 @@ void plan_rans_groups(std::vector<Group *> &gs, uint32_t num_sms, uint32_t share
       }
       g.lanes = lanes;
       g.pairs = pairs;
-      g.ctas_per_sm = ctas;
       g.lutb_bytes = 0;
       if (g.compact) {
         const uint64_t base = ctas * pc_cta_bytes(pairs, lanes, g.lut_bytes, lutb_min, 0);
@@ -1179,8 +1193,7 @@ void plan_rans_groups(std::vector<Group *> &gs, uint32_t num_sms, uint32_t share
       continue;
     }
     // ---- one warp per CTA (dcb_kernels.cu): spread the streams of an SM over its four sub-partitions ----
-    uint32_t ctas = std::max<uint32_t>((want + 31) / 32, std::min<uint32_t>(std::max<uint32_t>(1u, 4u / share), want));
-    if (env_flags().ctas_per_sm > 0) ctas = std::max<uint32_t>((want + 31) / 32, (uint32_t)env_flags().ctas_per_sm);  // experiments
+    const uint32_t ctas = std::max<uint32_t>((want + 31) / 32, std::min<uint32_t>(std::max<uint32_t>(1u, 4u / share), want));
     g.lanes = std::max<uint32_t>(1u, std::min<uint32_t>(32u, (want + ctas - 1) / ctas));
     // a CTA must fit an SM (with its alignment slack) and, for u16 tables, address its entries with 16 bits
     while (g.lanes > 1 && ((uint64_t)g.lanes * lane_bytes + g.lut_bytes + 256 > kSmemPerSM - kSmemPerCtaReserve ||
@@ -1263,7 +1276,7 @@ int issue_maps_copy(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index) {
   // piece into pinned staging (same layout as the device arena) while the DMA of the finished pieces is already running.
   constexpr uint64_t kMapsStageMin = 32ull << 20, kPiece = 8ull << 20;
   bool staged = false;
-  if (sh.maps_bytes >= kMapsStageMin && !env_flags().no_fanout) {
+  if (sh.maps_bytes >= kMapsStageMin) {
     if (!sh.h_maps && pinned_alloc(sh.pool, sh.maps_bytes, &sh.h_maps, &sh.cap_hmaps) != cudaSuccess) {
       cudaGetLastError();
       sh.h_maps = nullptr;
@@ -1650,22 +1663,8 @@ void absorb_descs(dcb_batch *b) {
   }
 }
 
-struct Timer {
-  cudaEvent_t a = nullptr, b = nullptr;
-};
-
-// Decode everything of one shard into (d_out, d_dbg).  Asynchronous on the shard's stream except
-// for the resolve round trips of Tagged streams.
-int decode_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index, uint8_t *d_out, uint8_t *d_dbg, uint32_t flags,
-                 bool timed) {
-  cudaStream_t st = ctx->streams[dev_index];
-  CUDA_TRY(cudaSetDevice(sh.device));
-  const uint32_t num_sms = (uint32_t)ctx->num_sms[dev_index];
-  // device 0 of the context writes the decode's statistics record; the other devices' decode threads count their
-  // launches and streams in records of their own, merged by finish_stats
-  dcb_launch_stats &stats = dev_index == 0 ? ctx->stats : ctx->dev_stats[dev_index];
-  if (sh.streams.empty()) return DCB_OK;
-  // fresh descriptors: the decode must not depend on what an earlier decode left behind
+// fresh descriptors: the decode must not depend on what an earlier decode left behind
+int reset_descriptors(Shard &sh, cudaStream_t st) {
   if (sh.dirty) {
     sh.streams = sh.streams0;
     sh.walks = sh.walks0;
@@ -1674,41 +1673,81 @@ int decode_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index, uint8_t *
     sh.dirty = false;
   }
   sh.tags_launched.assign(sh.streams.size(), 0);
-  // point order: the kernels write the entry-order staging, the point stage fills d_out from it
-  DevArenas A{sh.d_in, sh.pts ? sh.d_pts : d_out, d_dbg, sh.d_aux, sh.d_tab, sh.d_maps};
-  const uint32_t dump = flags & (DCB_DUMP_SYMBOLS | DCB_DUMP_QINTS);
-  const bool dbg_tl = timed && sh.device == ctx->devices[0] && env_flags().debug_timing;
-  auto tl_begin = [&](const char *name, cudaStream_t s) {
-    if (!dbg_tl) return;
-    cudaEvent_t a, b;
-    cudaEventCreate(&a);
-    cudaEventCreate(&b);
-    cudaEventRecord(a, s);
-    ctx->timeline.push_back({std::string(name) + " s" + std::to_string(dev_index), {a, b}});
-  };
-  auto tl_end = [&](cudaStream_t s) {
-    if (dbg_tl) cudaEventRecord(ctx->timeline.back().second.second, s);
-  };
-  // last writer of every attribute: behind the joins, on the main stream
-  auto point_stage = [&]() -> int {
-    if (!sh.pts) return DCB_OK;
-    int rc = issue_maps_copy(ctx, b, sh, dev_index);
-    if (rc) return rc;
-    DevArenas P = A;
-    P.out = d_out;
-    tl_begin("point stage", st);
-    CUDA_TRY(dcb_launch_point_stage(sh.pstage, sh.d_streams, P, num_sms, st));
-    tl_end(st);
-    stats.n_launches += 3;
-    return DCB_OK;
-  };
-  if (timed && dev_index == 0) CUDA_TRY(cudaEventRecord(ctx->ev[0], st));
+  return DCB_OK;
+}
 
-  // ---- Tagged streams: decode tags, resume the walks behind their bit areas ----
-  bool deferred_descs = false;
+// what the launches of one decode of a shard share
+struct ShardRun {
+  dcb_ctx *ctx;
+  dcb_batch *b;
+  Shard &sh;
+  int dev_index;
+  cudaStream_t st;  // the shard's stream
+  uint32_t num_sms;
+  dcb_launch_stats &stats;
+  DevArenas A;
+  uint32_t dump;
+  bool events;      // a timed decode on context device 0: records ctx->ev[] and the algorithm bytes
+  bool dbg_tl;      // DCB_DEBUG_TIMING spans of this decode
+  bool side_used[3] = {false, false, false};
+  // a DCB_DEBUG_TIMING span on stream s: begun with a name, ended without one
+  void tl(cudaStream_t s, const char *begin = nullptr) const {
+    if (dbg_tl) tl_mark(ctx, begin ? std::string(begin) + " s" + std::to_string(dev_index) : std::string(), s, begin != nullptr);
+  }
+};
+
+// DCB_DEBUG_PLAN: the planner's choices for one rANS group
+void print_plan(const Group &g) {
+  if (!env_flags().debug_plan) return;
+  fprintf(stderr, "[dcb plan] %s group ncp=%d wide=%d compact=%u prec=%u entries=%u mode=%u zig=%u: %u streams, %llu symbols, "
+                  "k=%u lut=%uB lutb=%uB ent=%uB lanes=%u pairs=%u split=%u direct=%u global=%d rec_ka=%u rec=%uB (need x8: %u %u %u %u, exc %u)\n",
+          g.tag ? "tag" : "raw", g.ncp, (int)g.wide, g.compact, g.prec_bits, g.entries, g.mode, g.zig, (uint32_t)g.order.size(),
+          (unsigned long long)g.total_symbols, g.lut_shift, g.lut_bytes, g.lutb_bytes, g.ent_bytes, g.lanes, g.pairs, g.split,
+          g.direct, (int)g.table_global, g.rec_ka, g.rec_bytes, g.rec_max[0], g.rec_max[1], g.rec_max[2], g.rec_max[3], g.exc_all);
+}
+
+// the launch of a planned group over n of its streams, listed at d_order
+RansLaunch rans_launch(const Group &g, StreamDesc *d_streams, const uint32_t *d_order, uint32_t n, uint32_t dump) {
+  return RansLaunch{d_streams, d_order, n, g.lanes, g.lut_bytes, g.lutb_bytes, g.ent_bytes, g.entries, g.rec_ka ? g.exc_all : g.exc,
+                    g.lut_shift, g.prec_bits, dump, g.compact, g.zig, g.mode, g.pairs, g.direct, g.rec_ka, g.rec_bytes, g.split};
+}
+
+// Walks blocked on their last stream, a Tagged one, finished on the host: their streams' kernels follow from header
+// fields the host already has.
+void finish_tagged_walks(Shard &sh, const std::vector<uint32_t> &blocked) {
+  for (uint32_t bi : blocked) {
+    BufWalk &w = sh.walks[bi];
+    for (int i = 0; i < w.stream_count; ++i) {
+      StreamDesc &s = sh.streams[w.stream_first + i];
+      if (s.state == ST_READY) continue;
+      if (s.state == ST_TAGS_PENDING) {
+        bool has_scheme, mesh_scheme;
+        int e;
+        walk_scheme_kind(w, s, has_scheme, mesh_scheme, e);
+        s.recon = !has_scheme ? (uint8_t)RECON_NONE
+                  : s.transform == XF_WRAP ? (uint8_t)(mesh_scheme ? RECON_PARA_WRAP : RECON_DELTA_WRAP)
+                  : s.transform == XF_OCT_CANON ? (uint8_t)(mesh_scheme ? RECON_GEO_OCT_CANON : RECON_DELTA_OCT_CANON)
+                                                : (uint8_t)(mesh_scheme ? RECON_GEO_OCT : RECON_DELTA_OCT);
+      }
+      if (s.seq_type == SEQ_QUANTIZATION) s.store = STORE_DEQUANT;
+      else if (s.seq_type == SEQ_NORMALS) s.store = STORE_OCT_UNIT;
+      else if (s.seq_type == SEQ_INTEGER) s.store = STORE_NARROW;
+      s.state = ST_READY;
+    }
+    w.blocked = -1;
+    w.phase = 2;
+  }
+}
+
+// Tagged streams: decode tags, resume the walks behind their bit areas, round by round.  `deferred`: the last round's
+// walks were finished on the host (finish_tagged_walks); the device descriptors hold what their resumed walks found.
+int run_tag_rounds(ShardRun &r, bool &deferred) {
+  dcb_ctx *ctx = r.ctx;
+  Shard &sh = r.sh;
+  const cudaStream_t st = r.st;
   for (;;) {
     Group g{};
-    g.kind = 1; g.ncp = 1; g.wide = false; g.compact = 1; g.prec_bits = 12; g.entries = 0; g.exc = 0; g.zig = 0; g.mode = 0;
+    g.tag = true; g.ncp = 1; g.compact = 1; g.prec_bits = 12;
     std::vector<uint32_t> blocked;
     for (size_t bi = 0; bi < sh.walks.size(); ++bi) {
       const BufWalk &w = sh.walks[bi];
@@ -1723,85 +1762,56 @@ int decode_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index, uint8_t *
       g.note_table(sh.streams[si]);
       blocked.push_back((uint32_t)bi);
     }
-    if (g.order.empty()) break;
+    if (g.order.empty()) return DCB_OK;
     sh.dirty = true;
     std::stable_sort(g.order.begin(), g.order.end(),
                      [&](uint32_t x, uint32_t y) { return sh.streams[x].n_entries > sh.streams[y].n_entries; });
     std::vector<Group *> gs{&g};
-    plan_rans_groups(gs, num_sms, (uint32_t)sh.share);
+    plan_rans_groups(gs, r.num_sms, (uint32_t)sh.share);
     if (g.table_global) return DCB_ERR_STATE;  // cannot happen: tag alphabets are tiny (<= 2^24 guarded by table size)
-    if (env_flags().debug_plan)
-      fprintf(stderr, "[dcb plan] tag group compact=%u prec=%u entries=%u: %u streams, %llu symbols, k=%u lut=%uB lutb=%uB ent=%uB "
-                      "lanes=%u pairs=%u split=%u direct=%u global=%d rec_ka=%u rec=%uB (need x8: %u %u %u %u, exc %u)\n",
-              g.compact, g.prec_bits, g.entries, (uint32_t)g.order.size(), (unsigned long long)g.total_symbols, g.lut_shift, g.lut_bytes,
-              g.lutb_bytes, g.ent_bytes, g.lanes, g.pairs, g.split, g.direct, (int)g.table_global, g.rec_ka, g.rec_bytes, g.rec_max[0],
-              g.rec_max[1], g.rec_max[2], g.rec_max[3], g.exc_all);
+    print_plan(g);
     int rc = ensure_order(sh, g.order.size() + blocked.size());
     if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(sh.d_order, g.order.data(), g.order.size() * 4, cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(sh.d_order + g.order.size(), blocked.data(), blocked.size() * 4, cudaMemcpyHostToDevice, st));
-    RansLaunch L{sh.d_streams, sh.d_order, (uint32_t)g.order.size(), g.lanes, g.lut_bytes, g.lutb_bytes, g.ent_bytes,
-                 g.entries, g.exc, g.lut_shift, g.prec_bits, dump, 1, 0, 0};
-    const bool time_tag = timed && dev_index == 0 && !ctx->ev_tag;
+    const RansLaunch L = rans_launch(g, sh.d_streams, sh.d_order, (uint32_t)g.order.size(), r.dump);
+    const bool time_tag = r.events && !ctx->ev_tag;
     if (time_tag) {
       CUDA_TRY(cudaEventRecord(ctx->ev[4], st));
       for (uint32_t si : g.order) ctx->algo_tag += sh.streams[si].payload_len + sh.streams[si].n_entries;
     }
-    L.pairs = g.pairs;
-    L.direct = g.direct;
-    L.rec_ka = g.rec_ka;
-    L.rec_bytes = g.rec_bytes;
-    L.split = g.split;
-    L.cap_exc = g.rec_ka ? g.exc_all : g.exc;
-    CUDA_TRY(g.rec_ka ? dcb_launch_rans_tag_rec(L, A, st) : g.pairs ? dcb_launch_rans_tag_pc(L, A, st) : dcb_launch_rans_tag(L, A, st));
+    CUDA_TRY(g.rec_ka ? dcb_launch_rans_tag_rec(L, r.A, st) : g.pairs ? dcb_launch_rans_tag_pc(L, r.A, st) : dcb_launch_rans_tag(L, r.A, st));
     if (time_tag) {
       CUDA_TRY(cudaEventRecord(ctx->ev[5], st));
       ctx->ev_tag = true;
     }
-    {  // the maps travel while the tag chains run
-      int rcm = issue_maps_copy(ctx, b, sh, dev_index);
-      if (rcm) return rcm;
-    }
-    CUDA_TRY(dcb_launch_resolve(A, sh.d_walks, sh.d_order + g.order.size(), (uint32_t)blocked.size(), sh.d_streams, st));
-    stats.n_launches += 2;
-    stats.n_streams += (int32_t)g.order.size();
+    rc = issue_maps_copy(ctx, r.b, sh, r.dev_index);  // the maps travel while the tag chains run
+    if (rc) return rc;
+    CUDA_TRY(dcb_launch_resolve(r.A, sh.d_walks, sh.d_order + g.order.size(), (uint32_t)blocked.size(), sh.d_streams, st));
+    r.stats.n_launches += 2;
+    r.stats.n_streams += (int32_t)g.order.size();
     // Nothing follows a Tagged attribute that closes its buffer, so the host does not need what the resumed walk finds
     // (wrap bounds, quantisation parameters: they stay in the device descriptors, where the kernels read them) -- only
     // WHICH kernels to launch, and that follows from the header fields it already has.  No round trip then.
     bool all_last = !env_flags().no_fast_tagged;
     for (uint32_t bi : blocked) all_last = all_last && sh.walks[bi].blocked == sh.walks[bi].stream_count - 1;
     if (all_last) {
-      for (uint32_t bi : blocked) {
-        BufWalk &w = sh.walks[bi];
-        for (int i = 0; i < w.stream_count; ++i) {
-          StreamDesc &s = sh.streams[w.stream_first + i];
-          if (s.state == ST_READY) continue;
-          if (s.state == ST_TAGS_PENDING) {
-            bool has_scheme, mesh_scheme;
-            int e;
-            walk_scheme_kind(w, s, has_scheme, mesh_scheme, e);
-            s.recon = !has_scheme ? (uint8_t)RECON_NONE
-                      : s.transform == XF_WRAP ? (uint8_t)(mesh_scheme ? RECON_PARA_WRAP : RECON_DELTA_WRAP)
-                      : s.transform == XF_OCT_CANON ? (uint8_t)(mesh_scheme ? RECON_GEO_OCT_CANON : RECON_DELTA_OCT_CANON)
-                                                    : (uint8_t)(mesh_scheme ? RECON_GEO_OCT : RECON_DELTA_OCT);
-          }
-          if (s.seq_type == SEQ_QUANTIZATION) s.store = STORE_DEQUANT;
-          else if (s.seq_type == SEQ_NORMALS) s.store = STORE_OCT_UNIT;
-          else if (s.seq_type == SEQ_INTEGER) s.store = STORE_NARROW;
-          s.state = ST_READY;
-        }
-        w.blocked = -1;
-        w.phase = 2;
-      }
-      deferred_descs = true;
-      break;
+      finish_tagged_walks(sh, blocked);
+      deferred = true;
+      return DCB_OK;
     }
     CUDA_TRY(cudaMemcpyAsync(sh.streams.data(), sh.d_streams, sh.streams.size() * sizeof(StreamDesc), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaMemcpyAsync(sh.walks.data(), sh.d_walks, sh.walks.size() * sizeof(BufWalk), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
   }
+}
 
-  // ---- classify ----
+constexpr int kWideAttrMode = 5;  // RawKey::mode of wide attributes: a group of their own, launched in mode 0
+
+// Sort the ready streams of a shard into its launches and plan them.  Host work only: it makes no CUDA call.  Wide
+// attributes it cannot decode get DCB_ERR_UNSUPPORTED in sh.streams.
+int plan_shard(const dcb_batch *b, Shard &sh, uint32_t num_sms, ShardPlan &p) {
+  p = ShardPlan{};
   // group key of a Raw stream; force_compact: -1 the natural table representation (compact when fewer than half of the
   // alphabet is in use), 0 / 1 dense / compact
   auto raw_key_of = [&](const StreamDesc &s, bool raw_normals, int force_compact) -> RawKey {
@@ -1835,19 +1845,23 @@ int decode_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index, uint8_t *
     }
   }
   std::map<RawKey, Group> raw;
-  Group post[5], para[5], cmp[5], par[5], copy{}, octs{}, octc{}, tex{}, geo{}, wide{};
-  wide.kind = 8;
-  octs.kind = 6;
-  octc.kind = 6;
-  tex.kind = 7;
-  bool par_delta[5] = {false, false, false, false, false};
-  for (int n = 1; n <= 4; ++n) {
-    post[n] = Group{}; post[n].kind = 2; post[n].ncp = n;
-    para[n] = Group{}; para[n].kind = 3; para[n].ncp = n;
-    par[n] = Group{}; par[n].kind = 5; par[n].ncp = n;
-  }
-  copy.kind = 4;
-  bool has_para = false;
+  // a Raw stream joins the group of its key; the symbols of a stream are n_entries * ncp one-component ones
+  auto add_raw = [&](const RawKey &key, uint32_t si) {
+    const StreamDesc &s = sh.streams[si];
+    Group &g = raw[key];
+    if (g.order.empty()) {
+      g.ncp = key.ncp; g.wide = key.wide != 0; g.compact = (uint32_t)key.compact; g.prec_bits = (uint32_t)key.prec;
+      g.zig = (uint32_t)key.zig;
+      g.force_single_warp = key.mode == kWideAttrMode;
+      g.mode = g.force_single_warp ? 0u : (uint32_t)key.mode;
+    }
+    g.entries = std::max(g.entries, key.compact ? s.n_active : s.num_symbols);
+    if (key.compact) g.exc = std::max(g.exc, s.n_active - std::min(s.n_active, s.dense_prefix));
+    g.total_symbols += (uint64_t)s.n_entries * s.ncp;
+    g.max_entries = std::max(g.max_entries, s.n_entries);
+    g.note_table(s);
+    g.order.push_back(si);
+  };
   for (size_t bi = 0; bi < sh.walks.size(); ++bi) {
     const BufWalk &w = sh.walks[bi];
     if (w.status != DCB_OK) continue;
@@ -1856,8 +1870,8 @@ int decode_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index, uint8_t *
       const StreamDesc &s = sh.streams[si];
       if (s.state != ST_READY) continue;
       if (s.scheme == SCHEME_GENERIC) {
-        copy.order.push_back(si);
-        copy.max_bytes = std::max(copy.max_bytes, s.out_bytes);
+        p.copy.order.push_back(si);
+        p.copy.max_bytes = std::max(p.copy.max_bytes, s.out_bytes);
         continue;
       }
       if (s.n_entries == 0) continue;
@@ -1872,34 +1886,22 @@ int decode_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index, uint8_t *
         if (s.scheme == SCHEME_RAW) {
           RawKey key = raw_key_of(s, false, -1);
           key.ncp = 1;
-          key.mode = 5;
-          const uint32_t entries = key.compact ? s.n_active : s.num_symbols;
-          Group &g = raw[key];
-          if (g.order.empty()) {
-            g.kind = 0; g.ncp = 1; g.wide = key.wide != 0; g.compact = (uint32_t)key.compact; g.prec_bits = (uint32_t)key.prec;
-            g.zig = (uint32_t)key.zig; g.mode = 0;
-          }
-          g.entries = std::max(g.entries, entries);
-          if (key.compact) g.exc = std::max(g.exc, s.n_active - std::min(s.n_active, s.dense_prefix));
-          g.total_symbols += (uint64_t)s.n_entries * s.ncp;
-          g.max_entries = std::max(g.max_entries, s.n_entries);
-          g.note_table(s);
-          g.order.push_back(si);
-          g.force_single_warp = true;
+          key.mode = kWideAttrMode;
+          add_raw(key, si);
         }
-        wide.order.push_back(si);
+        p.wide.order.push_back(si);
         continue;
       }
       // normals behind a Raw stream: the rANS kernel leaves corrections, oct_chain + oct_unit follow on its stream
       const bool raw_normals = is_raw_normals(s);
       const bool geo_normals = s.recon == RECON_GEO_OCT || s.recon == RECON_GEO_OCT_CANON;
       if (geo_normals) {  // geo_normal_kernel finishes the attribute behind the parallelogram kernels of its parent
-        geo.order.push_back(si);
-        geo.max_entries = std::max(geo.max_entries, s.n_entries);
-        has_para = true;
+        p.geo.order.push_back(si);
+        p.geo.max_entries = std::max(p.geo.max_entries, s.n_entries);
+        p.has_para = true;
       } else if (s.store == STORE_OCT_UNIT && !raw_normals) {
-        octs.order.push_back(si);
-        octs.max_entries = std::max(octs.max_entries, s.n_entries);
+        p.octs.order.push_back(si);
+        p.octs.max_entries = std::max(p.octs.max_entries, s.n_entries);
       }
       if (s.scheme == SCHEME_RAW) {
         RawKey key = raw_key_of(s, raw_normals, -1);
@@ -1911,42 +1913,30 @@ int decode_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index, uint8_t *
           const auto it_t = raw_count.find(twin), it_n = raw_count.find(key);
           if (it_t != raw_count.end() && it_t->second >= (size_t)num_sms * 8 && it_n->second < (size_t)num_sms) key = twin;
         }
-        const uint32_t entries = key.compact ? s.n_active : s.num_symbols;
-        Group &g = raw[key];
-        if (g.order.empty()) {
-          g.kind = 0; g.ncp = key.ncp; g.wide = key.wide != 0; g.compact = (uint32_t)key.compact; g.prec_bits = (uint32_t)key.prec;
-          g.zig = (uint32_t)key.zig; g.mode = (uint32_t)key.mode;
-        }
-        g.entries = std::max(g.entries, entries);
-        if (key.compact) g.exc = std::max(g.exc, s.n_active - std::min(s.n_active, s.dense_prefix));
-        g.total_symbols += (uint64_t)s.n_entries * s.ncp;
-        g.max_entries = std::max(g.max_entries, s.n_entries);
-        g.note_table(s);
-        g.order.push_back(si);
-      } else if ((s.recon == RECON_NONE || s.recon == RECON_DELTA_WRAP || s.recon == RECON_PARA_WRAP || (geo_normals && s.ncp == 2) ||
-                  ((s.recon == RECON_DELTA_OCT || s.recon == RECON_DELTA_OCT_CANON) && s.ncp == 2 && s.store == STORE_OCT_UNIT)) &&
-                 !env_flags().no_par_post) {
+        add_raw(key, si);
+      } else if (s.recon == RECON_NONE || s.recon == RECON_DELTA_WRAP || s.recon == RECON_PARA_WRAP || (geo_normals && s.ncp == 2) ||
+                 ((s.recon == RECON_DELTA_OCT || s.recon == RECON_DELTA_OCT_CANON) && s.ncp == 2 && s.store == STORE_OCT_UNIT)) {
         // Tagged / uncompressed source: point-parallel extraction; scan-able reconstructions finish there, octahedral
         // corrections go to the scratch and oct_chain_kernel runs the recurrence (as behind a Raw source)
-        par[s.ncp].max_entries = std::max(par[s.ncp].max_entries, s.n_entries);
-        par[s.ncp].order.push_back(si);
-        if (s.recon == RECON_DELTA_WRAP) par_delta[s.ncp] = true;
-        if (s.recon == RECON_DELTA_OCT || s.recon == RECON_DELTA_OCT_CANON) octc.order.push_back(si);
+        p.par[s.ncp].max_entries = std::max(p.par[s.ncp].max_entries, s.n_entries);
+        p.par[s.ncp].order.push_back(si);
+        if (s.recon == RECON_DELTA_WRAP) p.pp[s.ncp].delta = true;
+        if (s.recon == RECON_DELTA_OCT || s.recon == RECON_DELTA_OCT_CANON) p.octc.order.push_back(si);
       } else {
-        post[s.ncp].order.push_back(si);
+        p.post[s.ncp].order.push_back(si);
       }
       if (s.recon == RECON_PARA_WRAP && s.pred_method == PRED_TEX_COORDS_PORTABLE) {
-        tex.order.push_back(si);
-        tex.max_entries = std::max(tex.max_entries, s.n_entries);
-        has_para = true;
+        p.tex.order.push_back(si);
+        p.tex.max_entries = std::max(p.tex.max_entries, s.n_entries);
+        p.has_para = true;
       } else if (s.recon == RECON_PARA_WRAP && s.pred_method == PRED_CONSTRAINED_MULTI) {
-        cmp[s.ncp].order.push_back(si);
-        cmp[s.ncp].max_entries = std::max(cmp[s.ncp].max_entries, s.n_entries);
-        has_para = true;
+        p.cmp[s.ncp].order.push_back(si);
+        p.cmp[s.ncp].max_entries = std::max(p.cmp[s.ncp].max_entries, s.n_entries);
+        p.has_para = true;
       } else if (s.recon == RECON_PARA_WRAP) {
-        para[s.ncp].order.push_back(si);
-        para[s.ncp].max_entries = std::max(para[s.ncp].max_entries, s.n_entries);
-        has_para = true;
+        p.para[s.ncp].order.push_back(si);
+        p.para[s.ncp].max_entries = std::max(p.para[s.ncp].max_entries, s.n_entries);
+        p.has_para = true;
       }
     }
   }
@@ -1955,181 +1945,147 @@ int decode_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index, uint8_t *
   for (uint32_t si = sh.idx_first; si < sh.streams.size(); ++si) {
     const StreamDesc &s = sh.streams[si];
     if (s.status || sh.walks[b->bufs[s.buf_index].local].status != DCB_OK) continue;
-    const RawKey key = raw_key_of(s, false, -1);
-    const uint32_t entries = key.compact ? s.n_active : s.num_symbols;
-    Group &g = raw[key];
-    if (g.order.empty()) {
-      g.kind = 0; g.ncp = 1; g.wide = key.wide != 0; g.compact = (uint32_t)key.compact; g.prec_bits = (uint32_t)key.prec;
-      g.zig = 0; g.mode = (uint32_t)key.mode;
-    }
-    g.entries = std::max(g.entries, entries);
-    if (key.compact) g.exc = std::max(g.exc, s.n_active - std::min(s.n_active, s.dense_prefix));
-    g.total_symbols += s.n_entries;
-    g.max_entries = std::max(g.max_entries, s.n_entries);
-    g.note_table(s);
-    g.order.push_back(si);
+    add_raw(raw_key_of(s, false, -1), si);
   }
-  std::vector<Group *> rgs;
-  for (auto &kv : raw) rgs.push_back(&kv.second);
+  for (auto &kv : raw) p.raw.push_back(std::move(kv.second));
   // the groups run one after another on the shard's stream: each one may use the whole SM
-  bool side_followers = false;
-  for (Group *g : rgs) side_followers = side_followers || (g->mode == 3 && rgs.size() > 1);
-  for (Group *g : rgs) {
+  for (const Group &g : p.raw) p.side_followers = p.side_followers || (g.mode == 3 && p.raw.size() > 1);
+  for (Group &g : p.raw) {
     // A handful of outlier streams next to a machine-filling group (one cloud of a batch whose table came out dense)
     // must stay small: the direct slot LUT wants ~50 KB per stream, finds no room beside the big group's CTAs and would
     // run BEHIND it (measured: +17 ms on a 27 ms step); with the two-level tables it runs beside it, on a side stream.
-    g->no_direct = g->force_single_warp;
-    for (Group *o : rgs)
-      if (o != g && o->order.size() >= (size_t)num_sms * 8) g->no_direct = true;
-    std::vector<Group *> one{g};
-    plan_rans_groups(one, num_sms, (uint32_t)sh.share, side_followers ? 6u * 1024u : 0u);
+    g.no_direct = g.force_single_warp;
+    for (const Group &o : p.raw)
+      if (&o != &g && o.order.size() >= (size_t)num_sms * 8) g.no_direct = true;
+    std::vector<Group *> one{&g};
+    plan_rans_groups(one, num_sms, (uint32_t)sh.share, p.side_followers ? 6u * 1024u : 0u);
   }
-  // device order lists
-  uint64_t n_order = 0;
-  auto add = [&](Group &g) {
-    g.order_off = n_order;
-    n_order += g.order.size();
+  auto longest_first = [&](std::vector<uint32_t> &order) {
+    std::stable_sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) { return sh.streams[x].n_entries > sh.streams[y].n_entries; });
   };
-  for (Group *g : rgs) {
-    std::stable_sort(g->order.begin(), g->order.end(),
-                     [&](uint32_t x, uint32_t y) { return sh.streams[x].n_entries > sh.streams[y].n_entries; });
-    add(*g);
+  for (size_t i = 0; i < p.raw.size(); ++i) {
+    longest_first(p.raw[i].order);
+    if (p.dom < 0 || p.raw[i].total_symbols > p.raw[p.dom].total_symbols) p.dom = (int)i;
   }
-  for (int n = 1; n <= 4; ++n) { add(post[n]); add(para[n]); add(cmp[n]); add(par[n]); }
-  add(copy);
-  add(octs);
-  add(octc);
-  add(tex);
-  add(geo);
-  add(wide);
-  // par_post2_kernel: per group the run prefix of its streams (runs of par_run_len chunks) and one ticket word
-  std::vector<uint32_t> par_runs[5];
-  uint64_t par_aux_off[5] = {0, 0, 0, 0, 0};
-  uint32_t par_run_len[5] = {1, 1, 1, 1, 1}, par_claim[5] = {1, 1, 1, 1, 1}, par_rounds[5] = {0, 0, 0, 0, 0};
+  // par_post2_kernel: per group the run prefix of its streams (runs of run_len chunks) and one ticket word
   for (int n = 1; n <= 4; ++n) {
-    if (par[n].order.empty()) continue;
+    Stage &par = p.par[n];
+    ShardPlan::ParPost &pp = p.pp[n];
+    if (par.order.empty()) continue;
     // longest streams first: whole-stream runs are handed out by ticket, longest-processing-time first
-    std::stable_sort(par[n].order.begin(), par[n].order.end(),
-                     [&](uint32_t x, uint32_t y) { return sh.streams[x].n_entries > sh.streams[y].n_entries; });
+    longest_first(par.order);
     uint64_t total_chunks = 0, max_chunks = 0;
-    for (uint32_t si : par[n].order) {
+    for (uint32_t si : par.order) {
       const uint64_t nch = ((uint64_t)sh.streams[si].n_entries + DCB_TAG_CHUNK - 1) / DCB_TAG_CHUNK;
       total_chunks += nch;
       max_chunks = std::max(max_chunks, nch);
     }
-    dcb_par_post_plan((uint32_t)par[n].order.size(), total_chunks, (uint32_t)std::min<uint64_t>(max_chunks, 0xFFFFFFFFull),
-                      par_delta[n], num_sms, n, (uint32_t)sh.share, &par_run_len[n], &par_claim[n]);
-    if (env_flags().par_run > 0) {  // experiments
-      par_run_len[n] = (uint32_t)env_flags().par_run;
-      par_claim[n] = 1;
-    }
+    dcb_par_post_plan((uint32_t)par.order.size(), total_chunks, (uint32_t)std::min<uint64_t>(max_chunks, 0xFFFFFFFFull),
+                      pp.delta, num_sms, n, (uint32_t)sh.share, &pp.run_len, &pp.claim);
     // Chunk-sized runs that look back (delta streams) are ticketed ROUND by round -- chunk r of every stream that has
     // one, then chunk r + 1 -- so that the chunks a warp claims together, and the chunks of neighbouring claims, belong
     // to different streams: in stream-major order a claim's look-back waits for the previous claim's LAST chunk, which
     // waits for that claim's first look-back, and a stream decodes chunk after chunk (measured: 195 ms instead of ~8
     // for 2,000 streams of 100,000 points).  The prefix then runs over rounds: the streams are sorted by length, so
     // round r holds the first count(r) of them.
-    par_rounds[n] = 0;
-    if (par_run_len[n] == 1 && par_delta[n] && !getenv("DCB_PAR_STREAM_MAJOR") && max_chunks <= (1ull << 24)) {
-      par_rounds[n] = (uint32_t)max_chunks;
-      par_runs[n].assign((size_t)max_chunks + 2, 0u);
-      // count(r) = streams with more than r chunks; par_runs[r + 1] - par_runs[r] = count(r)
-      for (uint32_t si : par[n].order) {
+    if (pp.run_len == 1 && pp.delta && max_chunks <= (1ull << 24)) {
+      pp.rounds = (uint32_t)max_chunks;
+      pp.runs.assign((size_t)max_chunks + 2, 0u);
+      // count(r) = streams with more than r chunks; runs[r + 1] - runs[r] = count(r)
+      for (uint32_t si : par.order) {
         const uint64_t nch = ((uint64_t)sh.streams[si].n_entries + DCB_TAG_CHUNK - 1) / DCB_TAG_CHUNK;
-        if (nch > 0) par_runs[n][(size_t)nch] += 1;  // streams that END after round nch - 1
+        if (nch > 0) pp.runs[(size_t)nch] += 1;  // streams that END after round nch - 1
       }
       if (total_chunks > 0xFFFFFFF0ull) return DCB_ERR_UNSUPPORTED;
-      uint64_t alive = par[n].order.size(), acc = 0;
+      uint64_t alive = par.order.size(), acc = 0;
       for (uint64_t r = 0; r <= max_chunks; ++r) {
-        const uint32_t ending = par_runs[n][(size_t)r];  // streams with exactly r chunks: gone from round r on
+        const uint32_t ending = pp.runs[(size_t)r];  // streams with exactly r chunks: gone from round r on
         alive -= ending;
-        par_runs[n][(size_t)r] = (uint32_t)acc;
+        pp.runs[(size_t)r] = (uint32_t)acc;
         acc += alive;
       }
-      par_runs[n][(size_t)max_chunks + 1] = 0u;  // the ticket
+      pp.runs[(size_t)max_chunks + 1] = 0u;  // the ticket
     } else {
-      par_runs[n].reserve(par[n].order.size() + 2);
+      pp.runs.reserve(par.order.size() + 2);
       uint64_t acc = 0;
-      for (uint32_t si : par[n].order) {
-        par_runs[n].push_back((uint32_t)acc);
+      for (uint32_t si : par.order) {
+        pp.runs.push_back((uint32_t)acc);
         const uint64_t nch = ((uint64_t)sh.streams[si].n_entries + DCB_TAG_CHUNK - 1) / DCB_TAG_CHUNK;
-        acc += (nch + par_run_len[n] - 1) / par_run_len[n];
+        acc += (nch + pp.run_len - 1) / pp.run_len;
       }
       if (acc > 0xFFFFFFF0ull) return DCB_ERR_UNSUPPORTED;
-      par_runs[n].push_back((uint32_t)acc);
-      par_runs[n].push_back(0u);  // the ticket
+      pp.runs.push_back((uint32_t)acc);
+      pp.runs.push_back(0u);  // the ticket
     }
-    par_aux_off[n] = n_order;
-    n_order += par_runs[n].size();
   }
+  // the device order array: each list's offset is where it lands
+  auto append = [&](const std::vector<uint32_t> &v, uint64_t &off) {
+    off = p.order.size();
+    p.order.insert(p.order.end(), v.begin(), v.end());
+  };
+  for (Group &g : p.raw) append(g.order, g.order_off);
+  for (int n = 1; n <= 4; ++n)
+    for (Stage *l : {&p.post[n], &p.para[n], &p.cmp[n], &p.par[n]}) append(l->order, l->order_off);
+  for (Stage *l : {&p.copy, &p.octs, &p.octc, &p.tex, &p.geo, &p.wide}) append(l->order, l->order_off);
+  for (int n = 1; n <= 4; ++n) append(p.pp[n].runs, p.pp[n].runs_off);
+  return DCB_OK;
+}
 
-  if (n_order == 0) {
-    int rc = point_stage();
-    if (rc) return rc;
-    if (timed && dev_index == 0) CUDA_TRY(cudaEventRecord(ctx->ev[1], st));
-    if (deferred_descs || sh.pts) return queue_desc_copyback(ctx, sh, st);
-    return DCB_OK;
+// statistics and kernel name of the decode: those of its dominant Raw group
+void note_dominant(ShardRun &r, const Group &g) {
+  dcb_ctx *ctx = r.ctx;
+  dcb_launch_stats &stats = r.stats;
+  const uint32_t n = (uint32_t)g.order.size();
+  for (uint32_t si : g.order) {
+    const StreamDesc &sd = r.sh.streams[si];
+    ctx->algo_raw += (sd.payload_off + sd.payload_len - sd.table_off) + sd.out_bytes;
   }
-  {
-    int rc = ensure_order(sh, n_order);
-    if (rc) return rc;
-    std::vector<uint32_t> &all = sh.order_host;  // outlives the asynchronous upload
-    all.clear();
-    all.reserve(n_order);
-    for (Group *g : rgs) all.insert(all.end(), g->order.begin(), g->order.end());
-    for (int n = 1; n <= 4; ++n) {
-      all.insert(all.end(), post[n].order.begin(), post[n].order.end());
-      all.insert(all.end(), para[n].order.begin(), para[n].order.end());
-      all.insert(all.end(), cmp[n].order.begin(), cmp[n].order.end());
-      all.insert(all.end(), par[n].order.begin(), par[n].order.end());
-    }
-    all.insert(all.end(), copy.order.begin(), copy.order.end());
-    all.insert(all.end(), octs.order.begin(), octs.order.end());
-    all.insert(all.end(), octc.order.begin(), octc.order.end());
-    all.insert(all.end(), tex.order.begin(), tex.order.end());
-    all.insert(all.end(), geo.order.begin(), geo.order.end());
-    all.insert(all.end(), wide.order.begin(), wide.order.end());
-    for (int n = 1; n <= 4; ++n) all.insert(all.end(), par_runs[n].begin(), par_runs[n].end());
+  stats.lanes_per_warp = (int32_t)g.lanes;
+  stats.smem_per_stream = (uint64_t)g.lut_bytes + g.lutb_bytes + g.ent_bytes + DCB_RING_BYTES;
+  const RansLaunch Ls = rans_launch(g, nullptr, nullptr, n, 0);
+  const uint32_t cta_smem = (g.rec_ka ? dcb_rans_rec_smem_bytes(Ls, 4u * (uint32_t)g.ncp)
+                             : g.pairs ? dcb_rans_pc_smem_bytes(Ls, 4u * (uint32_t)g.ncp) : dcb_rans_smem_bytes(Ls, g.table_global)) + kSmemPerCtaReserve;
+  const uint64_t per_wave = (uint64_t)r.num_sms * std::max<uint32_t>(1u, std::min<uint32_t>(32u, (kSmemPerSM + 1024u) / cta_smem)) * g.lanes * std::max(1u, g.pairs);
+  stats.n_waves = g.table_global ? 1 : (int32_t)((n + per_wave - 1) / per_wave);
+  if (g.rec_ka)
+    snprintf(ctx->raw_name, sizeof ctx->raw_name, "rans_raw_rec<ncp=%d,u16,smem,mode=%u,bucket records 2^%u|16|1,%ux%u lanes,%uB>", g.ncp,
+             g.mode, g.rec_ka, g.pairs, g.lanes, g.rec_bytes);
+  else if (g.pairs)
+    snprintf(ctx->raw_name, sizeof ctx->raw_name, "rans_raw_pc<ncp=%d,u16,smem,mode=%u,%s,%s,%ux%u lanes>", g.ncp, g.mode,
+             g.direct ? "direct slot LUT" : "two-level LUT", g.compact ? "compact" : "dense", g.pairs, g.lanes);
+  else
+    snprintf(ctx->raw_name, sizeof ctx->raw_name, "rans_raw_fused<ncp=%d,%s,%s,mode=%u,k=%u,%s>", g.ncp,
+             g.wide ? "u32" : "u16", g.table_global ? "global" : "smem", g.mode, g.lut_shift,
+             g.compact ? "compact" : "dense");
+}
 
-    CUDA_TRY(cudaMemcpyAsync(sh.d_order, all.data(), all.size() * 4, cudaMemcpyHostToDevice, st));
-  }
-  // dominant group: most symbols
-  Group *dom = nullptr;
-  for (Group *g : rgs)
-    if (!dom || g->total_symbols > dom->total_symbols) dom = g;
-  // ---- launches ----
+// The Raw rANS groups.  `flags_early`: the flag kernels follow on side streams, so those fork too.
+int launch_rans_groups(ShardRun &r, const ShardPlan &p, bool flags_early) {
+  dcb_ctx *ctx = r.ctx;
+  Shard &sh = r.sh;
+  const int d = r.dev_index;
   // independent smem-table groups go to side streams so that their chains overlap (c3: positions, normals, colours)
-  const bool fan_out = rgs.size() > 1 && !env_flags().no_fanout;
-  // crease flags / flip bits of the 8f-3 predictors depend on the bitstream only: their (serial, small) rABS kernels run on
-  // a side stream next to the rANS kernels -- unless descriptors are still being resolved on the device behind Tagged bit areas
-  bool flag_kernels = !geo.order.empty();
-  for (int n = 1; n <= 4; ++n) flag_kernels = flag_kernels || !cmp[n].order.empty();
-  const bool flags_early = flag_kernels && !deferred_descs && !env_flags().no_fanout;
+  const bool fan_out = p.raw.size() > 1;
   if (fan_out || flags_early) {
-    CUDA_TRY(cudaEventRecord(ctx->fork_ev[dev_index], st));
-    for (cudaStream_t ss : ctx->side[dev_index]) CUDA_TRY(cudaStreamWaitEvent(ss, ctx->fork_ev[dev_index], 0));
+    CUDA_TRY(cudaEventRecord(ctx->fork_ev[d], r.st));
+    for (cudaStream_t ss : ctx->side[d]) CUDA_TRY(cudaStreamWaitEvent(ss, ctx->fork_ev[d], 0));
   }
-  bool side_used[3] = {false, false, false};
   size_t gi = 0;
-  const cudaStream_t st_main = st;
-  for (Group *g : rgs) {
-    const uint32_t n = (uint32_t)g->order.size();
-    const bool is_dom = timed && dev_index == 0 && g == dom;
-    cudaStream_t st = st_main;
-    if (fan_out && !g->table_global && (g != dom || g->mode == 3)) {
-      const size_t k = g->mode == 3 ? 0 : 1 + gi++ % 2;
-      st = ctx->side[dev_index][k];
-      side_used[k] = true;
+  for (size_t i = 0; i < p.raw.size(); ++i) {
+    const Group &g = p.raw[i];
+    const uint32_t n = (uint32_t)g.order.size();
+    const uint32_t *d_order = sh.d_order + g.order_off;
+    const bool is_dom = r.events && (int)i == p.dom;
+    cudaStream_t st = r.st;
+    if (fan_out && !g.table_global && ((int)i != p.dom || g.mode == 3)) {
+      const size_t k = g.mode == 3 ? 0 : 1 + gi++ % 2;
+      st = ctx->side[d][k];
+      r.side_used[k] = true;
     }
-    if (env_flags().debug_plan)
-      fprintf(stderr, "[dcb plan] raw group ncp=%d wide=%d compact=%u prec=%u entries=%u mode=%u zig=%u: %u streams, %llu symbols, "
-                      "k=%u lut=%uB lutb=%uB ent=%uB lanes=%u pairs=%u split=%u direct=%u global=%d rec_ka=%u rec=%uB (need x8: %u %u %u %u, exc %u)\n",
-              g->ncp, (int)g->wide, g->compact, g->prec_bits, g->entries, g->mode, g->zig, n,
-              (unsigned long long)g->total_symbols, g->lut_shift, g->lut_bytes, g->lutb_bytes, g->ent_bytes, g->lanes, g->pairs, g->split,
-              g->direct, (int)g->table_global, g->rec_ka, g->rec_bytes, g->rec_max[0], g->rec_max[1], g->rec_max[2], g->rec_max[3], g->exc_all);
+    print_plan(g);
     if (is_dom) CUDA_TRY(cudaEventRecord(ctx->ev[2], st));
-    if (g->table_global) {
-      const uint64_t slot_bytes = (uint64_t)g->lut_bytes + g->ent_bytes;
+    if (g.table_global) {
+      const uint64_t slot_bytes = (uint64_t)g.lut_bytes + g.ent_bytes;
       // chunk: a multiple of 32 slots whose tables fit the scratch budget and 32-bit entry offsets
       uint64_t per = std::max<uint64_t>(32, std::min<uint64_t>(kTabArenaBudget / slot_bytes, 0xF0000000ull / slot_bytes) / 32 * 32);
       const uint64_t chunk = std::min<uint64_t>(per, align_up(n, 32));
@@ -2140,135 +2096,123 @@ int decode_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index, uint8_t *
         CUDA_TRY(cudaMalloc(&sh.d_tab, chunk * slot_bytes));
         sh.tab_cap = chunk * slot_bytes;
       }
-      A.tab = sh.d_tab;
+      r.A.tab = sh.d_tab;
       for (uint64_t o = 0; o < n; o += chunk) {
-        RansLaunch L{sh.d_streams, sh.d_order + g->order_off + o, (uint32_t)std::min<uint64_t>(chunk, n - o), 32,
-                     g->lut_bytes, 0, g->ent_bytes, g->entries, g->exc, g->lut_shift, g->prec_bits, dump, g->compact, g->zig, 0};
-        CUDA_TRY(dcb_launch_rans_raw(L, g->ncp, g->wide, true, A, st));
-        stats.n_launches++;
+        // tables in global memory: 32 lanes, the uniform LUT, the generic post-processing
+        RansLaunch L = rans_launch(g, sh.d_streams, d_order + o, (uint32_t)std::min<uint64_t>(chunk, n - o), r.dump);
+        L.lanes_per_warp = 32;
+        L.lutb_bytes = 0;
+        L.mode = 0;
+        CUDA_TRY(dcb_launch_rans_raw(L, g.ncp, g.wide, true, r.A, st));
+        r.stats.n_launches++;
       }
     } else {
-      RansLaunch L{sh.d_streams, sh.d_order + g->order_off, n, g->lanes, g->lut_bytes, g->lutb_bytes, g->ent_bytes,
-                   g->entries, g->exc, g->lut_shift, g->prec_bits, dump, g->compact, g->zig, g->mode};
-      tl_begin(g->mode == 1 ? "rans mode1" : g->mode == 2 ? "rans mode2" : g->mode == 3 ? "rans mode3" : g->mode == 4 ? "rans mode4" : "rans mode0", st);
-      L.pairs = g->pairs;
-      L.direct = g->direct;
-      L.rec_ka = g->rec_ka;
-      L.rec_bytes = g->rec_bytes;
-      L.split = g->split;
-      if (g->rec_ka) L.cap_exc = g->exc_all;
-      CUDA_TRY(g->rec_ka ? dcb_launch_rans_raw_rec(L, g->ncp, A, st)
-               : g->pairs ? dcb_launch_rans_raw_pc(L, g->ncp, A, st) : dcb_launch_rans_raw(L, g->ncp, g->wide, false, A, st));
-      tl_end(st);
-      stats.n_launches++;
+      const RansLaunch L = rans_launch(g, sh.d_streams, d_order, n, r.dump);
+      r.tl(st, g.mode == 1 ? "rans mode1" : g.mode == 2 ? "rans mode2" : g.mode == 3 ? "rans mode3" : g.mode == 4 ? "rans mode4" : "rans mode0");
+      CUDA_TRY(g.rec_ka ? dcb_launch_rans_raw_rec(L, g.ncp, r.A, st)
+               : g.pairs ? dcb_launch_rans_raw_pc(L, g.ncp, r.A, st) : dcb_launch_rans_raw(L, g.ncp, g.wide, false, r.A, st));
+      r.tl(st);
+      r.stats.n_launches++;
     }
-    if (g->mode == 3) {
+    if (g.mode == 3) {
       // same stream, right behind the corrections; no shared memory, so they run next to the other groups' rANS kernels
-      tl_begin("oct_chain", st);
-      CUDA_TRY(dcb_launch_oct_chain(sh.d_streams, sh.d_order + g->order_off, n, dump, A, st));
-      tl_end(st);
-      tl_begin("oct_unit", st);
-      CUDA_TRY(dcb_launch_oct_unit(sh.d_streams, sh.d_order + g->order_off, n, g->max_entries, A, st));
-      tl_end(st);
-      stats.n_launches += 2;
+      r.tl(st, "oct_chain");
+      CUDA_TRY(dcb_launch_oct_chain(sh.d_streams, d_order, n, r.dump, r.A, st));
+      r.tl(st);
+      r.tl(st, "oct_unit");
+      CUDA_TRY(dcb_launch_oct_unit(sh.d_streams, d_order, n, g.max_entries, r.A, st));
+      r.tl(st);
+      r.stats.n_launches += 2;
     }
     if (is_dom) {
       CUDA_TRY(cudaEventRecord(ctx->ev[3], st));
       ctx->ev_raw = true;
-      for (uint32_t si : g->order) {
-        const StreamDesc &sd = sh.streams[si];
-        ctx->algo_raw += (sd.payload_off + sd.payload_len - sd.table_off) + sd.out_bytes;
-      }
-      stats.lanes_per_warp = (int32_t)g->lanes;
-      stats.smem_per_stream = (uint64_t)g->lut_bytes + g->lutb_bytes + g->ent_bytes + DCB_RING_BYTES;
-      RansLaunch Ls{nullptr, nullptr, n, g->lanes, g->lut_bytes, g->lutb_bytes, g->ent_bytes, g->entries, g->exc, g->lut_shift, g->prec_bits, 0, g->compact, g->zig, g->mode, g->pairs, g->direct};
-      Ls.rec_ka = g->rec_ka;
-      Ls.rec_bytes = g->rec_bytes;
-      const uint32_t cta_smem = (g->rec_ka ? dcb_rans_rec_smem_bytes(Ls, 4u * (uint32_t)g->ncp)
-                                 : g->pairs ? dcb_rans_pc_smem_bytes(Ls, 4u * (uint32_t)g->ncp) : dcb_rans_smem_bytes(Ls, g->table_global)) + kSmemPerCtaReserve;
-      const uint64_t per_wave = (uint64_t)num_sms * std::max<uint32_t>(1u, std::min<uint32_t>(32u, (kSmemPerSM + 1024u) / cta_smem)) * g->lanes * std::max(1u, g->pairs);
-      stats.n_waves = g->table_global ? 1 : (int32_t)((n + per_wave - 1) / per_wave);
-      if (g->rec_ka)
-        snprintf(ctx->raw_name, sizeof ctx->raw_name, "rans_raw_rec<ncp=%d,u16,smem,mode=%u,bucket records 2^%u|16|1,%ux%u lanes,%uB>", g->ncp,
-                 g->mode, g->rec_ka, g->pairs, g->lanes, g->rec_bytes);
-      else if (g->pairs)
-        snprintf(ctx->raw_name, sizeof ctx->raw_name, "rans_raw_pc<ncp=%d,u16,smem,mode=%u,%s,%s,%ux%u lanes>", g->ncp, g->mode,
-                 g->direct ? "direct slot LUT" : "two-level LUT", g->compact ? "compact" : "dense", g->pairs, g->lanes);
-      else
-        snprintf(ctx->raw_name, sizeof ctx->raw_name, "rans_raw_fused<ncp=%d,%s,%s,mode=%u,k=%u,%s>", g->ncp,
-                 g->wide ? "u32" : "u16", g->table_global ? "global" : "smem", g->mode, g->lut_shift,
-                 g->compact ? "compact" : "dense");
+      note_dominant(r, g);
     }
-    stats.n_streams += (int32_t)n;
+    r.stats.n_streams += (int32_t)n;
   }
+  return DCB_OK;
+}
+
+// Everything behind the rANS kernels: the flag kernels, the joins of the side streams, the post-processing, point-
+// parallel and mesh prediction kernels, on the shard's stream.
+int launch_after_rans(ShardRun &r, const ShardPlan &p, bool flags_early) {
+  dcb_ctx *ctx = r.ctx;
+  Shard &sh = r.sh;
+  const int d = r.dev_index;
+  const cudaStream_t st = r.st;
+  const uint32_t dump = r.dump;
+  DevArenas &A = r.A;
+  dcb_launch_stats &stats = r.stats;
   auto launch_flag_kernels = [&](cudaStream_t fs, cudaStream_t gs) -> int {
     for (int n = 1; n <= 4; ++n)
-      if (!cmp[n].order.empty()) {
-        CUDA_TRY(dcb_launch_cmp_flags(sh.d_streams, sh.d_order + cmp[n].order_off, (uint32_t)cmp[n].order.size(), A, fs));
+      if (!p.cmp[n].order.empty()) {
+        CUDA_TRY(dcb_launch_cmp_flags(sh.d_streams, sh.d_order + p.cmp[n].order_off, (uint32_t)p.cmp[n].order.size(), A, fs));
         stats.n_launches++;
       }
-    if (!geo.order.empty()) {
-      CUDA_TRY(dcb_launch_geo_flips(sh.d_streams, sh.d_order + geo.order_off, (uint32_t)geo.order.size(), A, gs));
+    if (!p.geo.order.empty()) {
+      CUDA_TRY(dcb_launch_geo_flips(sh.d_streams, sh.d_order + p.geo.order_off, (uint32_t)p.geo.order.size(), A, gs));
       stats.n_launches++;
     }
     return DCB_OK;
   };
   if (flags_early) {  // issued behind the rANS launches so that those get their SMs first; crease flags and flip bits on a
-    int rcf = launch_flag_kernels(ctx->side[dev_index][2], ctx->side[dev_index][1]);  // stream each (serial chains both)
+    int rcf = launch_flag_kernels(ctx->side[d][2], ctx->side[d][1]);  // stream each (serial chains both)
     if (rcf) return rcf;
-    side_used[2] = side_used[1] = true;
+    r.side_used[2] = r.side_used[1] = true;
   }
   {  // mesh maps: behind the rANS launches (their chains hide the copy), in front of the parallelogram kernels
-    int rcm = issue_maps_copy(ctx, b, sh, dev_index);
+    int rcm = issue_maps_copy(ctx, r.b, sh, d);
     if (rcm) return rcm;
   }
   auto launch_cmp_deps = [&](cudaStream_t ds) -> int {
     for (int n = 1; n <= 4; ++n)
-      if (!cmp[n].order.empty()) {
-        CUDA_TRY(dcb_launch_cmp_deps(sh.d_streams, sh.d_order + cmp[n].order_off, (uint32_t)cmp[n].order.size(), cmp[n].max_entries, A, ds));
+      if (!p.cmp[n].order.empty()) {
+        CUDA_TRY(dcb_launch_cmp_deps(sh.d_streams, sh.d_order + p.cmp[n].order_off, (uint32_t)p.cmp[n].order.size(), p.cmp[n].max_entries, A, ds));
         stats.n_launches++;
       }
     return DCB_OK;
   };
   if (flags_early) {  // the dependency lists need the maps only: next to the rANS kernels as well, behind the maps' copy
-    CUDA_TRY(cudaStreamWaitEvent(ctx->side[dev_index][2], ctx->maps_ev[dev_index], 0));
-    int rcd = launch_cmp_deps(ctx->side[dev_index][2]);
+    CUDA_TRY(cudaStreamWaitEvent(ctx->side[d][2], ctx->maps_ev[d], 0));
+    int rcd = launch_cmp_deps(ctx->side[d][2]);
     if (rcd) return rcd;
   }
   for (int k = 0; k < 3; ++k)
-    if (side_used[k]) {
-      CUDA_TRY(cudaEventRecord(ctx->join_ev[dev_index][k], ctx->side[dev_index][k]));
-      CUDA_TRY(cudaStreamWaitEvent(st, ctx->join_ev[dev_index][k], 0));
+    if (r.side_used[k]) {
+      CUDA_TRY(cudaEventRecord(ctx->join_ev[d][k], ctx->side[d][k]));
+      CUDA_TRY(cudaStreamWaitEvent(st, ctx->join_ev[d][k], 0));
     }
-  if (!wide.order.empty()) {
-    CUDA_TRY(dcb_launch_wide_post(sh.d_streams, sh.d_order + wide.order_off, (uint32_t)wide.order.size(), dump, A, st));
+  if (!p.wide.order.empty()) {
+    CUDA_TRY(dcb_launch_wide_post(sh.d_streams, sh.d_order + p.wide.order_off, (uint32_t)p.wide.order.size(), dump, A, st));
     stats.n_launches++;
   }
   for (int n = 1; n <= 4; ++n) {
-    if (!post[n].order.empty()) {
-      CUDA_TRY(dcb_launch_serial_post(sh.d_streams, sh.d_order + post[n].order_off, (uint32_t)post[n].order.size(), n, dump, 0, A, st));
+    if (!p.post[n].order.empty()) {
+      CUDA_TRY(dcb_launch_serial_post(sh.d_streams, sh.d_order + p.post[n].order_off, (uint32_t)p.post[n].order.size(), n, dump, 0, A, st));
       stats.n_launches++;
     }
-    if (!par[n].order.empty()) {
-      const uint32_t np = (uint32_t)par[n].order.size();
-      const bool time_par = timed && dev_index == 0 && !ctx->ev_par;
+    if (!p.par[n].order.empty()) {
+      const ShardPlan::ParPost &pp = p.pp[n];
+      const uint32_t np = (uint32_t)p.par[n].order.size();
+      const bool time_par = r.events && !ctx->ev_par;
       if (time_par) {
         CUDA_TRY(cudaEventRecord(ctx->ev[6], st));
-        for (uint32_t si : par[n].order) {
+        for (uint32_t si : p.par[n].order) {
           const StreamDesc &sd = sh.streams[si];
           ctx->algo_par += sd.out_bytes + (sd.scheme == SCHEME_TAGGED ? sd.n_entries
                                                                        : (uint64_t)sd.n_entries * sd.ncp * sd.raw_num_bytes);
           if (sd.scheme == SCHEME_TAGGED) ctx->par_streams.push_back({&sh, si});  // + its bit area, once bits_total is back
         }
       }
-      uint32_t *d_runs = sh.d_order + par_aux_off[n];
-      const uint32_t n_prefix = par_rounds[n] ? par_rounds[n] : np;  // entries of the run prefix (rounds or streams)
-      CUDA_TRY(dcb_launch_par_post(sh.d_streams, sh.d_order + par[n].order_off, d_runs, np, par_runs[n][n_prefix], par_run_len[n],
-                                   par_claim[n], par_rounds[n], d_runs + n_prefix + 1, num_sms, n, dump, next_epoch(sh), A, st));
+      uint32_t *d_runs = sh.d_order + pp.runs_off;
+      const uint32_t n_prefix = pp.rounds ? pp.rounds : np;  // entries of the run prefix (rounds or streams)
+      CUDA_TRY(dcb_launch_par_post(sh.d_streams, sh.d_order + p.par[n].order_off, d_runs, np, pp.runs[n_prefix], pp.run_len,
+                                   pp.claim, pp.rounds, d_runs + n_prefix + 1, r.num_sms, n, dump, next_epoch(sh), A, st));
       stats.n_launches += 1;
-      if (par_delta[n]) {
+      if (pp.delta) {
         // streams whose corrections break the modular-sum condition fall back to the exact serial recurrence
-        CUDA_TRY(dcb_launch_serial_post(sh.d_streams, sh.d_order + par[n].order_off, np, n, dump, 1, A, st));
+        CUDA_TRY(dcb_launch_serial_post(sh.d_streams, sh.d_order + p.par[n].order_off, np, n, dump, 1, A, st));
         stats.n_launches++;
       }
       if (time_par) {
@@ -2277,65 +2221,102 @@ int decode_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index, uint8_t *
       }
     }
   }
-  if (!octc.order.empty()) {  // octahedral recurrence of the normals whose corrections par_post2 left in the scratch
-    CUDA_TRY(dcb_launch_oct_chain(sh.d_streams, sh.d_order + octc.order_off, (uint32_t)octc.order.size(), dump, A, st));
+  if (!p.octc.order.empty()) {  // octahedral recurrence of the normals whose corrections par_post2 left in the scratch
+    CUDA_TRY(dcb_launch_oct_chain(sh.d_streams, sh.d_order + p.octc.order_off, (uint32_t)p.octc.order.size(), dump, A, st));
     stats.n_launches++;
   }
-  if (!octs.order.empty()) {
-    CUDA_TRY(dcb_launch_oct_unit(sh.d_streams, sh.d_order + octs.order_off, (uint32_t)octs.order.size(), octs.max_entries, A, st));
+  if (!p.octs.order.empty()) {
+    CUDA_TRY(dcb_launch_oct_unit(sh.d_streams, sh.d_order + p.octs.order_off, (uint32_t)p.octs.order.size(), p.octs.max_entries, A, st));
     stats.n_launches++;
   }
-  if (!copy.order.empty()) {
-    CUDA_TRY(dcb_launch_copy(sh.d_streams, sh.d_order + copy.order_off, (uint32_t)copy.order.size(), copy.max_bytes, A, st));
+  if (!p.copy.order.empty()) {
+    CUDA_TRY(dcb_launch_copy(sh.d_streams, sh.d_order + p.copy.order_off, (uint32_t)p.copy.order.size(), p.copy.max_bytes, A, st));
     stats.n_launches++;
   }
   // mesh prediction stage (ms_para of the stats): parallelogram, constrained multi-parallelogram, tex-coord and
   // geometric-normal kernels, timed as one span
-  bool any_mesh_stage = !tex.order.empty() || !geo.order.empty();
-  for (int n = 1; n <= 4; ++n) any_mesh_stage = any_mesh_stage || !para[n].order.empty() || !cmp[n].order.empty();
-  const bool time_para = timed && dev_index == 0 && !ctx->ev_para && any_mesh_stage;
+  bool any_mesh_stage = !p.tex.order.empty() || !p.geo.order.empty();
+  for (int n = 1; n <= 4; ++n) any_mesh_stage = any_mesh_stage || !p.para[n].order.empty() || !p.cmp[n].order.empty();
+  const bool time_para = r.events && !ctx->ev_para && any_mesh_stage;
   if (time_para) CUDA_TRY(cudaEventRecord(ctx->ev[8], st));
   for (int n = 1; n <= 4; ++n)
-    if (!para[n].order.empty()) {
-      CUDA_TRY(dcb_launch_para(sh.d_streams, sh.d_order + para[n].order_off, (uint32_t)para[n].order.size(), n,
-                               para[n].max_entries, dump, A, st));
+    if (!p.para[n].order.empty()) {
+      CUDA_TRY(dcb_launch_para(sh.d_streams, sh.d_order + p.para[n].order_off, (uint32_t)p.para[n].order.size(), n,
+                               p.para[n].max_entries, dump, A, st));
       stats.n_launches += 2;
     }
-  if (flag_kernels && !flags_early) {
+  if (p.flag_kernels() && !flags_early) {
     int rcf = launch_flag_kernels(st, st);
     if (rcf) return rcf;
     rcf = launch_cmp_deps(st);
     if (rcf) return rcf;
   }
   for (int n = 1; n <= 4; ++n)
-    if (!cmp[n].order.empty()) {  // constrained multi-parallelogram: the chain
-      CUDA_TRY(dcb_launch_cmp(sh.d_streams, sh.d_order + cmp[n].order_off, (uint32_t)cmp[n].order.size(), n, dump, A, st));
+    if (!p.cmp[n].order.empty()) {  // constrained multi-parallelogram: the chain
+      CUDA_TRY(dcb_launch_cmp(sh.d_streams, sh.d_order + p.cmp[n].order_off, (uint32_t)p.cmp[n].order.size(), n, dump, A, st));
       stats.n_launches++;
     }
-  if (!tex.order.empty()) {  // behind the parallelogram kernels: the predictor reads the decoded positions of its parent
-    CUDA_TRY(dcb_launch_tex(sh.d_streams, sh.d_order + tex.order_off, (uint32_t)tex.order.size(), tex.max_entries, dump, A, st));
+  if (!p.tex.order.empty()) {  // behind the parallelogram kernels: the predictor reads the decoded positions of its parent
+    CUDA_TRY(dcb_launch_tex(sh.d_streams, sh.d_order + p.tex.order_off, (uint32_t)p.tex.order.size(), p.tex.max_entries, dump, A, st));
     stats.n_launches += 2;
   }
-  if (!geo.order.empty()) {  // behind the parallelogram kernels: the predictor reads the decoded positions of its parent
-    CUDA_TRY(dcb_launch_geo_normal(sh.d_streams, sh.d_order + geo.order_off, (uint32_t)geo.order.size(), geo.max_entries, dump, A, st));
+  if (!p.geo.order.empty()) {  // behind the parallelogram kernels: the predictor reads the decoded positions of its parent
+    CUDA_TRY(dcb_launch_geo_normal(sh.d_streams, sh.d_order + p.geo.order_off, (uint32_t)p.geo.order.size(), p.geo.max_entries, dump, A, st));
     stats.n_launches++;
   }
   if (time_para) {
     CUDA_TRY(cudaEventRecord(ctx->ev[9], st));
     ctx->ev_para = true;
   }
-  {
-    int rc = point_stage();
-    if (rc) return rc;
+  return DCB_OK;
+}
+
+// Decode everything of one shard into (d_out, d_dbg).  Asynchronous on the shard's stream except
+// for the resolve round trips of Tagged streams.
+int decode_shard(dcb_ctx *ctx, dcb_batch *b, Shard &sh, int dev_index, uint8_t *d_out, uint8_t *d_dbg, uint32_t flags,
+                 bool timed) {
+  cudaStream_t st = ctx->streams[dev_index];
+  CUDA_TRY(cudaSetDevice(sh.device));
+  const uint32_t num_sms = (uint32_t)ctx->num_sms[dev_index];
+  // device 0 of the context writes the decode's statistics record; the other devices' decode threads count their
+  // launches and streams in records of their own, merged by finish_stats
+  dcb_launch_stats &stats = dev_index == 0 ? ctx->stats : ctx->dev_stats[dev_index];
+  if (sh.streams.empty()) return DCB_OK;
+  int rc = reset_descriptors(sh, st);
+  if (rc) return rc;
+  // point order: the kernels write the entry-order staging, the point stage fills d_out from it
+  ShardRun r{ctx, b, sh, dev_index, st, num_sms, stats, DevArenas{sh.d_in, sh.pts ? sh.d_pts : d_out, d_dbg, sh.d_aux, sh.d_tab, sh.d_maps},
+             flags & (DCB_DUMP_SYMBOLS | DCB_DUMP_QINTS), timed && dev_index == 0,
+             timed && sh.device == ctx->devices[0] && env_flags().debug_timing};
+  if (r.events) CUDA_TRY(cudaEventRecord(ctx->ev[0], st));
+  bool deferred_descs = false;
+  if ((rc = run_tag_rounds(r, deferred_descs))) return rc;
+  ShardPlan &p = sh.plan;
+  if ((rc = plan_shard(b, sh, num_sms, p))) return rc;
+  if (!p.order.empty()) {
+    if ((rc = ensure_order(sh, p.order.size()))) return rc;
+    CUDA_TRY(cudaMemcpyAsync(sh.d_order, p.order.data(), p.order.size() * 4, cudaMemcpyHostToDevice, st));
+    // crease flags / flip bits of the 8f-3 predictors depend on the bitstream only: their (serial, small) rABS kernels
+    // run on a side stream next to the rANS kernels -- unless descriptors are still being resolved on the device behind
+    // Tagged bit areas
+    const bool flags_early = p.flag_kernels() && !deferred_descs;
+    if ((rc = launch_rans_groups(r, p, flags_early))) return rc;
+    if ((rc = launch_after_rans(r, p, flags_early))) return rc;
   }
-  if (timed && dev_index == 0) CUDA_TRY(cudaEventRecord(ctx->ev[1], st));
-  if (has_para || deferred_descs || sh.pts) {
-    // parallelogram kernels and the point stage validate the caller's maps on the device, resumed walks parse and
-    // validate on the device: their verdicts travel back behind the kernels and are folded in after the caller's
-    // synchronisation
-    int rc = queue_desc_copyback(ctx, sh, st);
-    if (rc) return rc;
+  if (sh.pts) {  // last writer of every attribute: behind the joins, on the main stream
+    if ((rc = issue_maps_copy(ctx, b, sh, dev_index))) return rc;
+    DevArenas P = r.A;
+    P.out = d_out;
+    r.tl(st, "point stage");
+    CUDA_TRY(dcb_launch_point_stage(sh.pstage, sh.d_streams, P, num_sms, st));
+    r.tl(st);
+    stats.n_launches += 3;
   }
+  if (r.events) CUDA_TRY(cudaEventRecord(ctx->ev[1], st));
+  // parallelogram kernels and the point stage validate the caller's maps on the device, resumed walks parse and
+  // validate on the device: their verdicts travel back behind the kernels and are folded in after the caller's
+  // synchronisation
+  if (p.has_para || deferred_descs || sh.pts) return queue_desc_copyback(ctx, sh, st);
   return DCB_OK;
 }
 
